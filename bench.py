@@ -2,7 +2,7 @@
 """bench.py -- MCMC iterations/s of the SPOM engine on the shapes BASELINE.json names.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload cfg3|cfg2|cfg4|cfg4l|cfg5|cfg1|tiny]
-                    [--impl ours|reference] [--chains C] [--weak]
+                    [--impl ours|reference] [--chains C] [--weak] [--dump-outputs DIR]
 
 A "step" is one MCMC iteration (sweep) of every chain resident on the GPU: refresh of the
 connectivity S, Metropolis steps on (alpha, b) and c, Gibbs updates of the latent z cells and of
@@ -62,7 +62,39 @@ def parse_args():
     ap.add_argument("--blocks-k", type=int, default=4, help="cfg5: colours per axis of the block grid")
     ap.add_argument("--torch-collectives", action="store_true", help="cfg5 on several GPUs: round-1 exchange (torch.distributed all-reduce) instead of NCCL inside the library")
     ap.add_argument("--ess-sweeps", type=int, default=1000, help="extra sweeps after the timed regions for the ESS/s figure (0 = skip)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the timed steps computed in the last one to DIR/<name>.npy "
+                                                          "(rank 0's chains under torchrun), for comparing two builds")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the GPU arm's outputs: it needs --impl ours")
+    return args
+
+
+DUMP_SAMPLE = 1 << 20       # elements kept of a larger array: 3 such arrays in float64 stay below 64 MB
+
+
+def dump_outputs(dirname, arrays):
+    """--dump-outputs: every array as DIR/<name>.npy, in float64 if it is float64 and in float32 otherwise (0/1 states).  An
+    array of more than DUMP_SAMPLE elements becomes a sample of its flattened elements drawn with a fixed seed, so that two
+    runs with the same arguments store the same elements."""
+    out = Path(dirname)
+    out.mkdir(parents=True, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        a = a.astype(np.float64 if a.dtype == np.float64 else np.float32)
+        if a.size > DUMP_SAMPLE:
+            idx = np.sort(np.random.default_rng(0).choice(a.size, DUMP_SAMPLE, replace=False))
+            a = a.ravel()[idx]
+        np.save(out / f"{name}.npy", a)
+
+
+def sweep_outputs(eng):
+    """What a caller of mp_sweep receives after a sweep: its draws (chains x NDRAW: e, c, alpha, b, p, loglik, n_y1, n_z1, K,
+    Ksrc, dsrc), the latent states z and y, and the resident connectivity S (chains x years-1 x patches)."""
+    z, y = eng.get_state()
+    return dict(draws=eng.get_draws(eng.num_draws() - 1, 1)[0], z=z, y=y, S=eng.get_connectivity())
 
 
 def sampler_kwargs(wl):
@@ -309,7 +341,7 @@ def run_ours(args, rank, local_rank, world):
         dist.init_process_group("nccl", device_id=torch.device("cuda", local_rank))
     wl = synth.make_workload(args.workload)
     if args.workload.startswith("cfg5"):
-        line = run_cfg5(args, rank, local_rank, world, wl, args.steps, args.warmup)
+        line = run_cfg5(args, rank, local_rank, world, wl, args.steps, args.warmup, dump=args.dump_outputs)
         if rank == 0:
             emit(json.dumps(line), flush=True)
         if world > 1:
@@ -345,6 +377,8 @@ def run_ours(args, rank, local_rank, world):
         step_ms = arm.timed_steps(K, flush)
         barrier()
         t_wall = time.perf_counter() - t_wall0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, sweep_outputs(eng))      # before the other arms sweep the same chains further
     launches0 = sum(eng.get_timing(reset=True)[1].values())      # launch counters run with timing off too
     total_ms = float(sum(step_ms))
     # ---- end-to-end arm: host buffers in and out every step
@@ -569,10 +603,12 @@ def roofline(workload, wl, cpg, ncand, kms, klaunch, work, geo, probe, hbm_peak,
 
 
 # ----------------------------------------------------------------------------- cfg5: one chain, patch-sharded over the GPUs
-def run_cfg5(args, rank, local_rank, world, wl, steps, warmup):
+def run_cfg5(args, rank, local_rank, world, wl, steps, warmup, dump=None):
     """BASELINE config 5: one chain at N=100,000 x T=30 on the `world` GPUs of the box.  N=1: a single engine.  N>1:
     midaspom_b200/distributed.py ShardedChain (connectivity by target patches, y scan by years, collectives per sweep).
-    Total work is fixed: "scaling": "strong".  Returns the JSON line (rank 0) or None."""
+    Total work is fixed: "scaling": "strong".  `dump`: directory of --dump-outputs.  Returns the JSON line (rank 0) or None."""
+    if dump and world > 1:
+        raise SystemExit("bench.py: --dump-outputs does not support a chain sharded over several GPUs (cfg5 with --gpus > 1)")
     import torch
     import torch.distributed as dist
     import midaspom_b200 as mb
@@ -614,6 +650,8 @@ def run_cfg5(args, rank, local_rank, world, wl, steps, warmup):
             run(1)
             torch.cuda.synchronize()
             times.append(time.perf_counter() - t0)
+    if dump:
+        dump_outputs(dump, sweep_outputs(eng))
     t = torch.tensor([sum(times)], dtype=torch.float64, device=dev)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -664,7 +702,7 @@ def run_cfg1(args, rank):
     if args.impl == "reference":
         exe = ROOT / "oracle" / "_ref" / "MIDASPOM.out"
         if not exe.exists():
-            emit(json.dumps(dict(impl="reference", unavailable="oracle/_ref/MIDASPOM.out not built (no /root/reference at build time)")))
+            emit(json.dumps(dict(impl="reference", unavailable="oracle/_ref/MIDASPOM.out not built (make -C oracle ref REF=<reference checkout>)")))
             return
         tmp = tempfile.mkdtemp()
         threads = host_threads()
@@ -706,6 +744,8 @@ def run_cfg1(args, rank):
         ll, ltot, info = mb.exact_posterior(obs, a=1 / 400, d=100.0, prior_occ=0.5, nstep=101)
         if s >= args.warmup:
             times.append(time.perf_counter() - t0)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, dict(loglik=ll, ltot=np.array([ltot])))
     t = float(np.mean(times))
     v = nev / t
     emit(json.dumps(dict(metric="likelihood_evals_per_sec", value=v, unit="likelihood evaluations/s", n_gpus=1, steps=args.steps, warmup=args.warmup,

@@ -1,9 +1,9 @@
 """Generate tests/golden/golden.npz from THE REFERENCE ITSELF (run in the build container only).
 
-Needs /root/reference and oracle/_ref (make -C oracle ref).  The GPU box has neither the reference
-sources nor this script's inputs; tests there read the committed golden.npz.
+Needs a checkout of the reference and oracle/_ref built from it (make -C oracle ref REF=<dir>).  The
+tests read the committed golden.npz and need neither.
 
-    python tests/golden/make_golden.py
+    REF=<dir> python tests/golden/make_golden.py
 
 What is recorded (all produced by reference code, none by our oracle):
   example_obs        the bundled example as the reference's stream-order parser reads it
@@ -21,6 +21,7 @@ What is recorded (all produced by reference code, none by our oracle):
   future_*_runs      6 runs of `MIDASPOM_future.out -a 50 -m 400 -d 100 -q posterior.txt` (run_examples.sh:17,20): extinct counts per year
 """
 import ctypes as C
+import os
 import re
 import subprocess
 import sys
@@ -33,7 +34,9 @@ HERE = Path(__file__).resolve().parent
 sys.path.insert(0, str(HERE.parent))
 import oracle_lib as O  # noqa: E402
 
-EXAMPLE = "/root/reference/examples/input/occupancies.txt"
+if not os.environ.get("REF"):
+    sys.exit("make_golden.py needs REF=<directory of a reference checkout>")
+EXAMPLE = str(Path(os.environ["REF"]) / "examples" / "input" / "occupancies.txt")
 
 
 def run(prog, args):

@@ -1,6 +1,6 @@
-"""ctypes bindings for the TEST-ONLY oracle (oracle/libspom_oracle.so) and, when it was built in the
-container, the reference harness (oracle/_ref/libmidaspom_ref.so, the reference's own functions
-compiled from /root/reference/sources by oracle/Makefile).
+"""ctypes bindings for the TEST-ONLY oracle (oracle/libspom_oracle.so) and, when it was built by hand,
+the reference harness (oracle/_ref/libmidaspom_ref.so, the reference's own functions compiled from its
+sources by `make -C oracle ref REF=<reference checkout>`).
 
 Only tests/, __graft_entry__.smoke() and bench.py's cpu_baseline / --impl reference legs import this.
 """
@@ -49,11 +49,9 @@ class SpomSamplerCfg(C.Structure):
 
 
 def build_oracle(force: bool = False) -> None:
-    """Compile oracle/libspom_oracle.so (and oracle/_ref when /root/reference is present)."""
+    """Compile oracle/libspom_oracle.so (oracle/_ref is built by hand: make -C oracle ref REF=<reference checkout>)."""
     if force or not ORACLE_SO.exists() or ORACLE_SO.stat().st_mtime < (ORACLE_DIR / "spom_oracle.c").stat().st_mtime:
         subprocess.run(["make", "-C", str(ORACLE_DIR), "oracle"], check=True, capture_output=True)
-    if Path("/root/reference/sources").is_dir() and (force or not REF_SO.exists()):
-        subprocess.run(["make", "-C", str(ORACLE_DIR), "ref"], check=True, capture_output=True)
 
 
 _lib = None

@@ -105,3 +105,22 @@ def test_bench_roofline_from_work_counters():
     # no probe figure for the FP64 peak: the block is simply absent
     roof3 = bench.roofline("cfg3", wl, 64, 102752.0, kms, klaunch, work, geo, dict(probe, dadd_gops=0.0), 6650.0, True, sum(kms.values()))
     assert "fp64" not in roof3["conn"]
+
+
+def test_bench_dump_outputs_types_and_sample(tmp_path):
+    """bench.py --dump-outputs: float64 stays float64, 0/1 states become float32, an array above the size limit becomes the same
+    seeded sample of its elements in every run."""
+    import importlib.util
+    from pathlib import Path
+    spec = importlib.util.spec_from_file_location("bench_mod", Path(__file__).resolve().parents[1] / "bench.py")
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    rng = np.random.default_rng(4)
+    big = rng.random(bench.DUMP_SAMPLE + 1000)
+    z = (rng.random((3, 5, 7)) < 0.5).astype(np.uint8)
+    for d in ("a", "b"):
+        bench.dump_outputs(tmp_path / d, dict(S=big, z=z))
+    S, zd = np.load(tmp_path / "a" / "S.npy"), np.load(tmp_path / "a" / "z.npy")
+    assert S.dtype == np.float64 and S.shape == (bench.DUMP_SAMPLE,) and np.isin(S, big).all()
+    assert (S == np.load(tmp_path / "b" / "S.npy")).all()
+    assert zd.dtype == np.float32 and (zd == z).all()

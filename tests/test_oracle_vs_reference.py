@@ -117,7 +117,7 @@ def test_variant_terms_match_pije_pijc_pijcsource(golden):
         np.testing.assert_allclose(got, res[i], rtol=1e-13, atol=0)
 
 
-@pytest.mark.skipif(not O.have_ref(), reason="oracle/_ref not built (no /root/reference here)")
+@pytest.mark.skipif(not O.have_ref(), reason="oracle/_ref not built (make -C oracle ref REF=<reference checkout>)")
 def test_live_reference_compPePc_random():
     """Live call into the reference's compPePc on random small landscapes (not only the fixture)."""
     rng = np.random.default_rng(7)
