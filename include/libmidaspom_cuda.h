@@ -22,6 +22,7 @@
  *                             (main_MIDASPOM_MPI.c:361-372,483-505) becomes chain sharding (chain_offset)
  *   mp_set_era / mp_params.K,Ksrc,dsrc   dieoff.c:56-57,78 ; loss.c:93-101,365 ; future.c:67,90-97
  *   mp_simulate               future.c:64-110 (simpij) + :359-386 (simulation loop)
+ *   mp_forecast               future.c:359-386 at large N: the simulation loop started from the sampler's own chains
  *
  * All device memory is owned by the engine handle; host buffers are owned by the caller.  One
  * handle per GPU / host thread (thread-compatible, not thread-safe).  There is no CPU fallback:
@@ -188,6 +189,27 @@ int mp_simulate(mp_engine *h, const mp_params *par, const uint8_t *z0, int nyear
  * the posterior table and a completion of the last survey for every simulation) */
 int mp_simulate_ensemble(mp_engine *h, const mp_params *par_per_sim /* nsims */, const uint8_t *z0_per_sim /* nsims*N */,
                          int nyears, int nsims, uint64_t seed, int era_all, uint8_t *z_out, int32_t *occupied_out);
+/* Posterior-predictive forecast from the chains' current state (large-N counterpart of MIDASPOM_future.out,
+ * future.c:359-386).  Chain c starts nrep trajectories from its own latent occupancy of the last survey year,
+ * z[c][T-1], with its own resident parameters, and simulates nyears years of simpij (future.c:64-110).
+ * Trajectory (c, r) draws from the Philox streams that mp_simulate_ensemble gives simulation number
+ * (chain_offset + c) * nrep + r under `seed`, so results do not depend on how chains are sharded.
+ * scenario (nullable): {K, Ksrc, dsrc}.  Replaces the chains' K, Ksrc, dsrc and applies them in every forecast year
+ *   (era_all of mp_simulate; the reference's -D, -S, -s).  NULL: plain model.
+ * occupied_out  (nullable): n_chains * nrep * (nyears+1) int32, occupied patches per trajectory (year 0 = start).
+ * incidence_out (nullable): (nyears+1) * N uint32, the number of this engine's trajectories with patch k occupied in year t.
+ * Leaves all sampler state as it was: chain state, S and its validity flags, draws, sweep counter, scales, captured graphs.
+ * Synchronous, on the engine stream after any queued sweeps.
+ * One year: extinction draws, then the connectivity of every (chain, replicate) by k_conn with the replicates in place of the
+ * years (one weight per (target, source) pair and chain, shared by the chain's replicates; FP64 accumulation; FP32 engines on
+ * landscapes with positions skip source tiles whose weights add less than 2^-32 to any c K S, MP_CONN_CULL=0 disables),
+ * then the colonisation draws.  Counted under MP_K_SIM and in MP_CNT_CONN_*; mp_set_shard does not apply (every target).
+ * Device memory: one arena per call of about C nrep N (8 + 2 + 0.5 (FP32) | 1 (FP64)) bytes -- S, the current and surviving
+ * states, the source records -- plus C N (8 | 4) bytes of area weights and the outputs.
+ * MP_ERR_ARG: nyears < 1, nrep < 1 or > 65535, (chain_offset + n_chains) * nrep >= 2^32, scenario K <= 0.
+ * MP_ERR_STATE: no landscape, no chain state, a chain with alpha <= 0. */
+int mp_forecast(mp_engine *h, int nyears, int nrep, uint64_t seed, const double *scenario,
+                int32_t *occupied_out, uint32_t *incidence_out);
 
 /* ---- exact small-n engine: the reference's own algorithm (state enumeration on an (e,c) grid) ----
  * Replaces the whole hot loop of MIDASPOM.out, main_MIDASPOM.c:198-290 (state tables) and :341-395

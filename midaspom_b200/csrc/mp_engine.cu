@@ -57,19 +57,10 @@ template <typename R> static int launch_pack_sources(mp_engine *h, int set_mask)
     CK(cudaGetLastError());
     return MP_OK;
 }
-template <typename R, int GEOM> static int launch_conn_g(mp_engine *h, int set_base, int nsets, bool eval)
+// k_conn over the buffers of `a` (sets [a.set_base, a.set_base + nsets), every chain of a.nchains).  a32: the evaluation form
+// with the year contraction on the FP32 pipe (FP32 engines); otherwise the DFMA form.
+template <typename R, int GEOM> static int launch_conn_args(mp_engine *h, const ConnArgs<R> &a, int nsets, bool a32)
 {
-    Timed tm(h, MP_K_CONN);
-    ConnArgs<R> a;
-    a.ls = view<R>(h);
-    a.par[0] = h->d_par; a.par[1] = h->d_prop;
-    a.S[0] = h->d_S[0]; a.S[1] = h->d_S[1];
-    a.rec = (const SrcRec<R> *)h->d_srec;
-    a.ntrans = h->cfg.n_years - 1; a.nwords = h->nwords; a.nchains = h->cfg.n_chains; a.set_base = set_base;
-    a.k_lo = h->conn_lo; a.k_hi = h->conn_hi < 0 ? h->cfg.n_patches : h->conn_hi;
-    a.perm = h->d_perm; a.box32 = (const float4 *)h->d_tile_box;
-    a.mlow = h->d_mlow; a.area_max = (float)h->area_max; a.area_min = (float)h->area_min;   // bounds: launch_conn_bounds
-    a.stats = h->d_work;
     if (a.k_hi <= a.k_lo) return MP_OK;
     const int ny = a.ntrans;                          // year accumulators per target: next multiple of 4 (<= 32 per pass)
     // FP32 engines on landscapes with positions skip source tiles out of reach (see CONN_CULL_LOG2); FP64 never culls
@@ -79,20 +70,13 @@ template <typename R, int GEOM> static int launch_conn_g(mp_engine *h, int set_b
     // unequal (culled) work better, and the FP32 engines go on to 32 threads x 1 target (8x the CTAs, 96 registers: cfg3 with
     // 8 chains 1.41 -> 1.25 ms per launch; no difference at cfg5).  Every shape gives bit-identical sums.  MP_CONN_SHAPE=1|2|3|4
     // forces a shape.
-    const long long wide_ctas = (long long)((a.k_hi - a.k_lo + 255) / 256) * h->cfg.n_chains * nsets;
+    const long long wide_ctas = (long long)((a.k_hi - a.k_lo + 255) / 256) * a.nchains * nsets;
     // shape 1: 128 threads, 2: 64 threads, 3: 32 threads (2 targets per thread each), 4: 32 threads x 1 target (FP32 engines)
     int shape = h->conn_shape ? h->conn_shape : wide_ctas >= 16LL * h->sm_count ? 1 : wide_ctas >= 4LL * h->sm_count ? 2 : 4;
-    if (shape == 4 && (sizeof(R) != 4 || (eval && h->conn_acc32))) shape = 3;
+    if (shape == 4 && (sizeof(R) != 4 || a32)) shape = 3;
     const int per_cta = shape == 1 ? 256 : shape == 2 ? 128 : shape == 3 ? 64 : 32;
-    dim3 grid((a.k_hi - a.k_lo + per_cta - 1) / per_cta, h->cfg.n_chains, nsets);
-    // Evaluation entry points of the FP32 engines (mp_connectivity, mp_loglik, mp_loglik_host): the year contraction on the FP32
-    // pipe (FFMA2, FP32 partial sums per 32 sources joined in FP64; mp_conn32.cu), accurate to ~1e-7 of every S.  The sampler's
-    // own S keeps the DFMA form below: a weight the y scan later removes must cancel to the last bit even where S then falls
-    // by orders of magnitude.  MP_CONN_ACC32=0 keeps the DFMA form everywhere.
-    if (sizeof(R) == 4 && eval && h->conn_acc32) {
-        h->S_exact = false;
-        return mp_launch_conn32(h, &a, GEOM, ny, shape, cull ? 1 : 0, grid.x, grid.y, grid.z);
-    }
+    dim3 grid((a.k_hi - a.k_lo + per_cta - 1) / per_cta, a.nchains, nsets);
+    if (sizeof(R) == 4 && a32) return mp_launch_conn32(h, &a, GEOM, ny, shape, cull ? 1 : 0, grid.x, grid.y, grid.z);
 #define MP_CONN_T(NYB, NT) do { if (cull) k_conn<R, GEOM, NYB, CAN_CULL, 2, NT><<<grid, NT, 0, h->stream>>>(a);      \
                                 else k_conn<R, GEOM, NYB, false, 2, NT><<<grid, NT, 0, h->stream>>>(a); } while (0)
 #define MP_CONN_ONE(NYB) do { if constexpr (sizeof(R) == 4) { if (cull) k_conn<R, GEOM, NYB, CAN_CULL, 1, 32><<<grid, 32, 0, h->stream>>>(a);   \
@@ -106,6 +90,27 @@ template <typename R, int GEOM> static int launch_conn_g(mp_engine *h, int set_b
 #undef MP_CONN_T
     CK(cudaGetLastError());
     return MP_OK;
+}
+template <typename R, int GEOM> static int launch_conn_g(mp_engine *h, int set_base, int nsets, bool eval)
+{
+    Timed tm(h, MP_K_CONN);
+    ConnArgs<R> a;
+    a.ls = view<R>(h);
+    a.par[0] = h->d_par; a.par[1] = h->d_prop;
+    a.S[0] = h->d_S[0]; a.S[1] = h->d_S[1];
+    a.rec = (const SrcRec<R> *)h->d_srec;
+    a.ntrans = h->cfg.n_years - 1; a.nwords = h->nwords; a.nchains = h->cfg.n_chains; a.set_base = set_base;
+    a.k_lo = h->conn_lo; a.k_hi = h->conn_hi < 0 ? h->cfg.n_patches : h->conn_hi;
+    a.perm = h->d_perm; a.box32 = (const float4 *)h->d_tile_box;
+    a.mlow = h->d_mlow; a.area_max = (float)h->area_max; a.area_min = (float)h->area_min;   // bounds: launch_conn_bounds
+    a.stats = h->d_work;
+    // Evaluation entry points of the FP32 engines (mp_connectivity, mp_loglik, mp_loglik_host): the year contraction on the FP32
+    // pipe (FFMA2, FP32 partial sums per 32 sources joined in FP64; mp_conn32.cu), accurate to ~1e-7 of every S.  The sampler's
+    // own S keeps the DFMA form: a weight the y scan later removes must cancel to the last bit even where S then falls
+    // by orders of magnitude.  MP_CONN_ACC32=0 keeps the DFMA form everywhere.
+    const bool a32 = sizeof(R) == 4 && eval && h->conn_acc32;
+    if (a32 && a.k_hi > a.k_lo) h->S_exact = false;
+    return launch_conn_args<R, GEOM>(h, a, nsets, a32);
 }
 // Culling bounds of k_conn: a lower bound of every target group's S, taken from the resident S BEFORE it is overwritten
 // or zeroed (none before the first refresh: mlow = 0, nothing is skipped).
@@ -1336,6 +1341,114 @@ int mp_simulate_ensemble(mp_engine *h, const mp_params *par_per_sim, const uint8
                          uint64_t seed, int era_all, uint8_t *z_out, int32_t *occupied_out)
 {
     return simulate_impl(h, par_per_sim, 1, z0_per_sim, nyears, nsims, seed, era_all, z_out, occupied_out);
+}
+
+// ---- posterior-predictive forecast from the chains' own state
+// Buffers of one call (one arena); states and S are [chain][replicate][patch], records [chain][word][padded slot]
+struct FcBufs {
+    const mp_params *par; void *aw; uint8_t *zc, *yc; double *S; void *rec; float *mlow; int32_t *occ; uint32_t *inc;
+};
+extern "C++" template <typename R> int forecast_t(mp_engine *h, const FcBufs &b, int nyears, int nrep, uint64_t seed, int era_all)
+{
+    Timed tm(h, MP_K_SIM);
+    const int n = h->cfg.n_patches, C = h->cfg.n_chains, T = h->cfg.n_years, npad = conn_npad(n), nwords = (nrep + 31) / 32;
+    const unsigned tiles = (unsigned)((n + 255) / 256);
+    const uint32_t sim0 = (uint32_t)h->cfg.chain_offset * (uint32_t)nrep;
+    mp::Landscape<R> ls = view<R>(h), lsrc = ls;
+    if (h->geom != MP_GEOM_COORDS) { lsrc.px = nullptr; lsrc.py = nullptr; }
+    k_area_weights<R><<<dim3(tiles, C), 256, 0, h->stream>>>(b.par, h->have_area ? h->d_area : nullptr, (R *)b.aw, n);
+    CK(cudaGetLastError());
+    k_fc_init<<<dim3(tiles, C), 256, 0, h->stream>>>(h->d_z, T, n, nrep, nyears, b.zc, b.occ, b.inc);
+    CK(cudaGetLastError());
+    // k_conn over the forecast's own buffers: every target, the replicates in place of the years, the forecast's culling floor
+    ConnArgs<R> a;
+    a.ls = ls;
+    a.par[0] = a.par[1] = b.par;
+    a.S[0] = a.S[1] = b.S;
+    a.rec = (const SrcRec<R> *)b.rec;
+    a.ntrans = nrep; a.nwords = nwords; a.nchains = C; a.set_base = 0;
+    a.k_lo = 0; a.k_hi = n;
+    a.perm = h->d_perm; a.box32 = (const float4 *)h->d_tile_box;
+    a.mlow = b.mlow; a.area_max = (float)h->area_max; a.area_min = (float)h->area_min;
+    a.stats = h->d_work;
+    int rc;
+    for (int t = 0; t < nyears; t++) {
+        k_fc_ext<R><<<dim3(tiles, nrep, C), 256, 0, h->stream>>>(b.par, n, nrep, seed, sim0, t, era_all, b.zc, b.yc);
+        CK(cudaGetLastError());
+        k_pack_sources<R><<<dim3((npad + 255) / 256, C, nwords), 256, 0, h->stream>>>(lsrc, h->d_perm, (const R *)b.aw, nullptr, b.yc, nrep,
+                                                                                      nwords, 1, (SrcRec<R> *)b.rec);
+        CK(cudaGetLastError());
+        switch (h->geom) {
+        case MP_GEOM_LINEAR: rc = launch_conn_args<R, MP_GEOM_LINEAR>(h, a, 1, false); break;
+        case MP_GEOM_COORDS: rc = launch_conn_args<R, MP_GEOM_COORDS>(h, a, 1, false); break;
+        default: rc = launch_conn_args<R, MP_GEOM_DENSE>(h, a, 1, false); break;
+        }
+        if (rc != MP_OK) return rc;
+        k_fc_col<R><<<dim3(tiles, C), 256, 0, h->stream>>>(ls, b.par, nrep, seed, sim0, t, nyears, era_all, b.S, b.yc, b.zc, b.occ, b.inc);
+        CK(cudaGetLastError());
+    }
+    return MP_OK;
+}
+int mp_forecast(mp_engine *h, int nyears, int nrep, uint64_t seed, const double *scenario, int32_t *occupied_out, uint32_t *incidence_out)
+{
+    if (!h) return MP_ERR_ARG;
+    CK(cudaSetDevice(h->cfg.device));
+    REQUIRE(nyears >= 1 && nrep >= 1, MP_ERR_ARG, "mp_forecast: need nyears >= 1 and nrep >= 1");
+    REQUIRE(nrep <= 65535, MP_ERR_ARG, "mp_forecast: at most 65535 replicates per chain");
+    REQUIRE((uint64_t)(h->cfg.chain_offset + h->cfg.n_chains) * (uint64_t)nrep <= 0xffffffffull, MP_ERR_ARG,
+            "mp_forecast: simulation numbers (chain_offset + n_chains) * nrep must fit in 32 bits");
+    REQUIRE(!scenario || scenario[0] > 0.0, MP_ERR_ARG, "mp_forecast: the scenario needs K > 0");
+    int rc = check_ready(h);
+    if (rc != MP_OK) return rc;
+    const size_t N = nN(h), C = nC(h), cells = C * (size_t)nrep * N, ngroups = (N + 31) / 32;
+    const size_t nwords = ((size_t)nrep + 31) / 32, npad = (size_t)conn_npad((int)N);
+    // the chains' parameters after any queued sweeps; a scenario replaces K, Ksrc, dsrc and applies them every year
+    std::vector<mp_params> par(C);
+    CK(cudaMemcpyAsync(par.data(), h->d_par, C * sizeof(mp_params), cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    for (size_t c = 0; c < C; c++) {
+        REQUIRE(par[c].alpha > 0.0, MP_ERR_STATE, "mp_forecast: every chain needs alpha > 0");
+        if (scenario) { par[c].K = scenario[0]; par[c].Ksrc = scenario[1]; par[c].dsrc = scenario[2]; }
+    }
+    // Culling floor of k_conn (FP32 engines with positions): a source group is skipped for a target group when every weight
+    // between them is below 2^-30 mlow_c, so the skipped weights change c K S of a target by less than N 2^-30 mlow_c c K = 2^-32
+    // (the resolution of the uniform that decides a colonisation) with mlow_c = 2^-2 / (c K N); K = 1 without a scenario.
+    const double Keff = scenario ? scenario[0] : 1.0;
+    std::vector<float> mlow(C * ngroups);
+    for (size_t c = 0; c < C; c++)
+        std::fill(mlow.begin() + c * ngroups, mlow.begin() + (c + 1) * ngroups, (float)std::min(0.25 / (par[c].c * Keff * (double)N), 3.0e38));
+    // one arena per call: parameters, A^b, current / surviving states, S, source records, culling floor, outputs
+    size_t off = 0;
+    auto carve = [&](size_t bytes) { const size_t o = off; off += (bytes + 255) / 256 * 256; return o; };
+    const size_t rec_bytes = is64(h) ? sizeof(SrcRec<double>) : sizeof(SrcRec<float>);
+    const size_t occ_bytes = C * (size_t)nrep * (nyears + 1) * 4, inc_bytes = (size_t)(nyears + 1) * N * 4;
+    const size_t o_par = carve(C * sizeof(mp_params)), o_aw = carve(C * N * rsz(h)), o_zc = carve(cells), o_yc = carve(cells),
+                 o_S = carve(cells * 8), o_rec = carve(C * nwords * npad * rec_bytes), o_mlow = carve(C * ngroups * sizeof(float)),
+                 o_occ = carve(occupied_out ? occ_bytes : 0), o_inc = carve(incidence_out ? inc_bytes : 0);
+    unsigned char *arena = nullptr;
+    cudaError_t e;
+#define FCCK(call) if ((e = (call)) != cudaSuccess) { h->err = std::string(#call) + ": " + cudaGetErrorString(e); rc = MP_ERR_CUDA; goto done; }
+    FCCK(cudaMalloc(&arena, std::max<size_t>(off, 256)));
+    {
+        FcBufs b;
+        b.par = (const mp_params *)(arena + o_par); b.aw = arena + o_aw; b.zc = arena + o_zc; b.yc = arena + o_yc;
+        b.S = (double *)(arena + o_S); b.rec = arena + o_rec; b.mlow = (float *)(arena + o_mlow);
+        b.occ = occupied_out ? (int32_t *)(arena + o_occ) : nullptr; b.inc = incidence_out ? (uint32_t *)(arena + o_inc) : nullptr;
+        FCCK(cudaMemcpyAsync(arena + o_par, par.data(), C * sizeof(mp_params), cudaMemcpyHostToDevice, h->stream));
+        FCCK(cudaMemcpyAsync(b.mlow, mlow.data(), mlow.size() * sizeof(float), cudaMemcpyHostToDevice, h->stream));
+        if (b.occ) FCCK(cudaMemsetAsync(b.occ, 0, occ_bytes, h->stream));
+        if (b.inc) FCCK(cudaMemsetAsync(b.inc, 0, inc_bytes, h->stream));
+        rc = is64(h) ? forecast_t<double>(h, b, nyears, nrep, seed, scenario ? 1 : 0) : forecast_t<float>(h, b, nyears, nrep, seed, scenario ? 1 : 0);
+        if (rc != MP_OK) goto done;
+        if (occupied_out) FCCK(cudaMemcpyAsync(occupied_out, b.occ, occ_bytes, cudaMemcpyDeviceToHost, h->stream));
+        if (incidence_out) FCCK(cudaMemcpyAsync(incidence_out, b.inc, inc_bytes, cudaMemcpyDeviceToHost, h->stream));
+        FCCK(cudaStreamSynchronize(h->stream));
+    }
+#undef FCCK
+done:
+    cudaStreamSynchronize(h->stream);
+    cudaFree(arena);
+    return rc;
 }
 
 // ---- plumbing

@@ -9,6 +9,7 @@
 //  k_update_z      Gibbs update of latent occupancy cells (conditionally independent given y)
 //  k_propose_* / k_decide_* / k_update_ep / k_record   Metropolis bookkeeping, one warp per chain
 //  k_sim_init / k_sim_ext / k_sim_col   forward simulator (future.c:64-110)
+//  k_fc_init / k_fc_ext / k_fc_col      posterior-predictive forecast from the chains (with k_pack_sources + k_conn)
 #pragma once
 #include "mp_device.cuh"
 #include "mp_conn.cuh"   // k_pack_sources, k_group_min_S, k_conn
@@ -650,6 +651,91 @@ k_sim_col(Landscape<R> ls, const mp_params *__restrict__ pars, int per_sim, cons
     }
     const int c2 = __reduce_add_sync(0xffffffffu, v);
     if ((tid & 31) == 0 && occ_out && c2) atomicAdd(&occ_out[(size_t)si * (nyears + 1) + t + 1], c2);
+}
+
+// ------------------------------------------------------------------ posterior-predictive forecast (mp_forecast)
+// nrep trajectories per chain from the chain's own z[c][T-1] and parameters, states laid out [chain][replicate][patch].
+// Trajectory (c, r) is simulation number sim0 + c * nrep + r of mp_simulate_ensemble: the same Philox draws per patch number.
+// One year = k_fc_ext, then S of every (chain, replicate) from k_conn with the replicates in place of the years (k_pack_sources
+// packs 32 replicates per record word), then k_fc_col.
+//   k_fc_init  grid (patch tiles, chains): start states, year-0 counts and incidence
+static __global__ void __launch_bounds__(256)
+k_fc_init(const uint8_t *__restrict__ z, int T, int n, int nrep, int nyears, uint8_t *__restrict__ zc, int32_t *__restrict__ occ,
+          uint32_t *__restrict__ inc)
+{
+    __shared__ int s_cnt;
+    const int c = blockIdx.y, k = blockIdx.x * 256 + threadIdx.x;
+    if (threadIdx.x == 0) s_cnt = 0;
+    __syncthreads();
+    int v = 0;
+    if (k < n) {
+        v = z[((size_t)c * T + T - 1) * n + k] != 0;
+        for (int r = 0; r < nrep; r++) zc[((size_t)c * nrep + r) * n + k] = (uint8_t)v;
+        if (inc && v) atomicAdd(&inc[k], (uint32_t)nrep);
+    }
+    const int w = __reduce_add_sync(0xffffffffu, v);
+    if ((threadIdx.x & 31) == 0 && w) atomicAdd(&s_cnt, w);
+    __syncthreads();
+    if (occ && s_cnt)
+        for (int r = threadIdx.x; r < nrep; r += blockDim.x) atomicAdd(&occ[((size_t)c * nrep + r) * (nyears + 1)], s_cnt);
+}
+//   k_fc_ext   grid (patch tiles, replicates, chains): survive iff u > E, u keyed by (sim, year, patch number) as in k_sim_ext
+template <typename R>
+__global__ void __launch_bounds__(256)
+k_fc_ext(const mp_params *__restrict__ pars, int n, int nrep, uint64_t seed, uint32_t sim0, int t, int era_all,
+         const uint8_t *__restrict__ zc, uint8_t *__restrict__ yc)
+{
+    const int k = blockIdx.x * 256 + threadIdx.x, r = blockIdx.y, c = blockIdx.z;
+    if (k >= n) return;
+    const size_t i = ((size_t)c * nrep + r) * n + k;
+    uint8_t v = 0;
+    if (zc[i]) {
+        const Trans<R> tr = make_trans<R>(pars[c], era_all);
+        const uint4 u = rng(seed, sim0 + (uint32_t)c * (uint32_t)nrep + (uint32_t)r, (uint32_t)t, RK_SIM_EXT, (uint32_t)k, 0);
+        v = u01(u.x) > (double)tr.E;
+    }
+    yc[i] = v;
+}
+//   k_fc_col   grid (patch tiles, chains): one thread per (chain, patch) runs the colonisation draws of all replicates
+//              (u < C as in k_sim_col), writes next year's z, adds the occupied count of every trajectory (one shared-memory
+//              atomic per warp, one global atomic per CTA and replicate) and the patch's count over the replicates to incidence
+template <typename R>
+__global__ void __launch_bounds__(256)
+k_fc_col(Landscape<R> ls, const mp_params *__restrict__ pars, int nrep, uint64_t seed, uint32_t sim0, int t, int nyears, int era_all,
+         const double *__restrict__ S, const uint8_t *__restrict__ yc, uint8_t *__restrict__ zc, int32_t *__restrict__ occ,
+         uint32_t *__restrict__ inc)
+{
+    __shared__ int s_cnt[32];
+    const int n = ls.n, c = blockIdx.y, tid = threadIdx.x, k = blockIdx.x * 256 + tid;
+    const Trans<R> tr = make_trans<R>(pars[c], era_all);
+    const R g = k < n ? source_term<R>(ls, tr, k) : (R)0;
+    uint32_t mine = 0;
+    for (int r0 = 0; r0 < nrep; r0 += 32) {
+        const int nr = min(32, nrep - r0);
+        if (tid < 32) s_cnt[tid] = 0;
+        __syncthreads();
+        for (int j = 0; j < nr; j++) {
+            const int r = r0 + j;
+            int v = 0;
+            if (k < n) {
+                const size_t i = ((size_t)c * nrep + r) * n + k;
+                if (yc[i]) v = 1;
+                else {
+                    const R C = col_prob<R>(tr, (R)S[i], g);
+                    const uint4 u = rng(seed, sim0 + (uint32_t)c * (uint32_t)nrep + (uint32_t)r, (uint32_t)t, RK_SIM_COL, (uint32_t)k, 0);
+                    v = u01(u.x) < (double)C;
+                }
+                zc[i] = (uint8_t)v;
+            }
+            mine += v;
+            const int w = __reduce_add_sync(0xffffffffu, v);
+            if ((tid & 31) == 0 && w) atomicAdd(&s_cnt[j], w);
+        }
+        __syncthreads();
+        if (occ && tid < nr && s_cnt[tid]) atomicAdd(&occ[((size_t)c * nrep + r0 + tid) * (nyears + 1) + t + 1], s_cnt[tid]);
+        __syncthreads();
+    }
+    if (inc && mine) atomicAdd(&inc[(size_t)(t + 1) * n + k], mine);
 }
 
 // ------------------------------------------------------------------ peak probes (roofline denominators)

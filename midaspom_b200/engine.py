@@ -32,7 +32,7 @@ ABI_SYMBOLS = (
     "mp_get_timing", "mp_probe_peaks", "mp_get_stream", "mp_exact_posterior", "mp_exact_last_error", "mp_simulate_ensemble", "mp_exact_variant", "mp_set_shard", "mp_sweep_phase",
     "mp_get_scan_order", "mp_get_work_counters", "mp_get_scan_geometry", "mp_get_conn_path", "mp_set_scan_blocks",
     "mp_comm_unique_id", "mp_comm_init", "mp_comm_init_all", "mp_comm_destroy", "mp_comm_rank", "mp_comm_size", "mp_comm_last_error",
-    "mp_gather_draws", "mp_gather_draws_all", "mp_sweep_sharded", "mp_sweep_sharded_all",
+    "mp_gather_draws", "mp_gather_draws_all", "mp_sweep_sharded", "mp_sweep_sharded_all", "mp_forecast",
 )
 
 
@@ -128,6 +128,7 @@ def load_library(build_if_missing: bool = True) -> C.CDLL:
     L.mp_get_draws.argtypes = [vp, C.c_int, C.c_int, dp]
     L.mp_simulate.argtypes = [vp, pp, u8p, C.c_int, C.c_int, C.c_uint64, C.c_int, u8p, C.POINTER(C.c_int32)]
     L.mp_simulate_ensemble.argtypes = [vp, pp, u8p, C.c_int, C.c_int, C.c_uint64, C.c_int, u8p, C.POINTER(C.c_int32)]
+    L.mp_forecast.argtypes = [vp, C.c_int, C.c_int, C.c_uint64, dp, C.POINTER(C.c_int32), C.POINTER(C.c_uint32)]
     L.mp_device_ptr.argtypes = [vp, C.c_int, C.POINTER(vp), C.POINTER(C.c_size_t)]
     L.mp_get_stream.argtypes = [vp, C.POINTER(vp)]
     L.mp_set_timing.argtypes = [vp, C.c_int]
@@ -456,6 +457,19 @@ class Engine:
         self._ck(self.lib.mp_simulate_ensemble(self.h, arr, _p(z0, _u8p), nyears, nsims, seed, int(era_all), _p(z_out, _u8p),
                                                _p(occ, C.POINTER(C.c_int32))), "mp_simulate_ensemble")
         return z_out, occ
+
+    def forecast(self, nyears, nrep, seed=1, scenario=None, want_counts=True, want_incidence=True):
+        """Posterior-predictive forecast from the chains' current state (mp_forecast): nrep trajectories per chain from the
+        chain's z[c][T-1] and parameters.  scenario: dict with K, Ksrc, dsrc applied every year, or None for the plain model.
+        Returns (occupied [C, nrep, nyears+1] int32, incidence [nyears+1, N] uint32), each None when not requested."""
+        scen = None
+        if scenario is not None:
+            scen = np.array([float(scenario["K"]), float(scenario.get("Ksrc", 0.0)), float(scenario.get("dsrc", 0.0))])
+        occ = np.zeros((self.C, nrep, nyears + 1), dtype=np.int32) if want_counts else None
+        inc = np.zeros((nyears + 1, self.N), dtype=np.uint32) if want_incidence else None
+        self._ck(self.lib.mp_forecast(self.h, int(nyears), int(nrep), int(seed), _p(scen, _dp), _p(occ, C.POINTER(C.c_int32)),
+                                      _p(inc, C.POINTER(C.c_uint32))), "mp_forecast")
+        return occ, inc
 
     @staticmethod
     def _one_param(p):
