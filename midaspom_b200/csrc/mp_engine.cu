@@ -220,15 +220,19 @@ static int launch_sweep_y_fast(mp_engine *h)
     // large landscapes: a cluster of 8 holds the task's state; with few tasks per GPU (year sharding) spread each
     // task over 16 SMs instead -- the scan is latency-bound per flip
     const int ntask_own = (C * ntrans - h->task_first + h->task_stride - 1) / h->task_stride;
+    // exact spatial culling of the evaluation (mp_sweep_cull.cuh) where positions exist and the landscape is large
+    const bool culled = h->fast_cull && h->geom != MP_GEOM_DENSE && tpt >= 512;
+    // the culled scan at 512 threads per task runs in clusters of 4 x 128 threads whatever the task count: up to five such CTAs
+    // of different tasks share an SM, and their independent trips cover each other's latency.  Measured at cfg3 (one B200,
+    // 1,000 W), ms per launch for CS = 1 / 2 / 4 / 8: 64 chains 60.1 / 60.2 / 56.2 / 62.8, 32 chains 32.1 / 32.3 / 29.4 / 32.9,
+    // 16 chains 17.7 / 18.0 / 15.3 / 18.6, 8 chains 9.8 / 9.9 / 8.5 / 11.0 (pick_cluster's wave model chose 1, 2, 2 and 4)
     int cs = tpt > 1024 ? (h->fast_cs == 16 || (h->fast_cs == 0 && tpt >= 4096 && ntask_own * 16 <= h->sm_count) ? 16 : 8)
-                        : (h->fast_cs ? h->fast_cs : (tpt == 256 ? 1 : pick_cluster(C * ntrans, h->sm_count, 8)));
+                        : (h->fast_cs ? h->fast_cs : (tpt == 256 ? 1 : culled && tpt == 512 ? 4 : pick_cluster(C * ntrans, h->sm_count, 8)));
     // a CTA holds 16 bytes per target of its share (+ the 2 KB record ring of the culled scan): widen the cluster until that fits
     if (tpt >= 512 && tpt <= 1024) {
         const size_t ept = (size_t)(n + tpt - 1) / tpt;
         while (cs < 8 && ept * (size_t)(tpt / cs) * 16 + 2048 > 227 * 1024) cs *= 2;
     }
-    // exact spatial culling of the evaluation (mp_sweep_cull.cuh) where positions exist and the landscape is large
-    const bool culled = h->fast_cull && h->geom != MP_GEOM_DENSE && tpt >= 512;
     h->last_scan[0] = tpt; h->last_scan[1] = cs; h->last_scan[2] = culled ? (tpt > 1024 ? 4 : 2) : 1; h->last_scan[3] = culled;
     if (culled && h->blk_active) {
         // block grid: decide per task whether its halo suffices this sweep, scan those tasks colour by colour (the blocks of
