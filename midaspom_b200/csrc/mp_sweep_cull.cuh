@@ -59,6 +59,8 @@ k_sweep_y_cull(Landscape<float> ls, const int *__restrict__ perm, const mp_param
     constexpr int NSLOT = HIER ? CS : TPT / 32;
     extern __shared__ __align__(16) unsigned char smem_raw[];
     constexpr int NV = (SP + 3) / 4;                                 // float4 per sender in the exchange of the SP sums
+    // two sums from at most 16 senders (every 512-thread task): reduce-scatter over the two half-warps, one float2 per sender
+    constexpr bool PAIR = SP == 2 && !HIER && NSLOT <= 16;
     __shared__ __align__(16) float4 red[2][2][32][NV];
     __shared__ __align__(16) float4 wred[HIER ? 2 : 1][2][32][NV];
     __shared__ __align__(8) unsigned long long mbar[2][2];
@@ -76,6 +78,11 @@ k_sweep_y_cull(Landscape<float> ls, const int *__restrict__ perm, const mp_param
     const int ept = (nl + TPT - 1) / TPT;                            // slots per thread (<= ept_max, which sizes the shared memory)
     float4 *sT = reinterpret_cast<float4 *>(smem_raw);               // {S_hi, S_lo, x, y} (COORDS) or {S_hi, S_lo, patch, -} (LINEAR)
     float4 *ring = sT + ept_max * NT;                                // 2 chunks of RC candidate records (two float4 each)
+    // this thread's column of sT (slot j at sTt[j * NT]) from a shared address held in a register: left to the compiler, the
+    // column's base was rebuilt from the shared window base in every batch of the slot loops
+    uint32_t col_off = smem_u32(sT + tid);
+    asm volatile("" : "+r"(col_off));
+    float4 *const sTt = reinterpret_cast<float4 *>(__cvta_shared_to_generic(col_off));
 
     const Trans<float> tr = make_trans<float>(par[c], era ? era[t] : 0);
     const float cK = tr.c * tr.Kt;
@@ -160,7 +167,8 @@ k_sweep_y_cull(Landscape<float> ls, const int *__restrict__ perm, const mp_param
     uint32_t st_trips = 0, st_exec = 0, st_ret = 0, st_commit = 0;
 
     // sums of SP per-thread values over the task's TPT threads (warp shuffles, then st.async of the warp or CTA
-    // partials -- NV float4 per sender -- to every CTA of the cluster, completion counted on the destination's mbarrier)
+    // partials -- NV float4 per sender, one float2 with PAIR -- to every CTA of the cluster, completion counted on the
+    // destination's mbarrier)
     auto all_reduce = [&](int round, float (&v)[SP]) {
         const uint32_t u = uses[round]++;
         const int p = u & 1;
@@ -183,39 +191,66 @@ k_sweep_y_cull(Landscape<float> ls, const int *__restrict__ perm, const mp_param
             if (lane < nslot) t = base[lane * NV + q];
             return t;
         };
+        if constexpr (PAIR) {
+            // round 16 of the butterfly as a reduce-scatter: the low half-warp goes on adding v[0], the high half v[1].  Every
+            // node of the addition tree is one the full butterfly forms (IEEE addition commutes), so each low lane ends with
+            // the warp's v[0] sum and each high lane with its v[1] sum, bit for bit
+            const bool lo = lane < 16;
+            const float x = half_warp_sum_f((lo ? v[0] : v[1]) + __shfl_xor_sync(0xffffffffu, lo ? v[1] : v[0], 16));
+            const float2 part = make_float2(x, __shfl_xor_sync(0xffffffffu, x, 16));   // both sums in the low lanes
+            float2 *slots2 = reinterpret_cast<float2 *>(&red[0][0][0][0]) + (round * 2 + p) * 32;
+            if (CS > 1) {
+                const uint32_t boff = (uint32_t)(round * 2 + p) * 8u;
+                if (tid == 0) mbar_expect_tx(bar_local + boff, NSLOT * 8);
+                if (lane < CS) st_async_f32x2(red_remote + (uint32_t)((round * 2 + p) * 32 + (int)rank * NW + wid) * 8u, part, bar_remote + boff);
+                mbar_wait(bar_local + boff, (u >> 1) & 1u);
+            } else {
+                if (lane == 0) slots2[wid] = part;
+                __syncthreads();
+            }
+            // lane l adds up component l >> 4 of the senders' pairs.  With at most 16 senders the full butterfly's round 16 only
+            // added +0.0 here, which can change nothing but the sign of a zero sum, and no decision tells -0 from +0
+            float s = 0.f;
+            if (NSLOT == 16 || (lane & 15) < NSLOT) s = reinterpret_cast<const float *>(slots2)[2 * (lane & 15) + (lane >> 4)];
+            s = half_warp_sum_f(s);
+            const float o = __shfl_xor_sync(0xffffffffu, s, 16);
+            v[0] = lo ? s : o;
+            v[1] = lo ? o : s;
+        } else {
 #pragma unroll
-        for (int c = 0; c < SP; c++) v[c] = warp_sum_f(v[c]);
-        if (HIER) {
+            for (int c = 0; c < SP; c++) v[c] = warp_sum_f(v[c]);
+            if (HIER) {
+                if (lane == 0) {
+#pragma unroll
+                    for (int q = 0; q < NV; q++) wred[round][p][wid][q] = pack(q);
+                }
+                __syncthreads();
+#pragma unroll
+                for (int q = 0; q < NV; q++) unpack_sum(q, slot_of(&wred[round][p][0][0], NW, q));
+            }
+            if (CS > 1) {
+                const uint32_t boff = (uint32_t)(round * 2 + p) * 8u;
+                const uint32_t slot = HIER ? rank : rank * NW + wid;
+                const uint32_t roff = (uint32_t)(((round * 2 + p) * 32 + (int)slot) * NV) * 16u;
+                if (tid == 0) mbar_expect_tx(bar_local + boff, NSLOT * 16 * NV);
+                if (lane < CS && (!HIER || wid == 0)) {
+#pragma unroll
+                    for (int q = 0; q < NV; q++) st_async_f32x4(red_remote + roff + 16u * q, pack(q), bar_remote + boff);
+                }
+                mbar_wait(bar_local + boff, (u >> 1) & 1u);
+#pragma unroll
+                for (int q = 0; q < NV; q++) unpack_sum(q, slot_of(&red[round][p][0][0], NSLOT, q));
+                return;
+            }
+            if (HIER) return;
             if (lane == 0) {
 #pragma unroll
-                for (int q = 0; q < NV; q++) wred[round][p][wid][q] = pack(q);
+                for (int q = 0; q < NV; q++) red[round][p][wid][q] = pack(q);
             }
             __syncthreads();
 #pragma unroll
-            for (int q = 0; q < NV; q++) unpack_sum(q, slot_of(&wred[round][p][0][0], NW, q));
-        }
-        if (CS > 1) {
-            const uint32_t boff = (uint32_t)(round * 2 + p) * 8u;
-            const uint32_t slot = HIER ? rank : rank * NW + wid;
-            const uint32_t roff = (uint32_t)(((round * 2 + p) * 32 + (int)slot) * NV) * 16u;
-            if (tid == 0) mbar_expect_tx(bar_local + boff, NSLOT * 16 * NV);
-            if (lane < CS && (!HIER || wid == 0)) {
-#pragma unroll
-                for (int q = 0; q < NV; q++) st_async_f32x4(red_remote + roff + 16u * q, pack(q), bar_remote + boff);
-            }
-            mbar_wait(bar_local + boff, (u >> 1) & 1u);
-#pragma unroll
             for (int q = 0; q < NV; q++) unpack_sum(q, slot_of(&red[round][p][0][0], NSLOT, q));
-            return;
         }
-        if (HIER) return;
-        if (lane == 0) {
-#pragma unroll
-            for (int q = 0; q < NV; q++) red[round][p][wid][q] = pack(q);
-        }
-        __syncthreads();
-#pragma unroll
-        for (int q = 0; q < NV; q++) unpack_sum(q, slot_of(&red[round][p][0][0], NSLOT, q));
     };
     // weight of (candidate k, target in slot data tq)
     auto weight = [&](const float4 &tq, int k, float kx, float ky, float lawk) -> float {
@@ -233,7 +268,7 @@ k_sweep_y_cull(Landscape<float> ls, const int *__restrict__ perm, const mp_param
         return 1.001f * weight_of(nal2e, lawk, 0.99999f * dlow);     // sqrt.approx, ex2.approx: a few ulp each
     };
     auto own_term = [&](int kj, uint32_t cur) -> float {
-        const float4 tq = sT[tid + kj * NT];
+        const float4 tq = sTt[kj * NT];
         const float lg2e = 1.4426950408889634f;
         const float l0 = lg2e * tr.logE + Num<float>::lg2(__saturatef(cK * (tq.x + tq.y)));
         const float l1 = lg2e * tr.log1mE;
@@ -255,14 +290,7 @@ k_sweep_y_cull(Landscape<float> ls, const int *__restrict__ perm, const mp_param
         __syncthreads();
     }
     int chunk = 0;
-    struct Cand { int k; uint32_t cur; float kx, ky, lawk, thr; int kslot; };
-    auto read_cand = [&](int i) -> Cand {
-        const float4 a = ring[(i & (2 * RC - 1)) * 2], b = ring[(i & (2 * RC - 1)) * 2 + 1];
-        Cand cd;
-        cd.k = (int)(__float_as_uint(a.x) & 0x7fffffffu); cd.cur = __float_as_uint(a.x) >> 31;
-        cd.kx = a.y; cd.ky = a.z; cd.lawk = a.w; cd.thr = b.x; cd.kslot = blk ? (int)__float_as_uint(b.z) - slot_lo : (int)__float_as_uint(b.y);
-        return cd;
-    };
+    struct Cand { int k; uint32_t cur; float kx, ky, lawk; };
     auto bound_of = [&](int i) -> float {
         const float4 a = ring[(i & (2 * RC - 1)) * 2];
         return group_bound((int)(__float_as_uint(a.x) & 0x7fffffffu), a.y, a.z, a.w);
@@ -274,7 +302,7 @@ k_sweep_y_cull(Landscape<float> ls, const int *__restrict__ perm, const mp_param
         for (int j = 0; j < ept; j++) {
             const bool a = (Ae >> j) & 1u, b = (Be >> j) & 1u;
             if (!(a || b)) continue;
-            const float4 tq = sT[tid + j * NT];
+            const float4 tq = sTt[j * NT];
             const int s = g + j * TPT;
             const float w = weight(tq, cd.k, cd.kx, cd.ky, cd.lawk);
             const float sa = zero_after ? (float)src_offset(tl[s]) : fmaf(sgn, w, tq.x) + tq.y;
@@ -303,7 +331,7 @@ k_sweep_y_cull(Landscape<float> ls, const int *__restrict__ perm, const mp_param
                 int jj[B];
                 float4 tq[B];
 #pragma unroll
-                for (int u = 0; u < B; u++) { jj[u] = __ffs((int)m) - 1; m &= m - 1u; tq[u] = sT[tid + jj[u] * NT]; }
+                for (int u = 0; u < B; u++) { jj[u] = __ffs((int)m) - 1; m &= m - 1u; tq[u] = sTt[jj[u] * NT]; }
 #pragma unroll
                 for (int u = 0; u < B; u++) {
                     const int j = jj[u];
@@ -314,7 +342,7 @@ k_sweep_y_cull(Landscape<float> ls, const int *__restrict__ perm, const mp_param
                     const float lo2 = tq[u].y + e;
                     float hi = s + lo2, lo = lo2 - (hi - s);
                     if (hi < 0.f) { hi = 0.f; lo = 0.f; }
-                    *reinterpret_cast<float2 *>(&sT[tid + j * NT]) = make_float2(hi, lo);
+                    *reinterpret_cast<float2 *>(&sTt[j * NT]) = make_float2(hi, lo);
                     if (cd.cur) {
                         // a removal lowers S: exact new minimum of the group (S_hi >= 0, so the bit pattern is order
                         // preserving); after an addition the old minimum is still a lower bound
@@ -335,9 +363,9 @@ k_sweep_y_cull(Landscape<float> ls, const int *__restrict__ perm, const mp_param
                 int jj[B];
                 float4 tq[B];
 #pragma unroll
-                for (int u = 0; u < B; u++) { jj[u] = __ffs((int)mf) - 1; mf &= mf - 1u; tq[u] = sT[tid + jj[u] * NT]; }
+                for (int u = 0; u < B; u++) { jj[u] = __ffs((int)mf) - 1; mf &= mf - 1u; tq[u] = sTt[jj[u] * NT]; }
 #pragma unroll
-                for (int u = 0; u < B; u++) sT[tid + jj[u] * NT].y = fmaf(sgn, weight(tq[u], cd.k, cd.kx, cd.ky, cd.lawk), tq[u].y);
+                for (int u = 0; u < B; u++) sTt[jj[u] * NT].y = fmaf(sgn, weight(tq[u], cd.k, cd.kx, cd.ky, cd.lawk), tq[u].y);
             };
             while (mf) {                                  // warp-uniform; the candidate's own group is never far (distance 0)
                 const int left = __popc(mf);
@@ -351,7 +379,7 @@ k_sweep_y_cull(Landscape<float> ls, const int *__restrict__ perm, const mp_param
                 const int s = g + j * TPT;
                 const double so = s < nl ? src_offset(tl[s]) : 0.0;
                 const float hi = (float)so, lo = (float)(so - (double)hi);
-                *reinterpret_cast<float2 *>(&sT[tid + j * NT]) = make_float2(hi, lo);
+                *reinterpret_cast<float2 *>(&sTt[j * NT]) = make_float2(hi, lo);
             }
             Gw = 0.f;
         }
@@ -376,7 +404,7 @@ k_sweep_y_cull(Landscape<float> ls, const int *__restrict__ perm, const mp_param
             pre = load_chunk(chunk + 2);
         }
         const int nc = min(SP, ncand - i);
-        float kx[SP], ky[SP], lawk[SP], sgn[SP], pn[SP], acc[SP];
+        float kx[SP], ky[SP], lawk[SP], sgn[SP], thr[SP], pn[SP], acc[SP];
         int kj[SP], kk[SP];
         bool zero[SP];
         bool feel = false;
@@ -387,7 +415,7 @@ k_sweep_y_cull(Landscape<float> ls, const int *__restrict__ perm, const mp_param
             const int kslot = blk ? (int)__float_as_uint(rb.z) - slot_lo : (int)__float_as_uint(rb.y);
             const uint32_t cur = __float_as_uint(a.x) >> 31;
             kk[c] = (int)(__float_as_uint(a.x) & 0x7fffffffu);
-            kx[c] = a.y; ky[c] = a.z; lawk[c] = a.w; sgn[c] = cur ? -1.f : 1.f;
+            kx[c] = a.y; ky[c] = a.z; lawk[c] = a.w; sgn[c] = cur ? -1.f : 1.f; thr[c] = rb.x;
             kj[c] = (c < nc && (kslot % TPT) == g) ? kslot / TPT : 31;   // window entries past the list are zero records: no own cell
             zero[c] = (nocc + (cur ? -1 : 1)) == 0;
             pn[c] = 1.f; acc[c] = 0.f;
@@ -405,7 +433,7 @@ k_sweep_y_cull(Landscape<float> ls, const int *__restrict__ perm, const mp_param
             int jj[B];
             float4 tq[B];
 #pragma unroll
-            for (int u = 0; u < B; u++) { jj[u] = __ffs((int)m) - 1; m &= m - 1u; tq[u] = sT[tid + jj[u] * NT]; }
+            for (int u = 0; u < B; u++) { jj[u] = __ffs((int)m) - 1; m &= m - 1u; tq[u] = sTt[jj[u] * NT]; }
 #pragma unroll
             for (int u = 0; u < B; u++) {
                 const int j = jj[u];
@@ -441,24 +469,33 @@ k_sweep_y_cull(Landscape<float> ls, const int *__restrict__ perm, const mp_param
         for (int c = 0; c < SP; c++) nxt[c] = bound_of(i + SP + c);
         all_reduce(0, acc);
 
-        int adv = nc;
+        // decisions in order, from the window's registers; the accepted entry ca (if any) ends the window and is committed once
+        int adv = nc, ca = -1;
 #pragma unroll
         for (int c = 0; c < SP; c++) {
             if (c < adv) {                                // still undecided and inside the list (adv shrinks on the first accept)
-                const Cand cd = read_cand(i + c);
-                const bool own = kj[c] != 31;
-                const uint32_t bit = own ? 1u << kj[c] : 0u;
                 float tot = acc[c];
                 if (zero[c] || isnan(tot)) {
+                    const uint32_t bit = kj[c] != 31 ? 1u << kj[c] : 0u;
                     float v[SP];
 #pragma unroll
                     for (int d = 0; d < SP; d++) v[d] = 0.f;
-                    v[0] = evaluate_careful(cd, zero[c], own, kj[c], Amask & ~bit, Bmask);
+                    v[0] = evaluate_careful(Cand{ kk[c], sgn[c] < 0.f, kx[c], ky[c], lawk[c] }, zero[c], kj[c] != 31, kj[c], Amask & ~bit, Bmask);
                     all_reduce(1, v);
                     tot = v[0];
                 }
-                if (cd.thr < 0.6931471805599453f * tot) { commit(cd, wub[c], zero[c], own, kj[c], bit); adv = c + 1; }
+                if (thr[c] < 0.6931471805599453f * tot) { ca = c; adv = c + 1; }
             }
+        }
+        if (ca >= 0) {                                    // warp-uniform: every lane holds the task's sums
+            Cand cd{ kk[0], sgn[0] < 0.f, kx[0], ky[0], lawk[0] };
+            float wb = wub[0];
+            bool zr = zero[0];
+            int kjc = kj[0];
+#pragma unroll
+            for (int c = 1; c < SP; c++)
+                if (ca == c) { cd = Cand{ kk[c], sgn[c] < 0.f, kx[c], ky[c], lawk[c] }; wb = wub[c]; zr = zero[c]; kjc = kj[c]; }
+            commit(cd, wb, zr, kjc != 31, kjc, kjc != 31 ? 1u << kjc : 0u);
         }
         i += adv;
         st_trips++; st_exec += nfeel * (uint32_t)nc; st_ret += nfeel * (uint32_t)adv;

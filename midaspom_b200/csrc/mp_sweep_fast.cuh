@@ -87,6 +87,13 @@ __device__ __forceinline__ float warp_sum_f(float v)
     for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
     return v;
 }
+// rounds 8, 4, 2, 1 of warp_sum_f: the sum over each half-warp, formed by the same additions
+__device__ __forceinline__ float half_warp_sum_f(float v)
+{
+#pragma unroll
+    for (int o = 8; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+    return v;
+}
 
 // ------------------------------------------------------------------ candidate records
 // One CTA per (chain, transition): candidates in patch order, compacted by a block scan.
