@@ -527,6 +527,7 @@ int mp_create(const mp_config *cfg, mp_engine **out)
     if (const char *env = getenv("MP_CONN_SHAPE")) { const int v = atoi(env); if (v >= 0 && v <= 4) h->conn_shape = v; }
     if (const char *env = getenv("MP_REFRESH_EVERY")) { const int v = atoi(env); if (v >= 1) h->refresh_every = v; }
     if (const char *env = getenv("MP_FAST_CS")) { const int v = atoi(env); if (v == 1 || v == 2 || v == 4 || v == 8 || v == 16) h->fast_cs = v; }
+    if (const char *env = getenv("MP_CULL_BRANCH")) h->cull_branch = atoi(env) != 0;
     if (const char *env = getenv("MP_FAST_TPT")) { const int v = atoi(env); if (v == 128 || v == 256 || v == 512 || v == 1024 || v == 2048 || v == 4096 || v == 8192) h->fast_tpt = v; }
     if (const char *env = getenv("MP_GRAPH")) h->use_graph = atoi(env) != 0;
     if (const char *env = getenv("MP_BLK_TPT")) { const int v = atoi(env); if (v == 512 || v == 1024 || v == 2048 || v == 4096 || v == 8192) h->blk_tpt = v; }

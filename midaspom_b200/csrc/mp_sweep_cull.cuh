@@ -20,7 +20,14 @@
 //  * every trip evaluates SP consecutive candidates (the first and SP-1 speculative ones) in one pass over the union
 //    of their active groups and reduces the SP sums in ONE exchange: a rejected flip (2 of 3) costs no reduction
 //    latency of its own.  The decisions are exactly those of the one-at-a-time scan: a later candidate's sum is
-//    used only if every earlier one of the window left the state unchanged.
+//    used only if every earlier one of the window left the state unchanged;
+//  * BR (SP = 2 with at most 16 senders: every 512-thread task): a trip also forms a third sum, candidate i+1 GIVEN that i is
+//    accepted.  The state after i's commit differs only by +-w_i, which the pass already computes for every slot it visits:
+//    fn(fma(sgn_{i+1}, w_{i+1}, fma(sgn_i, w_i, S_hi)) + S_lo) over the post-commit denominator fn(fma(sgn_i, w_i, S_hi) + S_lo),
+//    which is candidate i's own numerator -- no weight is evaluated twice.  A trip thus retires both candidates whatever i's
+//    outcome (about 0.5 instead of 0.6 trips per candidate).  The branch sum stands for the exact post-commit evaluation up to
+//    ~ulp(S) on every S, i.e. up to FP32 ties, except under cancellation (a removal leaving less than S_hi/4 of a target, or the
+//    clamp at 0) and the careful cases: those poison it with NaN and defer i+1 to the next trip, as without the branch.
 #pragma once
 #include "mp_sweep_fast.cuh"
 
@@ -43,7 +50,7 @@ struct BlockTask { int task, tl_off, nl, slot_lo, slot_hi; };
 // CTAs of NT threads that should share an SM (registers: about 96 per thread)
 __host__ __device__ constexpr int cull_min_blocks(int nt) { return nt <= 32 ? 17 : nt <= 64 ? 9 : nt <= 128 ? 5 : nt <= 256 ? 2 : 1; }
 
-template <int GEOM, int CS, int TPT>
+template <int GEOM, int CS, int TPT, bool BR /* the "i+1 given i accepted" sum; PAIR shapes only (MP_CULL_BRANCH=0: off) */>
 __global__ void __launch_bounds__(TPT / CS, TPT > 1024 ? 1 : cull_min_blocks(TPT / CS))
 k_sweep_y_cull(Landscape<float> ls, const int *__restrict__ perm, const mp_params *__restrict__ par,
                const uint8_t *__restrict__ era, const uint8_t *__restrict__ z, uint8_t *__restrict__ y, double *__restrict__ S,
@@ -61,6 +68,8 @@ k_sweep_y_cull(Landscape<float> ls, const int *__restrict__ perm, const mp_param
     constexpr int NV = (SP + 3) / 4;                                 // float4 per sender in the exchange of the SP sums
     // two sums from at most 16 senders (every 512-thread task): reduce-scatter over the two half-warps, one float2 per sender
     constexpr bool PAIR = SP == 2 && !HIER && NSLOT <= 16;
+    static_assert(!BR || PAIR, "the branch sum exists for the PAIR shapes only");
+    constexpr int NS = SP + (BR ? 1 : 0);                            // sums exchanged per trip
     __shared__ __align__(16) float4 red[2][2][32][NV];
     __shared__ __align__(16) float4 wred[HIER ? 2 : 1][2][32][NV];
     __shared__ __align__(8) unsigned long long mbar[2][2];
@@ -169,7 +178,7 @@ k_sweep_y_cull(Landscape<float> ls, const int *__restrict__ perm, const mp_param
     // sums of SP per-thread values over the task's TPT threads (warp shuffles, then st.async of the warp or CTA
     // partials -- NV float4 per sender, one float2 with PAIR -- to every CTA of the cluster, completion counted on the
     // destination's mbarrier)
-    auto all_reduce = [&](int round, float (&v)[SP]) {
+    auto all_reduce = [&](int round, float (&v)[NS]) {
         const uint32_t u = uses[round]++;
         const int p = u & 1;
         auto pack = [&](int q) {
@@ -191,7 +200,41 @@ k_sweep_y_cull(Landscape<float> ls, const int *__restrict__ perm, const mp_param
             if (lane < nslot) t = base[lane * NV + q];
             return t;
         };
-        if constexpr (PAIR) {
+        if constexpr (BR) {
+            // three sums, one float4 {v0, v1, v2, 0} per sender: rounds 16 and 8 of the butterfly as a reduce-scatter, quarter-warp q
+            // going on adding v[q] (q = 3: zeros).  As with two sums below, every addition is one the full butterfly of that
+            // component forms (IEEE addition commutes), so each sum is bit for bit the full butterfly's, whatever the cluster split
+            const bool h16 = lane & 16, h8 = lane & 8;
+            const float a = (h16 ? v[2] : v[0]) + __shfl_xor_sync(0xffffffffu, h16 ? v[0] : v[2], 16);
+            const float b = (h16 ? 0.f : v[1]) + __shfl_xor_sync(0xffffffffu, h16 ? v[1] : 0.f, 16);
+            float x = (h8 ? b : a) + __shfl_xor_sync(0xffffffffu, h8 ? a : b, 8);
+#pragma unroll
+            for (int o = 4; o > 0; o >>= 1) x += __shfl_xor_sync(0xffffffffu, x, o);
+            // the senders (lanes < CS <= 8, quarter 0) gather the other quarters' sums
+            const float4 part = make_float4(x, __shfl_down_sync(0xffffffffu, x, 8), __shfl_down_sync(0xffffffffu, x, 16), 0.f);
+            float4 *slots4 = &red[round][p][0][0];
+            if (CS > 1) {
+                const uint32_t boff = (uint32_t)(round * 2 + p) * 8u;
+                if (tid == 0) mbar_expect_tx(bar_local + boff, NSLOT * 16);
+                if (lane < CS) st_async_f32x4(red_remote + (uint32_t)((round * 2 + p) * 32 + (int)rank * NW + wid) * 16u, part, bar_remote + boff);
+                mbar_wait(bar_local + boff, (u >> 1) & 1u);
+            } else {
+                if (lane == 0) slots4[wid] = part;
+                __syncthreads();
+            }
+            // second level: lane l adds component l >> 3 of senders l & 7 and (l & 7) + 8 -- round 8 of the butterfly over the
+            // senders (its round 16 only added +0.0) -- then rounds 4, 2, 1 within the quarter
+            const float *sf = reinterpret_cast<const float *>(slots4);
+            const int s = lane & 7, q = lane >> 3;
+            float y = 0.f;
+            if (NSLOT == 16 || s < NSLOT) y = sf[4 * s + q];
+            if (NSLOT == 16 || s + 8 < NSLOT) y += sf[4 * (s + 8) + q];
+#pragma unroll
+            for (int o = 4; o > 0; o >>= 1) y += __shfl_xor_sync(0xffffffffu, y, o);
+            v[0] = __shfl_sync(0xffffffffu, y, 0);
+            v[1] = __shfl_sync(0xffffffffu, y, 8);
+            v[2] = __shfl_sync(0xffffffffu, y, 16);
+        } else if constexpr (PAIR) {
             // round 16 of the butterfly as a reduce-scatter: the low half-warp goes on adding v[0], the high half v[1].  Every
             // node of the addition tree is one the full butterfly forms (IEEE addition commutes), so each low lane ends with
             // the warp's v[0] sum and each high lane with its v[1] sum, bit for bit
@@ -267,12 +310,16 @@ k_sweep_y_cull(Landscape<float> ls, const int *__restrict__ perm, const mp_param
         else dlow = ls.spacing * fmaxf(0.f, fmaxf(Gx - (float)k, (float)k - Gy));
         return 1.001f * weight_of(nal2e, lawk, 0.99999f * dlow);     // sqrt.approx, ex2.approx: a few ulp each
     };
-    auto own_term = [&](int kj, uint32_t cur) -> float {
-        const float4 tq = sTt[kj * NT];
+    // the flip's own cell, whose connectivity is s
+    auto own_term_s = [&](float s, uint32_t cur) -> float {
         const float lg2e = 1.4426950408889634f;
-        const float l0 = lg2e * tr.logE + Num<float>::lg2(__saturatef(cK * (tq.x + tq.y)));
+        const float l0 = lg2e * tr.logE + Num<float>::lg2(__saturatef(cK * s));
         const float l1 = lg2e * tr.log1mE;
         return cur ? ldiff<float>(l0, l1) : ldiff<float>(l1, l0);
+    };
+    auto own_term = [&](int kj, uint32_t cur) -> float {
+        const float4 tq = sTt[kj * NT];
+        return own_term_s(tq.x + tq.y, cur);
     };
 
     // ---- candidate records travel through a two-chunk ring in shared memory (chunks c and c+1 resident while i is in chunk c)
@@ -404,7 +451,7 @@ k_sweep_y_cull(Landscape<float> ls, const int *__restrict__ perm, const mp_param
             pre = load_chunk(chunk + 2);
         }
         const int nc = min(SP, ncand - i);
-        float kx[SP], ky[SP], lawk[SP], sgn[SP], thr[SP], pn[SP], acc[SP];
+        float kx[SP], ky[SP], lawk[SP], sgn[SP], thr[SP], pn[SP], acc[NS];
         int kj[SP], kk[SP];
         bool zero[SP];
         bool feel = false;
@@ -427,6 +474,12 @@ k_sweep_y_cull(Landscape<float> ls, const int *__restrict__ perm, const mp_param
         const uint32_t nfeel = __popc(m);
         float pd = 1.f;
         int cnt = 0;
+        // BR: product of the branch factors, and the cancellation cut of candidate 0 (a removal that leaves u0 = fl(S_hi - w0) below
+        // S_hi / 4; an addition never cancels).  Above the cut u0 + S_lo is within ~2^-23 of S_hi + S_lo - w0 relative to itself
+        // (|S_lo| < 2^-13 S_hi), the accuracy of the post-commit evaluation; below it S_lo and the commit's clamp at 0 matter
+        float pn2 = 1.f;
+        const float cut0 = sgn[0] < 0.f ? 0.25f : -1.f;
+        if constexpr (BR) acc[SP] = 0.f;
         // B slots x SP candidates per trip: B * SP independent (sqrt, ex2, FFMA.SAT) chains
         auto slots = [&](auto BB) {
             constexpr int B = decltype(BB)::value;
@@ -442,11 +495,23 @@ k_sweep_y_cull(Landscape<float> ls, const int *__restrict__ perm, const mp_param
                 const float mul = a ? cK : (b ? -cK : 0.f), add = a ? 0.f : 1.f;
                 const float fd = __saturatef(fmaf(mul, tq[u].x + tq[u].y, add));
                 pd *= fd;
+                float u0 = 0.f, fn0 = 1.f, w1 = 0.f;
 #pragma unroll
                 for (int c = 0; c < SP; c++) {
                     const float w = weight(tq[u], kk[c], kx[c], ky[c], lawk[c]);
-                    const float fn = __saturatef(fmaf(mul, fmaf(sgn[c], w, tq[u].x) + tq[u].y, add));
+                    const float uc = fmaf(sgn[c], w, tq[u].x);
+                    const float fn = __saturatef(fmaf(mul, uc + tq[u].y, add));
                     pn[c] *= j == kj[c] ? fd : fn;        // the candidate's own cell is handled by own_term
+                    if (c == 0) { u0 = uc; fn0 = fn; }
+                    if (c == 1) w1 = w;
+                }
+                if constexpr (BR) {
+                    // candidate 1 after candidate 0's commit: numerator fn(S + sgn0 w0 + sgn1 w1); the denominator fn(S + sgn0 w0) is fn0,
+                    // already in pn[0].  At candidate 0's own cell (S unchanged, class flipped) and at candidate 1's own cell the
+                    // factors cancel, the owners add those cells' terms after the loop
+                    const float f2 = u0 < cut0 * tq[u].x ? __int_as_float(0x7fffffff)
+                                                         : __saturatef(fmaf(mul, fmaf(sgn[1], w1, u0) + tq[u].y, add));
+                    pn2 *= j == kj[0] ? fd : (j == kj[1] ? fn0 : f2);
                 }
             }
             cnt += B;
@@ -456,46 +521,94 @@ k_sweep_y_cull(Landscape<float> ls, const int *__restrict__ perm, const mp_param
             else slots(std::integral_constant<int, 1>());
             if (cnt >= 4 || m == 0u) {                    // products of at most 4 factors stay far from underflow
                 const float lpd = Num<float>::lg2(pd);
+                float lpn[SP];
 #pragma unroll
-                for (int c = 0; c < SP; c++) { acc[c] += Num<float>::lg2(pn[c]) - lpd; pn[c] = 1.f; }
+                for (int c = 0; c < SP; c++) { lpn[c] = Num<float>::lg2(pn[c]); acc[c] += lpn[c] - lpd; pn[c] = 1.f; }
+                if constexpr (BR) { acc[SP] += Num<float>::lg2(pn2) - lpn[0]; pn2 = 1.f; }
                 pd = 1.f; cnt = 0;
             }
         }
 #pragma unroll
         for (int c = 0; c < SP; c++) if (kj[c] != 31) acc[c] += own_term(kj[c], sgn[c] < 0.f);
+        if constexpr (BR) {
+            if (kj[1] != 31) {                            // candidate 1's own cell, S after candidate 0's commit (same cut)
+                const float4 tq = sTt[kj[1] * NT];
+                const float u = fmaf(sgn[0], weight(tq, kk[0], kx[0], ky[0], lawk[0]), tq.x);
+                acc[SP] += u < cut0 * tq.x ? __int_as_float(0x7fffffff) : own_term_s(u + tq.y, sgn[1] < 0.f);
+            }
+            if (kj[0] != 31 && sgn[0] < 0.f) {            // candidate 0's own cell: its removal makes it class A with S unchanged
+                const float4 tq = sTt[kj[0] * NT];
+                const float w = weight(tq, kk[1], kx[1], ky[1], lawk[1]);
+                acc[SP] += Num<float>::lg2(__saturatef(cK * (fmaf(sgn[1], w, tq.x) + tq.y))) - Num<float>::lg2(__saturatef(cK * (tq.x + tq.y)));
+            }
+        }
         // bounds of the SP candidates after this window: independent of this trip's outcome, they complete under the reduction
         float nxt[SP];
 #pragma unroll
         for (int c = 0; c < SP; c++) nxt[c] = bound_of(i + SP + c);
         all_reduce(0, acc);
 
-        // decisions in order, from the window's registers; the accepted entry ca (if any) ends the window and is committed once
-        int adv = nc, ca = -1;
+        int adv = nc;
+        if constexpr (BR) {
+            // candidate 0 as below; candidate 1 from its own sum if 0 is rejected, from the branch sum if 0 is accepted.  The branch
+            // is deferred (adv = 1) when it is NaN (cut, or a zero factor), when candidate 0 took the careful path, and when
+            // candidate 1 would take it with or without 0's flip (the last occupied patch leaving)
+            bool take[SP];
 #pragma unroll
-        for (int c = 0; c < SP; c++) {
-            if (c < adv) {                                // still undecided and inside the list (adv shrinks on the first accept)
+            for (int c = 0; c < SP; c++) {
+                take[c] = false;
+                if (c >= nc) continue;
                 float tot = acc[c];
-                if (zero[c] || isnan(tot)) {
+                if (c == 1 && take[0]) {
+                    tot = acc[SP];
+                    const bool ok = !zero[0] && !isnan(acc[0]) && !zero[1] && nocc + (sgn[0] < 0.f ? -1 : 1) + (sgn[1] < 0.f ? -1 : 1) != 0;
+                    if (!ok || isnan(tot)) { adv = 1; continue; }
+                } else if (zero[c] || isnan(tot)) {
                     const uint32_t bit = kj[c] != 31 ? 1u << kj[c] : 0u;
-                    float v[SP];
-#pragma unroll
-                    for (int d = 0; d < SP; d++) v[d] = 0.f;
+                    float v[NS] = {};
                     v[0] = evaluate_careful(Cand{ kk[c], sgn[c] < 0.f, kx[c], ky[c], lawk[c] }, zero[c], kj[c] != 31, kj[c], Amask & ~bit, Bmask);
                     all_reduce(1, v);
                     tot = v[0];
                 }
-                if (thr[c] < 0.6931471805599453f * tot) { ca = c; adv = c + 1; }
+                take[c] = thr[c] < 0.6931471805599453f * tot;
             }
-        }
-        if (ca >= 0) {                                    // warp-uniform: every lane holds the task's sums
-            Cand cd{ kk[0], sgn[0] < 0.f, kx[0], ky[0], lawk[0] };
-            float wb = wub[0];
-            bool zr = zero[0];
-            int kjc = kj[0];
+            // commits in order, one inlined copy of the commit (warp-uniform)
+#pragma unroll 1
+            for (int c = 0; c < SP; c++) {
+                if (!(c ? take[1] : take[0])) continue;
+                const int kjc = c ? kj[1] : kj[0];
+                commit(c ? Cand{ kk[1], sgn[1] < 0.f, kx[1], ky[1], lawk[1] } : Cand{ kk[0], sgn[0] < 0.f, kx[0], ky[0], lawk[0] },
+                       c ? wub[1] : wub[0], c ? zero[1] : zero[0], kjc != 31, kjc, kjc != 31 ? 1u << kjc : 0u);
+            }
+        } else {
+            // decisions in order, from the window's registers; the accepted entry ca (if any) ends the window and is committed once
+            int ca = -1;
 #pragma unroll
-            for (int c = 1; c < SP; c++)
-                if (ca == c) { cd = Cand{ kk[c], sgn[c] < 0.f, kx[c], ky[c], lawk[c] }; wb = wub[c]; zr = zero[c]; kjc = kj[c]; }
-            commit(cd, wb, zr, kjc != 31, kjc, kjc != 31 ? 1u << kjc : 0u);
+            for (int c = 0; c < SP; c++) {
+                if (c < adv) {                                // still undecided and inside the list (adv shrinks on the first accept)
+                    float tot = acc[c];
+                    if (zero[c] || isnan(tot)) {
+                        const uint32_t bit = kj[c] != 31 ? 1u << kj[c] : 0u;
+                        float v[SP];
+#pragma unroll
+                        for (int d = 0; d < SP; d++) v[d] = 0.f;
+                        v[0] = evaluate_careful(Cand{ kk[c], sgn[c] < 0.f, kx[c], ky[c], lawk[c] }, zero[c], kj[c] != 31, kj[c], Amask & ~bit, Bmask);
+                        all_reduce(1, v);
+                        tot = v[0];
+                    }
+                    if (thr[c] < 0.6931471805599453f * tot) { ca = c; adv = c + 1; }
+                }
+            }
+            if (ca >= 0) {                                    // warp-uniform: every lane holds the task's sums
+                Cand cd{ kk[0], sgn[0] < 0.f, kx[0], ky[0], lawk[0] };
+                float wb = wub[0];
+                bool zr = zero[0];
+                int kjc = kj[0];
+#pragma unroll
+                for (int c = 1; c < SP; c++)
+                    if (ca == c) { cd = Cand{ kk[c], sgn[c] < 0.f, kx[c], ky[c], lawk[c] }; wb = wub[c]; zr = zero[c]; kjc = kj[c]; }
+                commit(cd, wb, zr, kjc != 31, kjc, kjc != 31 ? 1u << kjc : 0u);
+            }
         }
         i += adv;
         st_trips++; st_exec += nfeel * (uint32_t)nc; st_ret += nfeel * (uint32_t)adv;
@@ -558,12 +671,12 @@ k_block_valid(const double *__restrict__ S, const mp_params *__restrict__ par, c
 #if defined(MP_FAST_GEOM) && defined(MP_FAST_HAS_POSITIONS)
 namespace mp {
 // nclusters whole (chain, year) tasks (btasks == nullptr) or block tasks of one colour
-template <int CS, int TPT> static int launch_cull(mp_engine *h, int ept, int nclusters, const BlockTask *btasks)
+template <int CS, int TPT, bool BR> static int launch_cull(mp_engine *h, int ept, int nclusters, const BlockTask *btasks)
 {
     constexpr int NT = TPT / CS;
     const size_t smem = (size_t)ept * NT * 16 + 2 * 32 * 32;   // targets + the two-chunk record ring
     REQUIRE(smem <= 227 * 1024 && ept <= 31, MP_ERR_UNSUPPORTED, "n_patches too large for the fast y sweep");
-    auto kern = k_sweep_y_cull<MP_FAST_GEOM, CS, TPT>;
+    auto kern = k_sweep_y_cull<MP_FAST_GEOM, CS, TPT, BR>;
     CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     if (CS > 8) CK(cudaFuncSetAttribute(kern, cudaFuncAttributeNonPortableClusterSizeAllowed, 1));
     if (nclusters <= 0) return MP_OK;
@@ -582,26 +695,31 @@ template <int CS, int TPT> static int launch_cull(mp_engine *h, int ept, int ncl
                           h->d_work, btasks, (const int *)h->d_tlist, (const int *)(h->blk_active ? h->d_blockmode : nullptr)));
     return MP_OK;
 }
+// 512 threads per task: with or without the branch sum (h->cull_branch, MP_CULL_BRANCH)
+template <int CS> static int launch_cull_512(mp_engine *h, int ept, int nclusters, const BlockTask *btasks)
+{
+    return h->cull_branch ? launch_cull<CS, 512, true>(h, ept, nclusters, btasks) : launch_cull<CS, 512, false>(h, ept, nclusters, btasks);
+}
 // culled variants exist for 512 and 1024 threads per task (up to 31 slots per thread) and the large-landscape geometries
 static int launch_cull_any(mp_engine *h, int cs, int tpt, int nl_max, int nclusters, const void *btasks_v)
 {
     const BlockTask *btasks = (const BlockTask *)btasks_v;
     const int ept = (nl_max + tpt - 1) / tpt;
     if (tpt == 512) switch (cs) {
-        case 1: return launch_cull<1, 512>(h, ept, nclusters, btasks);
-        case 2: return launch_cull<2, 512>(h, ept, nclusters, btasks);
-        case 4: return launch_cull<4, 512>(h, ept, nclusters, btasks);
-        default: return launch_cull<8, 512>(h, ept, nclusters, btasks);
+        case 1: return launch_cull_512<1>(h, ept, nclusters, btasks);
+        case 2: return launch_cull_512<2>(h, ept, nclusters, btasks);
+        case 4: return launch_cull_512<4>(h, ept, nclusters, btasks);
+        default: return launch_cull_512<8>(h, ept, nclusters, btasks);
     }
     if (tpt == 1024) switch (cs) {
-        case 1: return launch_cull<1, 1024>(h, ept, nclusters, btasks);
-        case 2: return launch_cull<2, 1024>(h, ept, nclusters, btasks);
-        case 4: return launch_cull<4, 1024>(h, ept, nclusters, btasks);
-        default: return launch_cull<8, 1024>(h, ept, nclusters, btasks);
+        case 1: return launch_cull<1, 1024, false>(h, ept, nclusters, btasks);
+        case 2: return launch_cull<2, 1024, false>(h, ept, nclusters, btasks);
+        case 4: return launch_cull<4, 1024, false>(h, ept, nclusters, btasks);
+        default: return launch_cull<8, 1024, false>(h, ept, nclusters, btasks);
     }
-    if (tpt == 2048) return launch_cull<8, 2048>(h, ept, nclusters, btasks);
-    if (tpt == 4096) return cs == 16 ? launch_cull<16, 4096>(h, ept, nclusters, btasks) : launch_cull<8, 4096>(h, ept, nclusters, btasks);
-    if (tpt == 8192) return cs == 16 ? launch_cull<16, 8192>(h, ept, nclusters, btasks) : launch_cull<8, 8192>(h, ept, nclusters, btasks);
+    if (tpt == 2048) return launch_cull<8, 2048, false>(h, ept, nclusters, btasks);
+    if (tpt == 4096) return cs == 16 ? launch_cull<16, 4096, false>(h, ept, nclusters, btasks) : launch_cull<8, 4096, false>(h, ept, nclusters, btasks);
+    if (tpt == 8192) return cs == 16 ? launch_cull<16, 8192, false>(h, ept, nclusters, btasks) : launch_cull<8, 8192, false>(h, ept, nclusters, btasks);
     return MP_ERR_UNSUPPORTED;
 }
 }  // namespace mp
