@@ -240,7 +240,7 @@ int mp_get_timing(mp_engine *h, double *ms, int64_t *launches, int reset);
 /* Work actually executed by the hot kernels since the last reset (always on: warp-local counts, one atomic per warp and
  * launch).  Used by bench.py so that roofline fractions count executed work, not the dense algorithm's:
  *   MP_CNT_SCAN_TRIPS    warp-trips of the culled y scan (one trip = one exchange of SP candidate sums; with the branch sum of
- *                        the 512-thread tasks, MP_CULL_BRANCH, the exchange also carries "candidate 2 given candidate 1 accepted")
+ *                        the 512-thread tasks, the exchange also carries "candidate 2 given candidate 1 accepted")
  *   MP_CNT_SCAN_EXEC     (candidate, group of 32 targets) evaluations executed, speculative ones included; the branch sum
  *                        evaluates no weights of its own and adds nothing here
  *   MP_CNT_SCAN_RETIRED  the part of MP_CNT_SCAN_EXEC that belongs to candidates decided in their trip (with the branch sum:

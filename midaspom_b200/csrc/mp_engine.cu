@@ -221,7 +221,7 @@ static int launch_sweep_y_fast(mp_engine *h)
     // task over 16 SMs instead -- the scan is latency-bound per flip
     const int ntask_own = (C * ntrans - h->task_first + h->task_stride - 1) / h->task_stride;
     // exact spatial culling of the evaluation (mp_sweep_cull.cuh) where positions exist and the landscape is large
-    const bool culled = h->fast_cull && h->geom != MP_GEOM_DENSE && tpt >= 512;
+    const bool culled = h->geom != MP_GEOM_DENSE && tpt >= 512;
     // the culled scan at 512 threads per task runs in clusters of 4 x 128 threads whatever the task count: up to five such CTAs
     // of different tasks share an SM, and their independent trips cover each other's latency.  Measured at cfg3 (one B200,
     // 1,000 W), ms per launch for CS = 1 / 2 / 4 / 8: 64 chains 60.1 / 60.2 / 56.2 / 62.8, 32 chains 32.1 / 32.3 / 29.4 / 32.9,
@@ -519,7 +519,6 @@ int mp_create(const mp_config *cfg, mp_engine **out)
     }
     mp_engine *h = new mp_engine();
     h->cfg = *cfg;
-    if (const char *env = getenv("MP_FAST_CULL")) h->fast_cull = atoi(env) != 0;
     if (const char *env = getenv("MP_CONN_CULL")) h->conn_cull = atoi(env) != 0;
     if (const char *env = getenv("MP_CONN_GEMM")) h->use_gemm = atoi(env) != 0;
     if (const char *env = getenv("MP_CONN_GEMM_MIN_N")) { const int v = atoi(env); if (v >= 1) h->gemm_min_n = v; }
@@ -527,7 +526,6 @@ int mp_create(const mp_config *cfg, mp_engine **out)
     if (const char *env = getenv("MP_CONN_SHAPE")) { const int v = atoi(env); if (v >= 0 && v <= 4) h->conn_shape = v; }
     if (const char *env = getenv("MP_REFRESH_EVERY")) { const int v = atoi(env); if (v >= 1) h->refresh_every = v; }
     if (const char *env = getenv("MP_FAST_CS")) { const int v = atoi(env); if (v == 1 || v == 2 || v == 4 || v == 8 || v == 16) h->fast_cs = v; }
-    if (const char *env = getenv("MP_CULL_BRANCH")) h->cull_branch = atoi(env) != 0;
     if (const char *env = getenv("MP_FAST_TPT")) { const int v = atoi(env); if (v == 128 || v == 256 || v == 512 || v == 1024 || v == 2048 || v == 4096 || v == 8192) h->fast_tpt = v; }
     if (const char *env = getenv("MP_GRAPH")) h->use_graph = atoi(env) != 0;
     if (const char *env = getenv("MP_BLK_TPT")) { const int v = atoi(env); if (v == 512 || v == 1024 || v == 2048 || v == 4096 || v == 8192) h->blk_tpt = v; }

@@ -76,9 +76,7 @@ struct mp_engine {
     int *d_task_order = nullptr;               // scan tasks of this engine, longest first (k_order_tasks)
     int *d_perm = nullptr;                     // layout (Morton) order of the patches: perm[slot] = patch
     int *d_scan = nullptr, *d_minv = nullptr;  // visiting order of the y scan (position -> patch; = perm without a scan grid); patch -> layout slot
-    int fast_cull = 1;               // exact spatial culling in the fast sweep (MP_FAST_CULL=0 disables)
     int fast_cs = 0;                 // cluster size of the fast sweep (0 = choose); MP_FAST_CS overrides
-    int cull_branch = 1;             // culled scan at 512 threads: decide candidate i+1 given i accepted in the same trip (MP_CULL_BRANCH=0: off)
     int fast_tpt = 0;                // threads per task of the fast sweep (0 = choose from N); MP_FAST_TPT overrides
     // block grid of the y scan (landscapes with coordinates; mp_set_scan_blocks): blk_nx x blk_ny cells, blk_k x blk_k colours
     int blk_nx = 1, blk_ny = 1, blk_k = 1;

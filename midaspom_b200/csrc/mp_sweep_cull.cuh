@@ -21,26 +21,23 @@
 //    of their active groups and reduces the SP sums in ONE exchange: a rejected flip (2 of 3) costs no reduction
 //    latency of its own.  The decisions are exactly those of the one-at-a-time scan: a later candidate's sum is
 //    used only if every earlier one of the window left the state unchanged;
-//  * BR (SP = 2 with at most 16 senders: every 512-thread task): a trip also forms a third sum, candidate i+1 GIVEN that i is
-//    accepted.  The state after i's commit differs only by +-w_i, which the pass already computes for every slot it visits:
+//  * BR (SP = 2 with at most 16 senders: how every 512-thread task, whole-year or block, runs): a trip also forms a third sum,
+//    candidate i+1 GIVEN that i is accepted.  The state after i's commit differs only by +-w_i, which the pass already computes
+//    for every slot it visits:
 //    fn(fma(sgn_{i+1}, w_{i+1}, fma(sgn_i, w_i, S_hi)) + S_lo) over the post-commit denominator fn(fma(sgn_i, w_i, S_hi) + S_lo),
 //    which is candidate i's own numerator -- no weight is evaluated twice.  A trip thus retires both candidates whatever i's
 //    outcome (about 0.5 instead of 0.6 trips per candidate).  The branch sum stands for the exact post-commit evaluation up to
 //    ~ulp(S) on every S, i.e. up to FP32 ties, except under cancellation (a removal leaving less than S_hi/4 of a target, or the
-//    clamp at 0) and the careful cases: those poison it with NaN and defer i+1 to the next trip, as without the branch.
+//    clamp at 0) and the careful cases: those poison it with NaN and defer i+1 to the next trip.
 #pragma once
 #include "mp_sweep_fast.cuh"
 
+namespace mp {
+
 // candidates evaluated per trip (1 + speculative ones), measured: cfg3 (512 threads per task) 10.0 / 10.4 / 11.1 ms for 2 / 3 / 4,
 // cfg5t (4096 threads per task, exchange-latency bound) 43.4 / 39.3 / 38.3 ms (6: 42.9, 8: 51.3)
-#ifndef MP_CULL_SPEC
-#define MP_CULL_SPEC 2
-#endif
-#ifndef MP_CULL_SPEC_LARGE
-#define MP_CULL_SPEC_LARGE 4
-#endif
-
-namespace mp {
+constexpr int MP_CULL_SPEC = 2;
+constexpr int MP_CULL_SPEC_LARGE = 4;
 
 // One unit of work of a block launch: the candidates of one block of the scan grid in one (chain, year) task, with the
 // block's own patches and every patch within the halo around it as targets (mp_set_scan_blocks).  Blocks of one colour
@@ -50,7 +47,7 @@ struct BlockTask { int task, tl_off, nl, slot_lo, slot_hi; };
 // CTAs of NT threads that should share an SM (registers: about 96 per thread)
 __host__ __device__ constexpr int cull_min_blocks(int nt) { return nt <= 32 ? 17 : nt <= 64 ? 9 : nt <= 128 ? 5 : nt <= 256 ? 2 : 1; }
 
-template <int GEOM, int CS, int TPT, bool BR /* the "i+1 given i accepted" sum; PAIR shapes only (MP_CULL_BRANCH=0: off) */>
+template <int GEOM, int CS, int TPT>
 __global__ void __launch_bounds__(TPT / CS, TPT > 1024 ? 1 : cull_min_blocks(TPT / CS))
 k_sweep_y_cull(Landscape<float> ls, const int *__restrict__ perm, const mp_params *__restrict__ par,
                const uint8_t *__restrict__ era, const uint8_t *__restrict__ z, uint8_t *__restrict__ y, double *__restrict__ S,
@@ -66,9 +63,8 @@ k_sweep_y_cull(Landscape<float> ls, const int *__restrict__ perm, const mp_param
     constexpr int NSLOT = HIER ? CS : TPT / 32;
     extern __shared__ __align__(16) unsigned char smem_raw[];
     constexpr int NV = (SP + 3) / 4;                                 // float4 per sender in the exchange of the SP sums
-    // two sums from at most 16 senders (every 512-thread task): reduce-scatter over the two half-warps, one float2 per sender
-    constexpr bool PAIR = SP == 2 && !HIER && NSLOT <= 16;
-    static_assert(!BR || PAIR, "the branch sum exists for the PAIR shapes only");
+    // the "i+1 given i accepted" sum: two candidates from at most 16 senders (every 512-thread task)
+    constexpr bool BR = SP == 2 && !HIER && NSLOT <= 16;
     constexpr int NS = SP + (BR ? 1 : 0);                            // sums exchanged per trip
     __shared__ __align__(16) float4 red[2][2][32][NV];
     __shared__ __align__(16) float4 wred[HIER ? 2 : 1][2][32][NV];
@@ -175,8 +171,8 @@ k_sweep_y_cull(Landscape<float> ls, const int *__restrict__ perm, const mp_param
     // 32-target group) evaluations executed, the part of them that belongs to retired candidates, groups committed
     uint32_t st_trips = 0, st_exec = 0, st_ret = 0, st_commit = 0;
 
-    // sums of SP per-thread values over the task's TPT threads (warp shuffles, then st.async of the warp or CTA
-    // partials -- NV float4 per sender, one float2 with PAIR -- to every CTA of the cluster, completion counted on the
+    // sums of NS per-thread values over the task's TPT threads (warp shuffles, then st.async of the warp or CTA
+    // partials -- NV float4 per sender, one float4 with BR -- to every CTA of the cluster, completion counted on the
     // destination's mbarrier)
     auto all_reduce = [&](int round, float (&v)[NS]) {
         const uint32_t u = uses[round]++;
@@ -202,8 +198,8 @@ k_sweep_y_cull(Landscape<float> ls, const int *__restrict__ perm, const mp_param
         };
         if constexpr (BR) {
             // three sums, one float4 {v0, v1, v2, 0} per sender: rounds 16 and 8 of the butterfly as a reduce-scatter, quarter-warp q
-            // going on adding v[q] (q = 3: zeros).  As with two sums below, every addition is one the full butterfly of that
-            // component forms (IEEE addition commutes), so each sum is bit for bit the full butterfly's, whatever the cluster split
+            // going on adding v[q] (q = 3: zeros).  Every addition is one the full butterfly of that component forms (IEEE addition
+            // commutes), so each sum is bit for bit the full butterfly's, whatever the cluster split
             const bool h16 = lane & 16, h8 = lane & 8;
             const float a = (h16 ? v[2] : v[0]) + __shfl_xor_sync(0xffffffffu, h16 ? v[0] : v[2], 16);
             const float b = (h16 ? 0.f : v[1]) + __shfl_xor_sync(0xffffffffu, h16 ? v[1] : 0.f, 16);
@@ -223,7 +219,8 @@ k_sweep_y_cull(Landscape<float> ls, const int *__restrict__ perm, const mp_param
                 __syncthreads();
             }
             // second level: lane l adds component l >> 3 of senders l & 7 and (l & 7) + 8 -- round 8 of the butterfly over the
-            // senders (its round 16 only added +0.0) -- then rounds 4, 2, 1 within the quarter
+            // senders (its round 16 only added +0.0, which can change nothing but the sign of a zero sum, and no decision tells
+            // -0 from +0) -- then rounds 4, 2, 1 within the quarter
             const float *sf = reinterpret_cast<const float *>(slots4);
             const int s = lane & 7, q = lane >> 3;
             float y = 0.f;
@@ -234,31 +231,6 @@ k_sweep_y_cull(Landscape<float> ls, const int *__restrict__ perm, const mp_param
             v[0] = __shfl_sync(0xffffffffu, y, 0);
             v[1] = __shfl_sync(0xffffffffu, y, 8);
             v[2] = __shfl_sync(0xffffffffu, y, 16);
-        } else if constexpr (PAIR) {
-            // round 16 of the butterfly as a reduce-scatter: the low half-warp goes on adding v[0], the high half v[1].  Every
-            // node of the addition tree is one the full butterfly forms (IEEE addition commutes), so each low lane ends with
-            // the warp's v[0] sum and each high lane with its v[1] sum, bit for bit
-            const bool lo = lane < 16;
-            const float x = half_warp_sum_f((lo ? v[0] : v[1]) + __shfl_xor_sync(0xffffffffu, lo ? v[1] : v[0], 16));
-            const float2 part = make_float2(x, __shfl_xor_sync(0xffffffffu, x, 16));   // both sums in the low lanes
-            float2 *slots2 = reinterpret_cast<float2 *>(&red[0][0][0][0]) + (round * 2 + p) * 32;
-            if (CS > 1) {
-                const uint32_t boff = (uint32_t)(round * 2 + p) * 8u;
-                if (tid == 0) mbar_expect_tx(bar_local + boff, NSLOT * 8);
-                if (lane < CS) st_async_f32x2(red_remote + (uint32_t)((round * 2 + p) * 32 + (int)rank * NW + wid) * 8u, part, bar_remote + boff);
-                mbar_wait(bar_local + boff, (u >> 1) & 1u);
-            } else {
-                if (lane == 0) slots2[wid] = part;
-                __syncthreads();
-            }
-            // lane l adds up component l >> 4 of the senders' pairs.  With at most 16 senders the full butterfly's round 16 only
-            // added +0.0 here, which can change nothing but the sign of a zero sum, and no decision tells -0 from +0
-            float s = 0.f;
-            if (NSLOT == 16 || (lane & 15) < NSLOT) s = reinterpret_cast<const float *>(slots2)[2 * (lane & 15) + (lane >> 4)];
-            s = half_warp_sum_f(s);
-            const float o = __shfl_xor_sync(0xffffffffu, s, 16);
-            v[0] = lo ? s : o;
-            v[1] = lo ? o : s;
         } else {
 #pragma unroll
             for (int c = 0; c < SP; c++) v[c] = warp_sum_f(v[c]);
@@ -671,12 +643,12 @@ k_block_valid(const double *__restrict__ S, const mp_params *__restrict__ par, c
 #if defined(MP_FAST_GEOM) && defined(MP_FAST_HAS_POSITIONS)
 namespace mp {
 // nclusters whole (chain, year) tasks (btasks == nullptr) or block tasks of one colour
-template <int CS, int TPT, bool BR> static int launch_cull(mp_engine *h, int ept, int nclusters, const BlockTask *btasks)
+template <int CS, int TPT> static int launch_cull(mp_engine *h, int ept, int nclusters, const BlockTask *btasks)
 {
     constexpr int NT = TPT / CS;
     const size_t smem = (size_t)ept * NT * 16 + 2 * 32 * 32;   // targets + the two-chunk record ring
     REQUIRE(smem <= 227 * 1024 && ept <= 31, MP_ERR_UNSUPPORTED, "n_patches too large for the fast y sweep");
-    auto kern = k_sweep_y_cull<MP_FAST_GEOM, CS, TPT, BR>;
+    auto kern = k_sweep_y_cull<MP_FAST_GEOM, CS, TPT>;
     CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     if (CS > 8) CK(cudaFuncSetAttribute(kern, cudaFuncAttributeNonPortableClusterSizeAllowed, 1));
     if (nclusters <= 0) return MP_OK;
@@ -695,31 +667,26 @@ template <int CS, int TPT, bool BR> static int launch_cull(mp_engine *h, int ept
                           h->d_work, btasks, (const int *)h->d_tlist, (const int *)(h->blk_active ? h->d_blockmode : nullptr)));
     return MP_OK;
 }
-// 512 threads per task: with or without the branch sum (h->cull_branch, MP_CULL_BRANCH)
-template <int CS> static int launch_cull_512(mp_engine *h, int ept, int nclusters, const BlockTask *btasks)
-{
-    return h->cull_branch ? launch_cull<CS, 512, true>(h, ept, nclusters, btasks) : launch_cull<CS, 512, false>(h, ept, nclusters, btasks);
-}
 // culled variants exist for 512 and 1024 threads per task (up to 31 slots per thread) and the large-landscape geometries
 static int launch_cull_any(mp_engine *h, int cs, int tpt, int nl_max, int nclusters, const void *btasks_v)
 {
     const BlockTask *btasks = (const BlockTask *)btasks_v;
     const int ept = (nl_max + tpt - 1) / tpt;
     if (tpt == 512) switch (cs) {
-        case 1: return launch_cull_512<1>(h, ept, nclusters, btasks);
-        case 2: return launch_cull_512<2>(h, ept, nclusters, btasks);
-        case 4: return launch_cull_512<4>(h, ept, nclusters, btasks);
-        default: return launch_cull_512<8>(h, ept, nclusters, btasks);
+        case 1: return launch_cull<1, 512>(h, ept, nclusters, btasks);
+        case 2: return launch_cull<2, 512>(h, ept, nclusters, btasks);
+        case 4: return launch_cull<4, 512>(h, ept, nclusters, btasks);
+        default: return launch_cull<8, 512>(h, ept, nclusters, btasks);
     }
     if (tpt == 1024) switch (cs) {
-        case 1: return launch_cull<1, 1024, false>(h, ept, nclusters, btasks);
-        case 2: return launch_cull<2, 1024, false>(h, ept, nclusters, btasks);
-        case 4: return launch_cull<4, 1024, false>(h, ept, nclusters, btasks);
-        default: return launch_cull<8, 1024, false>(h, ept, nclusters, btasks);
+        case 1: return launch_cull<1, 1024>(h, ept, nclusters, btasks);
+        case 2: return launch_cull<2, 1024>(h, ept, nclusters, btasks);
+        case 4: return launch_cull<4, 1024>(h, ept, nclusters, btasks);
+        default: return launch_cull<8, 1024>(h, ept, nclusters, btasks);
     }
-    if (tpt == 2048) return launch_cull<8, 2048, false>(h, ept, nclusters, btasks);
-    if (tpt == 4096) return cs == 16 ? launch_cull<16, 4096, false>(h, ept, nclusters, btasks) : launch_cull<8, 4096, false>(h, ept, nclusters, btasks);
-    if (tpt == 8192) return cs == 16 ? launch_cull<16, 8192, false>(h, ept, nclusters, btasks) : launch_cull<8, 8192, false>(h, ept, nclusters, btasks);
+    if (tpt == 2048) return launch_cull<8, 2048>(h, ept, nclusters, btasks);
+    if (tpt == 4096) return cs == 16 ? launch_cull<16, 4096>(h, ept, nclusters, btasks) : launch_cull<8, 4096>(h, ept, nclusters, btasks);
+    if (tpt == 8192) return cs == 16 ? launch_cull<16, 8192>(h, ept, nclusters, btasks) : launch_cull<8, 8192>(h, ept, nclusters, btasks);
     return MP_ERR_UNSUPPORTED;
 }
 }  // namespace mp

@@ -70,11 +70,6 @@ __device__ __forceinline__ void st_async_f32(uint32_t remote_addr, float v, uint
     asm volatile("st.async.weak.shared::cluster.mbarrier::complete_tx::bytes.b32 [%0], %1, [%2];"
                  ::"r"(remote_addr), "r"(__float_as_uint(v)), "r"(remote_mbar) : "memory");
 }
-__device__ __forceinline__ void st_async_f32x2(uint32_t remote_addr, float2 v, uint32_t remote_mbar)
-{
-    asm volatile("st.async.weak.shared::cluster.mbarrier::complete_tx::bytes.v2.b32 [%0], {%1, %2}, [%3];"
-                 ::"r"(remote_addr), "r"(__float_as_uint(v.x)), "r"(__float_as_uint(v.y)), "r"(remote_mbar) : "memory");
-}
 __device__ __forceinline__ void st_async_f32x4(uint32_t remote_addr, float4 v, uint32_t remote_mbar)
 {
     asm volatile("st.async.weak.shared::cluster.mbarrier::complete_tx::bytes.v4.b32 [%0], {%1, %2, %3, %4}, [%5];"
@@ -85,13 +80,6 @@ __device__ __forceinline__ float warp_sum_f(float v)
 {
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-    return v;
-}
-// rounds 8, 4, 2, 1 of warp_sum_f: the sum over each half-warp, formed by the same additions
-__device__ __forceinline__ float half_warp_sum_f(float v)
-{
-#pragma unroll
-    for (int o = 8; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
     return v;
 }
 
@@ -445,13 +433,14 @@ template <int CS, int TPT> static int launch_fast_u(mp_engine *h, int ept)
 static int launch_fast_any(mp_engine *h, int cs, int tpt)
 {
     const int ept = (h->cfg.n_patches + tpt - 1) / tpt;
+    if (tpt == 256) return cs >= 2 ? launch_fast_u<2, 256>(h, ept) : launch_fast_u<1, 256>(h, ept);   // small landscapes
+    if (tpt == 128) return launch_fast_u<1, 128>(h, ept);
+#ifndef MP_FAST_HAS_POSITIONS                           // with positions, 512 threads per task and more take the culled scan
     if (tpt > 1024) {                                   // large landscapes: clusters of 8 (or 16), 256..1024 threads per CTA
         if (tpt == 2048) return launch_fast_u<8, 2048>(h, ept);
         if (tpt == 4096) return cs == 16 ? launch_fast_u<16, 4096>(h, ept) : launch_fast_u<8, 4096>(h, ept);
         return cs == 16 ? launch_fast_u<16, 8192>(h, ept) : launch_fast_u<8, 8192>(h, ept);
     }
-    if (tpt == 256) return cs >= 2 ? launch_fast_u<2, 256>(h, ept) : launch_fast_u<1, 256>(h, ept);   // small landscapes
-    if (tpt == 128) return launch_fast_u<1, 128>(h, ept);
     if (tpt == 512) switch (cs) {
         case 1: return launch_fast_u<1, 512>(h, ept);
         case 2: return launch_fast_u<2, 512>(h, ept);
@@ -466,6 +455,8 @@ static int launch_fast_any(mp_engine *h, int cs, int tpt)
     case 16: return launch_fast_u<16, 1024>(h, ept);
     default: return launch_fast_u<8, 1024>(h, ept);
     }
+#endif
+    return MP_ERR_UNSUPPORTED;
 }
 }  // namespace mp
 #endif

@@ -5,8 +5,7 @@ alternate over the repeats; each repeat reports the scan's ms per launch (the en
 ms (host wall time around K synchronous sweeps, per-kernel timing off).  One sweep from an identical state with fixed
 parameters gives the y cells that differ from the first geometry and the largest relative |S_inc - S_recomputed|.
     python scripts/scan_micro.py [--steps 10] [--warmup 5] [--repeats 3] [--geometries 512x1,512x2,512x4] [--chains 64] [--out FILE]
-A geometry is TPTxCS, set through MP_FAST_TPT / MP_FAST_CS before its engine is created; TPTxCSb0 / TPTxCSb1 also sets
-MP_CULL_BRANCH (the culled scan's branch sum off / on), e.g. --geometries 512x4b0,512x4b1."""
+A geometry is TPTxCS, set through MP_FAST_TPT / MP_FAST_CS before its engine is created."""
 import argparse
 import importlib.util
 import json
@@ -41,24 +40,13 @@ def bench_module():
     return mod
 
 
-def parse_geometry(text):
-    """TPTxCS or TPTxCSbB -> (tpt, cs, branch or None)"""
-    tpt, rest = text.split("x")
-    cs, _, br = rest.partition("b")
-    return int(tpt), int(cs), (int(br) if br else None)
-
-
 def make_engine(wl, geom, chains, max_draws):
-    tpt, cs, br = geom
-    env = dict(MP_FAST_TPT=str(tpt), MP_FAST_CS=str(cs))
-    if br is not None:
-        env["MP_CULL_BRANCH"] = str(br)
-    os.environ.update(env)
+    tpt, cs = geom
+    os.environ["MP_FAST_TPT"], os.environ["MP_FAST_CS"] = str(tpt), str(cs)
     try:
         eng = mb.Engine(wl["n"], wl["T"], chains, precision=mb.FP32, seed=1000, detect=wl["detect"], max_draws=max_draws)
     finally:
-        for k in env:
-            del os.environ[k]
+        del os.environ["MP_FAST_TPT"], os.environ["MP_FAST_CS"]
     eng.set_landscape_coords(wl["px"], wl["py"], wl["area"])
     eng.set_source_units(wl.get("src_unit"))
     eng.set_observations(wl["obs"])
@@ -85,7 +73,7 @@ def main():
     args = ap.parse_args()
     if mb.engine.load_library().mp_device_count() < 1:
         raise SystemExit("scan_micro.py: no CUDA device; there is nothing to measure without a B200")
-    geoms = [parse_geometry(g) for g in args.geometries.split(",")]
+    geoms = [tuple(int(v) for v in g.split("x")) for g in args.geometries.split(",")]
     bench = bench_module()
     wl = synth.make_workload("cfg3")
     sc = mb.engine.sampler_config(**bench.sampler_kwargs(wl))
@@ -139,8 +127,7 @@ def main():
     for g, eng in engines.items():
         yy, srel, scan, work = agree[g]
         r = runs[g]
-        geometry = dict(threads_per_task=g[0], cluster=g[1]) if g[2] is None else dict(threads_per_task=g[0], cluster=g[1], branch=g[2])
-        results.append(dict(geometry=geometry, scan=scan,
+        results.append(dict(geometry=dict(threads_per_task=g[0], cluster=g[1]), scan=scan,
                             sweep_y_ms_per_launch=dict(median=float(np.median(r["sweep_y_ms"])), runs=[round(v, 3) for v in r["sweep_y_ms"]]),
                             step_ms=dict(median=float(np.median(r["step_ms"])), runs=[round(v, 3) for v in r["step_ms"]]),
                             one_sweep=dict(y_cells_differing=int((yy != y_ref).sum()), candidates=cand, max_rel_S_inc_vs_recomputed=srel,
@@ -150,7 +137,7 @@ def main():
         eng.close()
     out = dict(gpu=gpu_info(), workload="cfg3", desc=wl["desc"], n_patches=wl["n"], years=wl["T"], chains=C, steps=K,
                warmup=args.warmup, repeats=args.repeats,
-               method="engines built per geometry (MP_FAST_TPT / MP_FAST_CS, MP_CULL_BRANCH), all from one sampler state; after warm-up the geometries "
+               method="engines built per geometry (MP_FAST_TPT / MP_FAST_CS), all from one sampler state; after warm-up the geometries "
                       "alternate; sweep_y = per-kernel CUDA events (ms per launch), step = host wall time around K synchronous sweeps "
                       "with the per-kernel timing off; one_sweep compares y with the first geometry after one fixed-parameter sweep",
                results=results)

@@ -1,7 +1,8 @@
-"""The culled y scan's branch sum (MP_CULL_BRANCH, on by default at 512 threads per task): one trip also decides candidate
-i+1 given that candidate i was accepted, from the weights the trip already evaluated.  The decisions must be those of the
-scan without it up to FP32 ties, S must stay consistent, and the cancellation guard must defer i+1 where the shortcut
-would lose accuracy."""
+"""The culled y scan's branch sum (how every 512-thread task runs): one trip also decides candidate i+1 given that candidate i
+was accepted, from the weights the trip already evaluated.  The reference without the branch is the culled scan at 1,024
+threads per task (MP_FAST_TPT=1024), which takes the same two-candidate trips and evaluates the same 32-target groups.  The
+decisions must be the reference's up to FP32 ties, S must stay consistent, and the cancellation guard must defer i+1 where the
+shortcut would lose accuracy."""
 import numpy as np
 import pytest
 
@@ -16,8 +17,12 @@ FIXED = dict(sample_e=0, sample_c=0, update_z=0, n_adapt=0)
 
 
 def one_sweep(monkeypatch, spec, z, y, par, C, prec=mb.FP32, branch=True, seed=13, grid=None):
-    """One fixed-parameter sweep from (z, y): new y, incremental S, recomputed S, scan geometry, work counters."""
-    monkeypatch.setenv("MP_CULL_BRANCH", "1" if branch else "0")
+    """One fixed-parameter sweep from (z, y): new y, incremental S, recomputed S, scan geometry, work counters.
+    branch=False: the reference scan without the branch, 1,024 threads per task."""
+    if branch:
+        monkeypatch.delenv("MP_FAST_TPT", raising=False)
+    else:
+        monkeypatch.setenv("MP_FAST_TPT", "1024")
     with make_engine(spec, n_chains=C, precision=prec, seed=seed, max_draws=1) as eng:
         if grid is not None:
             eng.set_scan_blocks(*grid)
@@ -40,10 +45,11 @@ def max_rel(a, b, floor=1e-9):
     return float(np.max(np.abs(a - b) / np.maximum(np.abs(b), floor)))
 
 
-def test_branch_on_and_off_agree_at_the_cfg3_shape(monkeypatch):
-    """N = 10,000, 20 years, 64 chains (clusters of 4 x 128 threads): with and without the branch the same sweep decides the
-    same cells up to FP32 ties; with it a trip retires two candidates (about 0.5 trips per candidate), without it one after
-    an accepted flip (1 / (2 - p) trips per candidate at acceptance rate p)."""
+def test_branch_agrees_with_the_1024_thread_scan_at_the_cfg3_shape(monkeypatch):
+    """N = 10,000, 20 years, 64 chains (clusters of 4 x 128 threads): the 512-thread scan with the branch and the 1,024-thread
+    scan without it decide the same cells in the same sweep up to FP32 ties; with the branch a trip retires two candidates
+    (about 0.5 trips per candidate), without it one after an accepted flip (1 / (2 - p) trips per candidate at acceptance
+    rate p)."""
     monkeypatch.delenv("MP_FAST_TPT", raising=False); monkeypatch.delenv("MP_FAST_CS", raising=False)
     rng = np.random.default_rng(515)
     n, T, C = 10000, 20, 64
@@ -51,8 +57,9 @@ def test_branch_on_and_off_agree_at_the_cfg3_shape(monkeypatch):
     par = pdict(e=0.35, c=0.004, alpha=1 / 400, b=0.5)
     on = one_sweep(monkeypatch, spec, z, y, par, C, branch=True)
     off = one_sweep(monkeypatch, spec, z, y, par, C, branch=False)
+    assert on["geo"]["threads_per_task"] == 512 and on["geo"]["cluster"] == 4 and on["geo"]["culled"], on["geo"]
+    assert off["geo"]["threads_per_task"] == 1024 and off["geo"]["culled"], off["geo"]
     for r in (on, off):
-        assert r["geo"]["threads_per_task"] == 512 and r["geo"]["cluster"] == 4 and r["geo"]["culled"], r["geo"]
         assert max_rel(r["S"], r["S_new"]) <= 1e-6
     cand = int(((z[:-1] & z[1:]) == 1).sum()) * C
     differ = int((on["y"] != off["y"]).sum())
@@ -72,8 +79,9 @@ def test_guard_defers_on_isolated_targets(monkeypatch):
     """Pairs of patches 50 m apart, 4 km from any other pair (1/alpha = 400 m): the removal of one member takes nearly all of
     the other's S, the case where fl(S_hi - w) + S_lo is not accurate enough for the branch.  The guard must fire (trips whose
     second candidate is deferred: executed > retired evaluations), the decisions still agree with the FP64 path, and y and S
-    are those of the scan without the branch.  (The incremental S of the most isolated targets, ~1e-14 here, differs from a
-    recomputation by more than the 1e-6 the other landscapes meet, identically with and without the branch.)"""
+    are those of the scan without the branch (1,024 threads per task: the same groups, so the same commits).  (The
+    incremental S of the most isolated targets, ~1e-14 here, differs from a recomputation by more than the 1e-6 the other
+    landscapes meet, identically with and without the branch.)"""
     rng = np.random.default_rng(77)
     npair, T, C = 2200, 4, 2
     n = 2 * npair
@@ -90,6 +98,7 @@ def test_guard_defers_on_isolated_targets(monkeypatch):
     r32 = one_sweep(monkeypatch, spec, z, y, par, C)
     off = one_sweep(monkeypatch, spec, z, y, par, C, branch=False)
     assert r32["geo"]["threads_per_task"] == 512 and r32["geo"]["culled"], r32["geo"]
+    assert off["geo"]["threads_per_task"] == 1024 and off["geo"]["culled"], off["geo"]
     cand = int(((z[:-1] & z[1:]) == 1).sum()) * C
     w = r32["work"]
     print(f"evaluations executed {w['scan_exec']}, retired {w['scan_retired']}")
