@@ -13,6 +13,8 @@
  *   -c CHAINS   chains (default 8)      -b BURNIN  sweeps discarded (default SWEEPS/5)
  *   -r SEED     Philox seed (default 1) -g DEVICE  CUDA ordinal (default 0)
  *   -t FILE     also write the raw draws (one row per sweep and chain)
+ *   -O FILE     also write the posterior occupancy of every patch-year after the burn-in (mp_set_summaries): the T x N
+ *               table of P(z_tk = 1 | data), rows = years and columns = patches as in the input, "%.20lf\t" like -o
  *   -G 0,1,2,3  run the chains on several GPUs: the drop-in for `mpirun -np 4 MIDASPOM_MPI.out` (run_examples_MPI.sh:8).
  *               Where MIDASPOM_MPI splits the rows of the (e, c) grid over ranks and rank 0 collects them with MPI_Send /
  *               MPI_Recv (main_MIDASPOM_MPI.c:361-372,483-505), the chains are split over the listed devices (device g
@@ -54,7 +56,7 @@ static int run_grid(const int8_t *obs, int tmax, int n, double a, double d, floa
 #define MAXDEV 16
 static int run_mcmc(const int8_t *obs, int tmax, int n, double a, double d, float prioroc, int nstep, double ecmin,
                     double ecmax, const int *devices, int ndev, const char *fout, int nsweeps, int nchains, int burn, unsigned long long seed,
-                    const char *fdraws)
+                    const char *fdraws, const char *focc)
 {
     const int cpg = nchains / ndev;                                   /* chains per GPU (main checked divisibility) */
     mp_engine *hs[MAXDEV] = { NULL };
@@ -70,6 +72,7 @@ static int run_mcmc(const int8_t *obs, int tmax, int n, double a, double d, floa
     double *gath = (double *)malloc((size_t)nsweeps * nchains * MP_NDRAW * sizeof(double));
     double *draws = (double *)malloc((size_t)nsweeps * nchains * MP_NDRAW * sizeof(double));
     double *dens = (double *)calloc((size_t)nstep * nstep, sizeof(double));
+    double *occ = focc ? (double *)calloc((size_t)tmax * n * 2, sizeof(double)) : NULL;   /* sum over devices, one device's sums */
     for (int g = 0; g < ndev; g++) {
         mp_config cfg;
         memset(&cfg, 0, sizeof cfg);
@@ -77,7 +80,9 @@ static int run_mcmc(const int8_t *obs, int tmax, int n, double a, double d, floa
         cfg.max_draws = nsweeps; cfg.seed = seed; cfg.prior_occ = prioroc;
         if (mp_create(&cfg, &hs[g]) != MP_OK) { fprintf(stderr, "mp_create (device %d): %s\n", devices[g], mp_last_error(NULL)); goto out; }
         if (mp_set_landscape_linear(hs[g], d, NULL) || mp_set_source_units(hs[g], NULL) || mp_set_observations(hs[g], obs) ||
-            mp_set_params(hs[g], par) || mp_init_chains(hs[g], &sc, 1)) { fprintf(stderr, "setup: %s\n", mp_last_error(hs[g])); goto out; }
+            mp_set_params(hs[g], par) || mp_init_chains(hs[g], &sc, 1) || (focc && mp_set_summaries(hs[g], burn, 1))) {
+            fprintf(stderr, "setup: %s\n", mp_last_error(hs[g])); goto out;
+        }
     }
     if (ndev > 1 && mp_comm_init_all(hs, ndev)) { fprintf(stderr, "mp_comm_init_all: %s %s\n", mp_last_error(hs[0]), mp_comm_last_error()); goto out; }
     printf("Starting MCMC: %d chains x %d sweeps (%d burn-in) on %d GPU%s\n", nchains, nsweeps, burn, ndev, ndev > 1 ? "s" : "");
@@ -116,6 +121,21 @@ static int run_mcmc(const int8_t *obs, int tmax, int n, double a, double d, floa
     printf("Writing output in file %s... ", fout);
     if (mp_write_table(fout, dens, nstep, nstep)) goto out;
     printf("done\n");
+    if (focc) {
+        /* Rao-Blackwellised occupancy, summed over the devices' chains (each device holds its own chains' sums) */
+        const size_t cells = (size_t)tmax * n;
+        int64_t ns = 0;
+        for (int g = 0; g < ndev; g++) {
+            int64_t nsg = 0;
+            if (mp_get_summaries(hs[g], &nsg, NULL, occ + cells, NULL, NULL, 0)) { fprintf(stderr, "summaries: %s\n", mp_last_error(hs[g])); goto out; }
+            for (size_t i = 0; i < cells; i++) occ[i] += occ[cells + i];
+            ns += nsg;
+        }
+        for (size_t i = 0; i < cells; i++) occ[i] = ns > 0 ? occ[i] / (double)ns : 0.0;
+        printf("Writing posterior occupancy (%lld samples) in file %s... ", (long long)ns, focc);
+        if (mp_write_table(focc, occ, tmax, n)) goto out;
+        printf("done\n");
+    }
     if (fdraws) {
         FILE *f = fopen(fdraws, "wb");
         if (f) {
@@ -130,7 +150,7 @@ static int run_mcmc(const int8_t *obs, int tmax, int n, double a, double d, floa
     }
     rc = 0;
 out:
-    free(par); free(draws); free(gath); free(dens);
+    free(par); free(draws); free(gath); free(dens); free(occ);
     for (int g = 0; g < ndev; g++) if (hs[g]) mp_destroy(hs[g]);
     return rc;
 }
@@ -139,13 +159,13 @@ int main(int argc, char **argv)
 {
     printf("------ MIDASPOM on B200 (midaspom_b200; model and formats of MIDASPOM beta, Alcala, Cole & Rosenberg) ------\n");
     float prioroc = 0.5f;                 /* defaults of main_MIDASPOM.c:66-73 */
-    const char *fname = "input.txt", *fout = "posterior.txt", *fdraws = NULL;
+    const char *fname = "input.txt", *fout = "posterior.txt", *fdraws = NULL, *focc = NULL;
     double d = 100, a = 1.0 / 400, ecmin = 0.0, ecmax = 1.0;
     int nstep = 101, nsweeps = 0, nchains = 8, burn = -1, device = 0, c;
     unsigned long long seed = 1;
     int devices[MAXDEV], ndev = 0;
     opterr = 0;
-    while ((c = getopt(argc, argv, "m:p:d:i:o:s:l:u:n:c:b:r:g:t:G:")) != -1)
+    while ((c = getopt(argc, argv, "m:p:d:i:o:s:l:u:n:c:b:r:g:t:G:O:")) != -1)
         switch (c) {
         case 'm': a = 1.0 / atof(optarg); break;
         case 'p': prioroc = (float)atof(optarg); break;
@@ -161,6 +181,7 @@ int main(int argc, char **argv)
         case 'r': seed = strtoull(optarg, NULL, 10); break;
         case 'g': device = atoi(optarg); break;
         case 't': fdraws = optarg; break;
+        case 'O': focc = optarg; break;
         case 'G':
             for (char *tok = strtok(optarg, ","); tok && ndev < MAXDEV; tok = strtok(NULL, ",")) devices[ndev++] = atoi(tok);
             break;
@@ -168,6 +189,7 @@ int main(int argc, char **argv)
         }
     if (nstep < 2) { fprintf(stderr, "-s must be at least 2\n"); return 1; }
     if (ndev == 0) { devices[0] = device; ndev = 1; }
+    if (focc && nsweeps <= 0) { fprintf(stderr, "-O needs -n SWEEPS (the occupancy comes from the chains)\n"); return 1; }
     if (ndev > 1 && (nsweeps <= 0 || nchains % ndev)) { fprintf(stderr, "-G needs -n SWEEPS and a chain count divisible by the number of GPUs\n"); return 1; }
     const double win = (ecmax - ecmin) / (nstep - 1);
     printf("Parameters for numerical approximation of the posterior density:\n\tWindow size=%lf, number of steps=%d\n", win, nstep);
@@ -199,7 +221,7 @@ int main(int argc, char **argv)
     int rc;
     if (nsweeps > 0) {
         if (burn < 0) burn = nsweeps / 5;
-        rc = run_mcmc(obs, tmax, n, a, d, prioroc, nstep, ecmin, ecmax, devices, ndev, fout, nsweeps, nchains, burn, seed, fdraws);
+        rc = run_mcmc(obs, tmax, n, a, d, prioroc, nstep, ecmin, ecmax, devices, ndev, fout, nsweeps, nchains, burn, seed, fdraws, focc);
     } else rc = run_grid(obs, tmax, n, a, d, prioroc, nstep, ecmin, ecmax, devices[0], fout);
     free(obs);
     printf(" Total running time: %.2lf min\n", difftime(time(NULL), start) / 60.0);

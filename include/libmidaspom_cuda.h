@@ -23,6 +23,7 @@
  *   mp_set_era / mp_params.K,Ksrc,dsrc   dieoff.c:56-57,78 ; loss.c:93-101,365 ; future.c:67,90-97
  *   mp_simulate               future.c:64-110 (simpij) + :359-386 (simulation loop)
  *   mp_forecast               future.c:359-386 at large N: the simulation loop started from the sampler's own chains
+ *   mp_set_summaries / mp_get_summaries   (no counterpart) posterior occupancy, survival and connectivity of every patch-year
  *
  * All device memory is owned by the engine handle; host buffers are owned by the caller.  One
  * handle per GPU / host thread (thread-compatible, not thread-safe).  There is no CPU fallback:
@@ -179,6 +180,30 @@ int mp_num_draws(mp_engine *h);
 int mp_get_draws(mp_engine *h, int first, int count, double *out /* count*C*MP_NDRAW */);
 int mp_reset_draws(mp_engine *h);
 int mp_sweep_index(mp_engine *h);
+/* Posterior summaries of the latent state (no reference counterpart: the reference marginalises the missing cells away),
+ * accumulated on the device at the end of every qualifying sweep, summed over this engine's chains.  first_sweep: the first
+ * sweep index (as mp_sweep_index counts) that is accumulated; thin: every thin-th sweep from there.  thin = 0 switches the
+ * summaries off and frees them.  Setting them zeroes every array.  A sweep adds the state it ends with: z, y, S after the
+ * y scan and the parameters after the e/p update.  The sweep counter is read on the device, so captured sweeps replay
+ * unchanged; without summaries a sweep launches exactly what it launched before.  One kernel per qualifying sweep, counted
+ * under MP_K_SMALL.  Device memory: T N 12 + (T-1) N 12 bytes.
+ * mp_forecast, mp_connectivity, mp_loglik, mp_loglik_host, mp_simulate* and mp_flip_delta leave the sums unchanged.
+ * mp_sweep_sharded[_all] ranks hold identical sums (phase 3 runs replicated); chain-sharded engines (chain_offset) add theirs.
+ * MP_ERR_ARG: first_sweep < 0 or thin < 0. */
+int mp_set_summaries(mp_engine *h, int first_sweep, int thin);
+/* Copy (and with reset != 0 zero) the sums.  Every output is nullable.  Synchronous, after any queued sweeps.
+ *   nsamples   accumulated sweeps x n_chains
+ *   z_count    T*N      uint32   number of samples with z_tk = 1
+ *   z_prob     T*N      double   sum of P(z_tk = 1 | y, theta, obs) (Rao-Blackwellised: the log-odds of k_update_z, in the
+ *                                engine's precision; 1 for cells an adjacent y = 1 forces; the indicator for cells the data fix;
+ *                                0 where the log-odds is NaN, as the Gibbs draw)
+ *   y_count    (T-1)*N  uint32   number of samples with y_tk = 1 (patch occupied and survived extinction in t -> t+1)
+ *   S_sum      (T-1)*N  double   sum of the connectivity S_tk
+ * Extinctions in t -> t+1 = z_count[t] - y_count[t]; colonisations = z_count[t+1] - y_count[t].
+ * MP_ERR_STATE: summaries not set.  mp_sweep (and the sharded and phase forms) refuses with MP_ERR_STATE, before launching,
+ * when the queued sweeps could push nsamples past 2^32 - 1, the limit of the uint32 counts. */
+int mp_get_summaries(mp_engine *h, int64_t *nsamples, uint32_t *z_count, double *z_prob, uint32_t *y_count,
+                     double *S_sum, int reset);
 
 /* ---- forward simulator ---- */
 /* nsims independent trajectories of nyears from z0 (N bytes); era_all != 0 applies K/Ksrc every

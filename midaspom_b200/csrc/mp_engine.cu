@@ -430,6 +430,48 @@ template <typename R> static int phase_sweep_y(mp_engine *h)
     if (h->sc.update_y) return launch_sweep_y<R>(h);
     return MP_OK;
 }
+// ---- posterior summaries (mp_set_summaries): z_prob [T][N], S_sum [T-1][N], z_count [T][N], y_count [T-1][N], sample counter
+struct SumLayout { size_t z_prob, S_sum, z_count, y_count, nsamples, bytes; };
+static SumLayout sum_layout(const mp_engine *h)
+{
+    SumLayout L;
+    size_t off = 0;
+    auto carve = [&](size_t bytes) { const size_t o = off; off += (bytes + 255) / 256 * 256; return o; };
+    L.z_prob = carve(zcells(h) * 8); L.S_sum = carve(ycells(h) * 8); L.z_count = carve(zcells(h) * 4);
+    L.y_count = carve(ycells(h) * 4); L.nsamples = carve(8); L.bytes = off;
+    return L;
+}
+static bool summary_due(const mp_engine *h, uint32_t s)
+{
+    return h->sum_thin > 0 && s >= (uint32_t)h->sum_first && (s - (uint32_t)h->sum_first) % (uint32_t)h->sum_thin == 0;
+}
+// refuse sweeps that could push the sample counter past the range of the uint32 counts
+static int summaries_room(mp_engine *h, int nsweeps)
+{
+    if (h->sum_thin <= 0 || nsweeps <= 0) return MP_OK;
+    // qualifying sweeps first + k thin (k >= 0) in [lo, hi)
+    const long long first = h->sum_first, thin = h->sum_thin, hi = (long long)h->sweep + nsweeps;
+    const long long lo = std::max<long long>(h->sweep, first);
+    const unsigned long long due = hi <= lo ? 0ull : (unsigned long long)((hi - first + thin - 1) / thin - (lo - first + thin - 1) / thin);
+    REQUIRE(h->sum_samples + due * nC(h) <= 0xffffffffull, MP_ERR_STATE,
+            "mp_sweep: the summaries would pass 2^32 - 1 samples (read them with reset, or set them again)");
+    return MP_OK;
+}
+template <typename R> static int launch_summaries(mp_engine *h)
+{
+    const SumLayout L = sum_layout(h);
+    SumBufs b;
+    b.z_prob = (double *)(h->d_sum + L.z_prob); b.S_sum = (double *)(h->d_sum + L.S_sum);
+    b.z_count = (uint32_t *)(h->d_sum + L.z_count); b.y_count = (uint32_t *)(h->d_sum + L.y_count);
+    b.nsamples = (unsigned long long *)(h->d_sum + L.nsamples);
+    const long long threads = (long long)nT(h) * (long long)((nN(h) + 3) / 4);
+    k_summaries<R><<<(unsigned)((threads + 255) / 256), 256, 0, h->stream>>>(sampler_dev(h), h->d_ctr, h->sum_first, h->sum_thin,
+        view<R>(h), h->d_par, h->d_obs, h->have_era ? h->d_era : nullptr, h->d_z, h->d_y, h->d_S[0], h->cfg.n_years, h->cfg.n_chains, b);
+    CK(cudaGetLastError());
+    if (summary_due(h, h->sweep)) h->sum_samples += nC(h);
+    return MP_OK;
+}
+
 // phase 3: e and p from the sufficient counts, record the draw
 template <typename R> static int phase_finish(mp_engine *h)
 {
@@ -447,6 +489,12 @@ template <typename R> static int phase_finish(mp_engine *h)
         // no per-sweep host value, so a captured sweep can be replayed (mp_sweep)
         k_record<<<C, 32, 0, h->stream>>>(sd, h->d_par, h->d_counts, h->d_partial[0], h->nblk_col, h->d_draws, nullptr, h->d_ctr, h->cfg.max_draws);
         CK(cudaGetLastError());
+        // the sweep's final z, y, S and theta, gated on the device by the sweep counter before k_advance moves it; one more
+        // launch in this span (without summaries the sweep keeps its launches and counts)
+        if (h->sum_thin > 0) {
+            h->t_launch[MP_K_SMALL]++;
+            if ((rc = launch_summaries<R>(h)) != MP_OK) return rc;
+        }
         k_advance<<<1, 1, 0, h->stream>>>(h->d_ctr, h->cfg.max_draws);
         CK(cudaGetLastError());
     }
@@ -488,7 +536,7 @@ int mp_destroy(mp_engine *h)
     for (auto e : h->pool) cudaEventDestroy(e);
     void *ptrs[] = { h->d_area, h->d_src_unit, h->d_px, h->d_py, h->d_dist, h->d_obs, h->d_era, h->d_par, h->d_prop,
                      h->d_lsig, h->d_z, h->d_y, h->d_srec, h->d_S[0], h->d_S[1], h->d_aw[0], h->d_aw[1], h->d_partial[0],
-                     h->d_partial[1], h->d_llc, h->d_logu, h->d_parts, h->d_scalar, h->d_flags, h->d_counts, h->d_draws, h->d_cand, h->d_cand_count, h->d_task_order, h->d_ljac, h->d_perm, h->d_scan, h->d_minv, h->d_tile_box, h->d_mlow, h->d_work, h->d_gemm, h->d_tlist, h->d_btasks, h->d_blockmode, h->d_scan_work, h->d_comm_send, h->d_comm_recv, h->d_ctr };
+                     h->d_partial[1], h->d_llc, h->d_logu, h->d_parts, h->d_scalar, h->d_flags, h->d_counts, h->d_draws, h->d_cand, h->d_cand_count, h->d_task_order, h->d_ljac, h->d_perm, h->d_scan, h->d_minv, h->d_tile_box, h->d_mlow, h->d_work, h->d_gemm, h->d_tlist, h->d_btasks, h->d_blockmode, h->d_scan_work, h->d_comm_send, h->d_comm_recv, h->d_ctr, h->d_sum };
     for (void *p : ptrs) if (p) cudaFree(p);
     if (h->stream) cudaStreamDestroy(h->stream);
     delete h;
@@ -1092,6 +1140,7 @@ int mp_sweep(mp_engine *h, int nsweeps)
     int rc = check_ready(h);
     if (rc != MP_OK) return rc;
     REQUIRE(h->have_sc && h->have_obs, MP_ERR_STATE, "sampler not configured (mp_init_chains / mp_set_sampler)");
+    if ((rc = summaries_room(h, nsweeps)) != MP_OK) return rc;
     h->par_host_valid = false;                           // the sampler moves the parameters on the device
     for (int s = 0; s < nsweeps; s++) {
         // A sweep is ~20 launches that carry no per-sweep host value (the kernels read the sweep and draw counters from device
@@ -1101,7 +1150,7 @@ int mp_sweep(mp_engine *h, int nsweeps)
         if (h->use_graph && !h->timing && h->S_valid && h->S_exact && whole) {
             const int v = (is64(h) || h->refresh_every <= 1 || (h->sweep % (uint32_t)h->refresh_every) == 0) ? 1 : 0;
             if (!h->gexec[v] && h->gwarm[v]) {
-                const uint32_t sweep0 = h->sweep; const int ndraws0 = h->ndraws;
+                const uint32_t sweep0 = h->sweep; const int ndraws0 = h->ndraws; const unsigned long long samples0 = h->sum_samples;
                 long long before[MP_K_NCAT];
                 for (int i = 0; i < MP_K_NCAT; i++) before[i] = h->t_launch[i];
                 cudaGraph_t g = nullptr;
@@ -1112,7 +1161,7 @@ int mp_sweep(mp_engine *h, int nsweeps)
                     if (ok) ok = cudaGraphInstantiate(&h->gexec[v], g, 0) == cudaSuccess;
                     if (g) cudaGraphDestroy(g);
                 }
-                h->sweep = sweep0; h->ndraws = ndraws0;       // nothing ran yet: the capture only advanced the host mirrors ...
+                h->sweep = sweep0; h->ndraws = ndraws0; h->sum_samples = samples0;   // nothing ran yet: the capture only advanced the host mirrors ...
                 for (int i = 0; i < MP_K_NCAT; i++) { h->glaunch[v][i] = h->t_launch[i] - before[i]; h->t_launch[i] = before[i]; }   // ... and the launch counts, which every replay adds
                 if (!ok) { cudaGetLastError(); h->gexec[v] = nullptr; h->use_graph = 0; }
             }
@@ -1120,6 +1169,7 @@ int mp_sweep(mp_engine *h, int nsweeps)
                 CK(cudaGraphLaunch(h->gexec[v], h->stream));
                 for (int i = 0; i < MP_K_NCAT; i++) h->t_launch[i] += h->glaunch[v][i];
                 if (h->ndraws < h->cfg.max_draws) h->ndraws++;
+                if (summary_due(h, h->sweep)) h->sum_samples += nC(h);
                 h->sweep++;
                 continue;
             }
@@ -1158,7 +1208,9 @@ int mp_sweep_phase(mp_engine *h, int phase, int *flags_out)
     case PH_PROPOSE_CONN: return is64(h) ? phase_propose_conn<double>(h, flags_out) : phase_propose_conn<float>(h, flags_out);
     case PH_DECIDE_Z: return is64(h) ? phase_decide_z<double>(h) : phase_decide_z<float>(h);
     case PH_SWEEP_Y: return is64(h) ? phase_sweep_y<double>(h) : phase_sweep_y<float>(h);
-    case PH_FINISH: return is64(h) ? phase_finish<double>(h) : phase_finish<float>(h);
+    case PH_FINISH:
+        if ((rc = summaries_room(h, 1)) != MP_OK) return rc;
+        return is64(h) ? phase_finish<double>(h) : phase_finish<float>(h);
     default: h->err = "mp_sweep_phase: unknown phase"; return MP_ERR_ARG;
     }
 }
@@ -1237,6 +1289,7 @@ int mp_sweep_sharded_all(mp_engine **hs, int n, int nsweeps)
     if (!hs || n < 1 || !hs[0]) return MP_ERR_ARG;
     int rc;
     for (int i = 0; i < n; i++) { if (!hs[i]) return MP_ERR_ARG; if ((rc = sharded_prepare(hs[i])) != MP_OK) return rc; }
+    for (int i = 0; i < n; i++) if ((rc = summaries_room(hs[i], nsweeps)) != MP_OK) return rc;
     for (int s = 0; s < nsweeps; s++)
         for (int stage = SH_CONN; stage <= SH_FINISH; stage++) {
             const bool coll = stage == SH_GATHER || stage == SH_ROWS;   // the collectives of all local engines form one NCCL group
@@ -1252,6 +1305,45 @@ int mp_synchronize(mp_engine *h)
     if (!h) return MP_ERR_ARG;
     CK(cudaSetDevice(h->cfg.device));
     CK(cudaStreamSynchronize(h->stream));
+    return MP_OK;
+}
+int mp_set_summaries(mp_engine *h, int first_sweep, int thin)
+{
+    if (!h) return MP_ERR_ARG;
+    REQUIRE(first_sweep >= 0 && thin >= 0, MP_ERR_ARG, "mp_set_summaries: first_sweep and thin must be >= 0");
+    CK(cudaSetDevice(h->cfg.device));
+    int rc = quiesce(h);                                 // the captured sweeps launch k_summaries or not: capture again
+    if (rc != MP_OK) return rc;
+    h->sum_first = first_sweep; h->sum_thin = thin; h->sum_samples = 0;
+    if (thin == 0) {
+        if (h->d_sum) { CK(cudaFree(h->d_sum)); h->d_sum = nullptr; }
+        return MP_OK;
+    }
+    const SumLayout L = sum_layout(h);
+    if (!h->d_sum) {
+        cudaError_t e = cudaMalloc(&h->d_sum, L.bytes);
+        if (e != cudaSuccess) { h->d_sum = nullptr; h->sum_thin = 0; h->err = std::string("mp_set_summaries: ") + cudaGetErrorString(e); return MP_ERR_CUDA; }
+    }
+    CK(cudaMemsetAsync(h->d_sum, 0, L.bytes, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    return MP_OK;
+}
+int mp_get_summaries(mp_engine *h, int64_t *nsamples, uint32_t *z_count, double *z_prob, uint32_t *y_count, double *S_sum, int reset)
+{
+    if (!h) return MP_ERR_ARG;
+    REQUIRE(h->d_sum, MP_ERR_STATE, "mp_get_summaries: summaries not set (mp_set_summaries)");
+    CK(cudaSetDevice(h->cfg.device));
+    const SumLayout L = sum_layout(h);
+    unsigned long long ns = 0;
+    CK(cudaMemcpyAsync(&ns, h->d_sum + L.nsamples, 8, cudaMemcpyDeviceToHost, h->stream));
+    if (z_count) CK(cudaMemcpyAsync(z_count, h->d_sum + L.z_count, zcells(h) * 4, cudaMemcpyDeviceToHost, h->stream));
+    if (z_prob) CK(cudaMemcpyAsync(z_prob, h->d_sum + L.z_prob, zcells(h) * 8, cudaMemcpyDeviceToHost, h->stream));
+    if (y_count) CK(cudaMemcpyAsync(y_count, h->d_sum + L.y_count, ycells(h) * 4, cudaMemcpyDeviceToHost, h->stream));
+    if (S_sum) CK(cudaMemcpyAsync(S_sum, h->d_sum + L.S_sum, ycells(h) * 8, cudaMemcpyDeviceToHost, h->stream));
+    if (reset) CK(cudaMemsetAsync(h->d_sum, 0, L.bytes, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    if (nsamples) *nsamples = (int64_t)ns;
+    if (reset) h->sum_samples = 0;
     return MP_OK;
 }
 int mp_num_draws(mp_engine *h) { return h ? h->ndraws : MP_ERR_ARG; }

@@ -101,6 +101,10 @@ struct mp_engine {
     int comm_size = 1, comm_rank = 0, comm_per = 0;   // comm_per: scan-order slots per rank of the sharded connectivity
     double *d_comm_send = nullptr, *d_comm_recv = nullptr;   // packed connectivity columns of the sharded sweep
     int shard_flags = 0;              // what phase 0 of the current sharded sweep computed (bit 0: S, bit 1: S_prop)
+    // posterior summaries of the latent state (mp_set_summaries): z_prob, S_sum, z_count, y_count and the sample counter
+    unsigned char *d_sum = nullptr;
+    int sum_first = 0, sum_thin = 0;  // sum_thin == 0: off
+    unsigned long long sum_samples = 0;   // host mirror of the device sample counter, queued sweeps included
     // timing
     bool timing = false;
     struct Span { cudaEvent_t a, b; int cat; };

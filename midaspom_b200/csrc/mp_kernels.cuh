@@ -7,6 +7,7 @@
 //  k_flip_delta    rank-1 log-odds of one intermediate-state flip
 //  k_sweep_y       Gibbs scan of y_t | z with rank-1 updates of S_t in shared memory
 //  k_update_z      Gibbs update of latent occupancy cells (conditionally independent given y)
+//  k_summaries     posterior sums of z, P(z = 1 | y, theta), y and S over the chains (mp_set_summaries)
 //  k_propose_* / k_decide_* / k_update_ep / k_record   Metropolis bookkeeping, one warp per chain
 //  k_sim_init / k_sim_ext / k_sim_col   forward simulator (future.c:64-110)
 //  k_fc_init / k_fc_ext / k_fc_col      posterior-predictive forecast from the chains (with k_pack_sources + k_conn)
@@ -365,6 +366,27 @@ static __global__ void k_advance(uint32_t *__restrict__ ctr, int max_draws)
 }
 
 // ------------------------------------------------------------------ latent occupancy cells
+// Log-odds of z_tk = 1 given y and theta for a latent cell (observation o) that no adjacent y = 1 forces: colonisation
+// term of t-1 -> t, extinction term of t -> t+1, year-0 prior, missed detection.  The colonisation and extinction terms are
+// formed in R, the rest in FP64.  Shared by the Gibbs draw (k_update_z) and its Rao-Blackwellised mean (k_summaries) so that
+// both see the same number.  Sc: the chain's S [transition][patch]; i = t n + k.
+template <typename R>
+__device__ __forceinline__ double z_logodds(const SamplerDev &sd, const Landscape<R> &ls, const mp_params &p, const Trans<R> &tr0,
+                                            const Trans<R> &tr1, const uint8_t *__restrict__ era, const double *__restrict__ Sc,
+                                            int o, long long i, int t, int k, int ntrans)
+{
+    R lo = 0;
+    if (t > 0) {
+        const Trans<R> tr = pick_trans<R>(tr0, tr1, era ? era[t - 1] != 0 : 0);
+        const R C = col_prob<R>(tr, (R)Sc[i - ls.n], source_term<R>(ls, tr, k));
+        lo += Num<R>::logv(C) - Num<R>::log1m(C);
+    }
+    if (t < ntrans) lo += (era && era[t]) ? tr1.logE : tr0.logE;
+    double lod = (double)lo;
+    if (t == 0) lod += log(sd.p0) - log(1.0 - sd.p0);
+    if (sd.detect && o == 0) lod += log(1.0 - p.p);
+    return lod;
+}
 // z_tk | y, theta for every latent cell at once: S depends on y only, so the cells are
 // conditionally independent.  Forced to 1 when an adjacent intermediate state is 1.
 template <typename R>
@@ -386,19 +408,91 @@ __global__ void k_update_z(SamplerDev sd, const uint32_t *__restrict__ sweep_p /
         const int t = (int)(i / n), k = (int)(i - (long long)t * n);
         const bool forced = (t > 0 && yc[i - n]) || (t < ntrans && yc[i]);
         if (forced) { zc[i] = 1; continue; }
-        R lo = 0;
-        if (t > 0) {
-            const Trans<R> tr = pick_trans<R>(tr0, tr1, era ? era[t - 1] != 0 : 0);
-            const R C = col_prob<R>(tr, (R)Sc[i - n], source_term<R>(ls, tr, k));
-            lo += Num<R>::logv(C) - Num<R>::log1m(C);
-        }
-        if (t < ntrans) lo += (era && era[t]) ? tr1.logE : tr0.logE;
-        double lod = (double)lo;
-        if (t == 0) lod += log(sd.p0) - log(1.0 - sd.p0);
-        if (sd.detect && o == 0) lod += log(1.0 - p.p);
+        const double lod = z_logodds<R>(sd, ls, p, tr0, tr1, era, Sc, o, i, t, k, ntrans);
         const uint4 r = rng(sd.seed, (uint32_t)(sd.chain_offset + c), sweep, RK_Z, (uint32_t)k, (uint32_t)t);
         zc[i] = isnan(lod) ? 0 : (logit_u(r.x) < lod);
     }
+}
+
+// ------------------------------------------------------------------ posterior summaries of the latent state (mp_set_summaries)
+// Sums over this engine's chains, added at the end of every sweep s with s >= first and (s - first) % thin == 0 (the sweep
+// counter is read on the device, so a captured sweep replays unchanged).  Layout [year][patch]; y_count and S_sum have T-1 rows.
+struct SumBufs {
+    double *z_prob, *S_sum;
+    uint32_t *z_count, *y_count;
+    unsigned long long *nsamples;
+};
+// 4 bytes of a row of z or y, byte j = patch k0 + j (m <= 4 valid patches); rows start on a 4-byte boundary when n % 4 == 0
+__device__ __forceinline__ uint32_t load_cells4(const uint8_t *__restrict__ p, int m, bool words)
+{
+    if (words) return *reinterpret_cast<const uint32_t *>(p);
+    uint32_t v = 0;
+    for (int j = 0; j < m; j++) v |= (uint32_t)p[j] << (8 * j);
+    return v;
+}
+// One thread per (year, 4 consecutive patches) visits the chains in order c = 0 .. C-1 and read-modify-writes only its own
+// cells: no atomics, and every sum is the same whatever the launch geometry.  z_prob adds P(z_tk = 1 | y, theta) for the latent
+// cells (1 when forced, 0 for a NaN log-odds, as k_update_z draws there) and the indicator for the cells the data fix.
+template <typename R>
+__global__ void __launch_bounds__(256)
+k_summaries(SamplerDev sd, const uint32_t *__restrict__ sweep_p /* device-resident sweep counter (k_advance) */, int first, int thin,
+            Landscape<R> ls, const mp_params *__restrict__ par, const int8_t *__restrict__ obs, const uint8_t *__restrict__ era,
+            const uint8_t *__restrict__ z, const uint8_t *__restrict__ y, const double *__restrict__ S, int T, int nchains, SumBufs b)
+{
+    const uint32_t s = *sweep_p;
+    if (s < (uint32_t)first || (s - (uint32_t)first) % (uint32_t)thin) return;
+    const int n = ls.n, ntrans = T - 1, nq = (n + 3) >> 2;
+    const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (idx == 0) *b.nsamples += (unsigned long long)nchains;
+    if (idx >= (long long)T * nq) return;
+    const int t = (int)(idx / nq), k0 = 4 * (int)(idx - (long long)t * nq), m = min(4, n - k0);
+    const bool words = (n & 3) == 0, has_y = t < ntrans;
+    const size_t row = (size_t)t * n + k0;
+    int o[4];
+    bool latent[4], any_latent = false;
+    uint32_t zc[4] = { 0, 0, 0, 0 }, yc[4] = { 0, 0, 0, 0 };
+    double zp[4] = { 0, 0, 0, 0 }, ss[4] = { 0, 0, 0, 0 };
+#pragma unroll
+    for (int j = 0; j < 4; j++) {
+        o[j] = j < m ? obs[row + j] : 1;
+        latent[j] = o[j] == -1 || (sd.detect && o[j] == 0);
+        any_latent |= latent[j];
+        if (j < m) {
+            zc[j] = b.z_count[row + j]; zp[j] = b.z_prob[row + j];
+            if (has_y) { yc[j] = b.y_count[row + j]; ss[j] = b.S_sum[row + j]; }
+        }
+    }
+    for (int c = 0; c < nchains; c++) {
+        const uint8_t *zch = z + (size_t)c * T * n, *ych = y + (size_t)c * ntrans * n;
+        const double *Sc = S + (size_t)c * ntrans * n;
+        const uint32_t zw = load_cells4(zch + row, m, words);
+        const uint32_t yw = has_y ? load_cells4(ych + row, m, words) : 0u;
+        const uint32_t yprev = t > 0 ? load_cells4(ych + row - n, m, words) : 0u;
+        mp_params p;
+        Trans<R> tr0, tr1;
+        if (any_latent) { p = par[c]; tr0 = make_trans<R>(p, 0); tr1 = make_trans<R>(p, 1); }
+#pragma unroll
+        for (int j = 0; j < 4; j++) {
+            if (j >= m) continue;
+            const uint32_t zz = ((zw >> (8 * j)) & 0xffu) != 0u;
+            double pr = (double)zz;
+            if (latent[j]) {
+                if (((yw | yprev) >> (8 * j)) & 0xffu) pr = 1.0;
+                else {
+                    const double lod = z_logodds<R>(sd, ls, p, tr0, tr1, era, Sc, o[j], (long long)(row + j), t, k0 + j, ntrans);
+                    pr = isnan(lod) ? 0.0 : 1.0 / (1.0 + exp(-lod));
+                }
+            }
+            zc[j] += zz; zp[j] += pr;
+            if (has_y) { yc[j] += ((yw >> (8 * j)) & 0xffu) != 0u; ss[j] += Sc[row + j]; }
+        }
+    }
+#pragma unroll
+    for (int j = 0; j < 4; j++)
+        if (j < m) {
+            b.z_count[row + j] = zc[j]; b.z_prob[row + j] = zp[j];
+            if (has_y) { b.y_count[row + j] = yc[j]; b.S_sum[row + j] = ss[j]; }
+        }
 }
 
 // ------------------------------------------------------------------ rank-1 flip of the intermediate state

@@ -33,6 +33,7 @@ ABI_SYMBOLS = (
     "mp_get_scan_order", "mp_get_work_counters", "mp_get_scan_geometry", "mp_get_conn_path", "mp_set_scan_blocks",
     "mp_comm_unique_id", "mp_comm_init", "mp_comm_init_all", "mp_comm_destroy", "mp_comm_rank", "mp_comm_size", "mp_comm_last_error",
     "mp_gather_draws", "mp_gather_draws_all", "mp_sweep_sharded", "mp_sweep_sharded_all", "mp_forecast",
+    "mp_set_summaries", "mp_get_summaries",
 )
 
 
@@ -129,6 +130,8 @@ def load_library(build_if_missing: bool = True) -> C.CDLL:
     L.mp_simulate.argtypes = [vp, pp, u8p, C.c_int, C.c_int, C.c_uint64, C.c_int, u8p, C.POINTER(C.c_int32)]
     L.mp_simulate_ensemble.argtypes = [vp, pp, u8p, C.c_int, C.c_int, C.c_uint64, C.c_int, u8p, C.POINTER(C.c_int32)]
     L.mp_forecast.argtypes = [vp, C.c_int, C.c_int, C.c_uint64, dp, C.POINTER(C.c_int32), C.POINTER(C.c_uint32)]
+    L.mp_set_summaries.argtypes = [vp, C.c_int, C.c_int]
+    L.mp_get_summaries.argtypes = [vp, C.POINTER(C.c_int64), C.POINTER(C.c_uint32), dp, C.POINTER(C.c_uint32), dp, C.c_int]
     L.mp_device_ptr.argtypes = [vp, C.c_int, C.POINTER(vp), C.POINTER(C.c_size_t)]
     L.mp_get_stream.argtypes = [vp, C.POINTER(vp)]
     L.mp_set_timing.argtypes = [vp, C.c_int]
@@ -470,6 +473,25 @@ class Engine:
         self._ck(self.lib.mp_forecast(self.h, int(nyears), int(nrep), int(seed), _p(scen, _dp), _p(occ, C.POINTER(C.c_int32)),
                                       _p(inc, C.POINTER(C.c_uint32))), "mp_forecast")
         return occ, inc
+
+    # -- posterior summaries of the latent state
+    def set_summaries(self, first_sweep=0, thin=1):
+        """mp_set_summaries: accumulate the latent state at the end of sweeps first_sweep, first_sweep + thin, ... (thin=0: off).
+        Zeroes the sums."""
+        self._ck(self.lib.mp_set_summaries(self.h, int(first_sweep), int(thin)), "mp_set_summaries")
+
+    def summaries(self, reset=False):
+        """mp_get_summaries: dict(nsamples, z_count [T, N] uint32, z_prob [T, N], y_count [T-1, N] uint32, S_sum [T-1, N]),
+        sums over the accumulated sweeps and this engine's chains; z_prob / nsamples is the posterior occupancy."""
+        ns = C.c_int64()
+        zc = np.zeros((self.T, self.N), dtype=np.uint32)
+        zp = np.zeros((self.T, self.N))
+        yc = np.zeros((self.T - 1, self.N), dtype=np.uint32)
+        ss = np.zeros((self.T - 1, self.N))
+        u32p = C.POINTER(C.c_uint32)
+        self._ck(self.lib.mp_get_summaries(self.h, C.byref(ns), _p(zc, u32p), _p(zp, _dp), _p(yc, u32p), _p(ss, _dp), int(reset)),
+                 "mp_get_summaries")
+        return dict(nsamples=ns.value, z_count=zc, z_prob=zp, y_count=yc, S_sum=ss)
 
     @staticmethod
     def _one_param(p):
