@@ -24,6 +24,7 @@
  *   mp_simulate               future.c:64-110 (simpij) + :359-386 (simulation loop)
  *   mp_forecast               future.c:359-386 at large N: the simulation loop started from the sampler's own chains
  *   mp_set_summaries / mp_get_summaries   (no counterpart) posterior occupancy, survival and connectivity of every patch-year
+ *   mp_set_waic / mp_get_waic  Rscript/hypothesis_test.R at large N: pointwise predictive densities for WAIC
  *
  * All device memory is owned by the engine handle; host buffers are owned by the caller.  One
  * handle per GPU / host thread (thread-compatible, not thread-safe).  There is no CPU fallback:
@@ -204,6 +205,32 @@ int mp_set_summaries(mp_engine *h, int first_sweep, int thin);
  * when the queued sweeps could push nsamples past 2^32 - 1, the limit of the uint32 counts. */
 int mp_get_summaries(mp_engine *h, int64_t *nsamples, uint32_t *z_count, double *z_prob, uint32_t *y_count,
                      double *S_sum, int reset);
+/* Pointwise predictive densities of the observations for WAIC (no reference counterpart: the large-N counterpart of the
+ * model comparison of Rscript/hypothesis_test.R), accumulated on the device at the end of every qualifying sweep, summed
+ * over this engine's chains.  first_sweep / thin as for mp_set_summaries; thin = 0 switches them off and frees them;
+ * setting them zeroes the sums, and so does mp_set_observations while they are on.  For every observed cell (obs 0 or 1,
+ * year 0 included) a sample adds the density p of the observation given the chain's state of the previous year:
+ *   pi = p0 (year 0);  pi = s + (1 - s) C_{t-1,k},  s = z_{t-1,k} (1 - E_{t-1})  (t >= 1, E and C of transition t-1,
+ *        C from the S the sweep ends with)
+ *   p  = q pi (obs 1),  1 - q pi (obs 0),  q = p (detection on) or 1
+ * This is a conditional predictive: values compare only between fits to the same observations and prior_occ.
+ * One kernel per qualifying sweep, counted under MP_K_SMALL; without WAIC a sweep launches exactly what it launched before.
+ * Device memory: T N 24 + 8 bytes.  mp_forecast, mp_connectivity, mp_loglik, mp_loglik_host, mp_simulate* and mp_flip_delta
+ * leave the sums unchanged.  mp_sweep_sharded[_all] ranks hold identical sums; chain-sharded engines add theirs.
+ * MP_ERR_ARG: first_sweep < 0 or thin < 0.  MP_ERR_STATE: switched on before mp_set_observations. */
+int mp_set_waic(mp_engine *h, int first_sweep, int thin);
+/* Copy (and with reset != 0 zero) the sums.  Every output is nullable; each array is T*N, 0 in cells that are not
+ * observations.  Synchronous, after any queued sweeps.
+ *   nsamples    accumulated sweeps x n_chains (S)
+ *   lik_sum     L_i = sum of p
+ *   loglik_sum  G_i = sum of log p
+ *   loglik_sq   Q_i = sum of (log p)^2
+ * Reduction (Watanabe 2010; Vehtari, Gelman and Gabry 2017), over the observed cells i, after adding the arrays of
+ * chain-sharded engines:  lppd_i = log(L_i / S),  p_waic_i = max(0, (Q_i - G_i^2 / S) / (S - 1)) (needs S >= 2),
+ * elpd_i = lppd_i - p_waic_i;  elpd_waic = sum_i elpd_i, waic = -2 elpd_waic.  Two fits A, B to the same observations:
+ * delta = sum_i (elpd_i^A - elpd_i^B), se = sqrt(n_obs var_i(elpd_i^A - elpd_i^B)).
+ * MP_ERR_STATE: WAIC sums not set. */
+int mp_get_waic(mp_engine *h, int64_t *nsamples, double *lik_sum, double *loglik_sum, double *loglik_sq, int reset);
 
 /* ---- forward simulator ---- */
 /* nsims independent trajectories of nyears from z0 (N bytes); era_all != 0 applies K/Ksrc every

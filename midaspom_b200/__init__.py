@@ -6,6 +6,8 @@ The product is ``lib/libmidaspom_cuda.so`` (hand-written sm_100a CUDA, built in-
 """
 from .engine import (Engine, MpConfig, MpParams, MpSamplerConfig, MpError, load_library, GEOM_LINEAR, GEOM_COORDS,
                      GEOM_DENSE, FP32, FP64, NDRAW, NLSIG, NPART, KERNEL_CATEGORIES, ABI_SYMBOLS, exact_posterior, exact_variant)
+from .waic import waic, compare_waic
 
 __all__ = ["Engine", "MpConfig", "MpParams", "MpSamplerConfig", "MpError", "load_library", "GEOM_LINEAR",
-           "GEOM_COORDS", "GEOM_DENSE", "FP32", "FP64", "NDRAW", "NLSIG", "NPART", "KERNEL_CATEGORIES", "ABI_SYMBOLS", "exact_posterior", "exact_variant"]
+           "GEOM_COORDS", "GEOM_DENSE", "FP32", "FP64", "NDRAW", "NLSIG", "NPART", "KERNEL_CATEGORIES", "ABI_SYMBOLS", "exact_posterior", "exact_variant",
+           "waic", "compare_waic"]

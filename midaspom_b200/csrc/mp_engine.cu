@@ -471,6 +471,20 @@ template <typename R> static int launch_summaries(mp_engine *h)
     if (summary_due(h, h->sweep)) h->sum_samples += nC(h);
     return MP_OK;
 }
+// ---- pointwise predictive densities for WAIC (mp_set_waic): lik, loglik, loglik_sq [T][N] doubles, then the uint64 sample
+// counter: T N 24 + 8 bytes
+static size_t waic_bytes(const mp_engine *h) { return zcells(h) * 24 + 8; }
+template <typename R> static int launch_waic(mp_engine *h)
+{
+    WaicBufs b;
+    b.lik = (double *)h->d_waic; b.loglik = b.lik + zcells(h); b.loglik_sq = b.loglik + zcells(h);
+    b.nsamples = (unsigned long long *)(b.loglik_sq + zcells(h));
+    const long long threads = (long long)nT(h) * (long long)((nN(h) + 3) / 4);
+    k_waic<R><<<(unsigned)((threads + 255) / 256), 256, 0, h->stream>>>(sampler_dev(h), h->d_ctr, h->waic_first, h->waic_thin,
+        view<R>(h), h->d_par, h->d_obs, h->have_era ? h->d_era : nullptr, h->d_z, h->d_S[0], h->cfg.n_years, h->cfg.n_chains, b);
+    CK(cudaGetLastError());
+    return MP_OK;
+}
 
 // phase 3: e and p from the sufficient counts, record the draw
 template <typename R> static int phase_finish(mp_engine *h)
@@ -494,6 +508,10 @@ template <typename R> static int phase_finish(mp_engine *h)
         if (h->sum_thin > 0) {
             h->t_launch[MP_K_SMALL]++;
             if ((rc = launch_summaries<R>(h)) != MP_OK) return rc;
+        }
+        if (h->waic_thin > 0) {                              // the same for the WAIC sums
+            h->t_launch[MP_K_SMALL]++;
+            if ((rc = launch_waic<R>(h)) != MP_OK) return rc;
         }
         k_advance<<<1, 1, 0, h->stream>>>(h->d_ctr, h->cfg.max_draws);
         CK(cudaGetLastError());
@@ -536,7 +554,7 @@ int mp_destroy(mp_engine *h)
     for (auto e : h->pool) cudaEventDestroy(e);
     void *ptrs[] = { h->d_area, h->d_src_unit, h->d_px, h->d_py, h->d_dist, h->d_obs, h->d_era, h->d_par, h->d_prop,
                      h->d_lsig, h->d_z, h->d_y, h->d_srec, h->d_S[0], h->d_S[1], h->d_aw[0], h->d_aw[1], h->d_partial[0],
-                     h->d_partial[1], h->d_llc, h->d_logu, h->d_parts, h->d_scalar, h->d_flags, h->d_counts, h->d_draws, h->d_cand, h->d_cand_count, h->d_task_order, h->d_ljac, h->d_perm, h->d_scan, h->d_minv, h->d_tile_box, h->d_mlow, h->d_work, h->d_gemm, h->d_tlist, h->d_btasks, h->d_blockmode, h->d_scan_work, h->d_comm_send, h->d_comm_recv, h->d_ctr, h->d_sum };
+                     h->d_partial[1], h->d_llc, h->d_logu, h->d_parts, h->d_scalar, h->d_flags, h->d_counts, h->d_draws, h->d_cand, h->d_cand_count, h->d_task_order, h->d_ljac, h->d_perm, h->d_scan, h->d_minv, h->d_tile_box, h->d_mlow, h->d_work, h->d_gemm, h->d_tlist, h->d_btasks, h->d_blockmode, h->d_scan_work, h->d_comm_send, h->d_comm_recv, h->d_ctr, h->d_sum, h->d_waic };
     for (void *p : ptrs) if (p) cudaFree(p);
     if (h->stream) cudaStreamDestroy(h->stream);
     delete h;
@@ -884,6 +902,7 @@ int mp_set_observations(mp_engine *h, const int8_t *obs)
     REQUIRE(obs, MP_ERR_ARG, "null observations");
     for (size_t i = 0; i < zcells(h); i++) REQUIRE(obs[i] >= -1 && obs[i] <= 1, MP_ERR_ARG, "observations must be -1, 0 or 1");
     CK(cudaMemcpyAsync(h->d_obs, obs, zcells(h), cudaMemcpyHostToDevice, h->stream));
+    if (h->d_waic) CK(cudaMemsetAsync(h->d_waic, 0, waic_bytes(h), h->stream));   // sums over other observations mean nothing now
     CK(cudaStreamSynchronize(h->stream));
     h->have_obs = true;
     return MP_OK;
@@ -1344,6 +1363,43 @@ int mp_get_summaries(mp_engine *h, int64_t *nsamples, uint32_t *z_count, double 
     CK(cudaStreamSynchronize(h->stream));
     if (nsamples) *nsamples = (int64_t)ns;
     if (reset) h->sum_samples = 0;
+    return MP_OK;
+}
+int mp_set_waic(mp_engine *h, int first_sweep, int thin)
+{
+    if (!h) return MP_ERR_ARG;
+    REQUIRE(first_sweep >= 0 && thin >= 0, MP_ERR_ARG, "mp_set_waic: first_sweep and thin must be >= 0");
+    REQUIRE(thin == 0 || h->have_obs, MP_ERR_STATE, "mp_set_waic: no observations (mp_set_observations)");
+    CK(cudaSetDevice(h->cfg.device));
+    int rc = quiesce(h);                                 // the captured sweeps launch k_waic or not: capture again
+    if (rc != MP_OK) return rc;
+    h->waic_first = first_sweep; h->waic_thin = thin;
+    if (thin == 0) {
+        if (h->d_waic) { CK(cudaFree(h->d_waic)); h->d_waic = nullptr; }
+        return MP_OK;
+    }
+    if (!h->d_waic) {
+        cudaError_t e = cudaMalloc(&h->d_waic, waic_bytes(h));
+        if (e != cudaSuccess) { h->d_waic = nullptr; h->waic_thin = 0; h->err = std::string("mp_set_waic: ") + cudaGetErrorString(e); return MP_ERR_CUDA; }
+    }
+    CK(cudaMemsetAsync(h->d_waic, 0, waic_bytes(h), h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    return MP_OK;
+}
+int mp_get_waic(mp_engine *h, int64_t *nsamples, double *lik_sum, double *loglik_sum, double *loglik_sq, int reset)
+{
+    if (!h) return MP_ERR_ARG;
+    REQUIRE(h->d_waic, MP_ERR_STATE, "mp_get_waic: WAIC sums not set (mp_set_waic)");
+    CK(cudaSetDevice(h->cfg.device));
+    const size_t plane = zcells(h) * 8;
+    unsigned long long ns = 0;
+    CK(cudaMemcpyAsync(&ns, h->d_waic + 3 * plane, 8, cudaMemcpyDeviceToHost, h->stream));
+    if (lik_sum) CK(cudaMemcpyAsync(lik_sum, h->d_waic, plane, cudaMemcpyDeviceToHost, h->stream));
+    if (loglik_sum) CK(cudaMemcpyAsync(loglik_sum, h->d_waic + plane, plane, cudaMemcpyDeviceToHost, h->stream));
+    if (loglik_sq) CK(cudaMemcpyAsync(loglik_sq, h->d_waic + 2 * plane, plane, cudaMemcpyDeviceToHost, h->stream));
+    if (reset) CK(cudaMemsetAsync(h->d_waic, 0, waic_bytes(h), h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    if (nsamples) *nsamples = (int64_t)ns;
     return MP_OK;
 }
 int mp_num_draws(mp_engine *h) { return h ? h->ndraws : MP_ERR_ARG; }

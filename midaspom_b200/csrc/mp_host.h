@@ -105,6 +105,9 @@ struct mp_engine {
     unsigned char *d_sum = nullptr;
     int sum_first = 0, sum_thin = 0;  // sum_thin == 0: off
     unsigned long long sum_samples = 0;   // host mirror of the device sample counter, queued sweeps included
+    // pointwise predictive densities for WAIC (mp_set_waic): lik, loglik, loglik_sq [T][N] and the uint64 sample counter
+    unsigned char *d_waic = nullptr;
+    int waic_first = 0, waic_thin = 0;    // waic_thin == 0: off
     // timing
     bool timing = false;
     struct Span { cudaEvent_t a, b; int cat; };

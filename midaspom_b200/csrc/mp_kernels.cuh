@@ -8,6 +8,7 @@
 //  k_sweep_y       Gibbs scan of y_t | z with rank-1 updates of S_t in shared memory
 //  k_update_z      Gibbs update of latent occupancy cells (conditionally independent given y)
 //  k_summaries     posterior sums of z, P(z = 1 | y, theta), y and S over the chains (mp_set_summaries)
+//  k_waic          sums of the pointwise predictive density of every observation, its log and squared log (mp_set_waic)
 //  k_propose_* / k_decide_* / k_update_ep / k_record   Metropolis bookkeeping, one warp per chain
 //  k_sim_init / k_sim_ext / k_sim_col   forward simulator (future.c:64-110)
 //  k_fc_init / k_fc_ext / k_fc_col      posterior-predictive forecast from the chains (with k_pack_sources + k_conn)
@@ -387,6 +388,30 @@ __device__ __forceinline__ double z_logodds(const SamplerDev &sd, const Landscap
     if (sd.detect && o == 0) lod += log(1.0 - p.p);
     return lod;
 }
+// Log predictive density of the observation o (0 or 1) of cell (t, k) given the chain's state of the previous year (DESIGN
+// §2, WAIC): pi = p0 in year 0; for t >= 1 pi = s + (1 - s) C with s = z_{t-1,k} (1 - E_{t-1}), which marginalises the
+// patch's own y_{t-1,k} (S excludes the patch itself).  C is formed in R exactly as z_logodds forms it, the rest in FP64;
+// p = q pi for o = 1, 1 - q pi for o = 0 (its log by log1p), q the detection probability (1 without detection).  Returns
+// log p and writes p to dens.
+template <typename R>
+__device__ __forceinline__ double obs_logpred(const SamplerDev &sd, const Landscape<R> &ls, const mp_params &p, const Trans<R> &tr0,
+                                              const Trans<R> &tr1, const uint8_t *__restrict__ era, const double *__restrict__ Sc,
+                                              int o, bool zprev, long long i, int t, int k, double &dens)
+{
+    double pi = sd.p0;
+    if (t > 0) {
+        const bool pre = era ? era[t - 1] != 0 : false;
+        const Trans<R> tr = pick_trans<R>(tr0, tr1, pre);
+        const double C = (double)col_prob<R>(tr, (R)Sc[i - ls.n], source_term<R>(ls, tr, k));
+        double E = pre ? p.e / p.K : p.e;
+        if (E > 1.0) E = 1.0;
+        const double s = zprev ? 1.0 - E : 0.0;
+        pi = s + (1.0 - s) * C;
+    }
+    const double qpi = sd.detect ? p.p * pi : pi;
+    dens = o ? qpi : 1.0 - qpi;
+    return o ? log(qpi) : log1p(-qpi);
+}
 // z_tk | y, theta for every latent cell at once: S depends on y only, so the cells are
 // conditionally independent.  Forced to 1 when an adjacent intermediate state is 1.
 template <typename R>
@@ -422,6 +447,11 @@ struct SumBufs {
     uint32_t *z_count, *y_count;
     unsigned long long *nsamples;
 };
+// whether sweep s adds to sums set with (first, thin > 0): the gate of k_summaries and k_waic
+__device__ __forceinline__ bool sweep_due(uint32_t s, int first, int thin)
+{
+    return s >= (uint32_t)first && (s - (uint32_t)first) % (uint32_t)thin == 0;
+}
 // 4 bytes of a row of z or y, byte j = patch k0 + j (m <= 4 valid patches); rows start on a 4-byte boundary when n % 4 == 0
 __device__ __forceinline__ uint32_t load_cells4(const uint8_t *__restrict__ p, int m, bool words)
 {
@@ -439,8 +469,7 @@ k_summaries(SamplerDev sd, const uint32_t *__restrict__ sweep_p /* device-reside
             Landscape<R> ls, const mp_params *__restrict__ par, const int8_t *__restrict__ obs, const uint8_t *__restrict__ era,
             const uint8_t *__restrict__ z, const uint8_t *__restrict__ y, const double *__restrict__ S, int T, int nchains, SumBufs b)
 {
-    const uint32_t s = *sweep_p;
-    if (s < (uint32_t)first || (s - (uint32_t)first) % (uint32_t)thin) return;
+    if (!sweep_due(*sweep_p, first, thin)) return;
     const int n = ls.n, ntrans = T - 1, nq = (n + 3) >> 2;
     const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (idx == 0) *b.nsamples += (unsigned long long)nchains;
@@ -493,6 +522,58 @@ k_summaries(SamplerDev sd, const uint32_t *__restrict__ sweep_p /* device-reside
             b.z_count[row + j] = zc[j]; b.z_prob[row + j] = zp[j];
             if (has_y) { b.y_count[row + j] = yc[j]; b.S_sum[row + j] = ss[j]; }
         }
+}
+
+// ------------------------------------------------------------------ pointwise predictive densities for WAIC (mp_set_waic)
+// Sums over this engine's chains and the qualifying sweeps (the gate of k_summaries), per observed cell (obs 0 or 1):
+// lik = sum p, loglik = sum log p, loglik_sq = sum (log p)^2, p from obs_logpred.  Layout [year][patch]; cells that are
+// not observations are never written.
+struct WaicBufs {
+    double *lik, *loglik, *loglik_sq;
+    unsigned long long *nsamples;
+};
+// One thread per (year, 4 consecutive patches), the chains in order c = 0 .. C-1, only its own cells: no atomics, the sums
+// do not depend on the launch geometry.  Reads z of the previous year and S of the previous transition.
+template <typename R>
+__global__ void __launch_bounds__(256)
+k_waic(SamplerDev sd, const uint32_t *__restrict__ sweep_p /* device-resident sweep counter (k_advance) */, int first, int thin,
+       Landscape<R> ls, const mp_params *__restrict__ par, const int8_t *__restrict__ obs, const uint8_t *__restrict__ era,
+       const uint8_t *__restrict__ z, const double *__restrict__ S, int T, int nchains, WaicBufs b)
+{
+    if (!sweep_due(*sweep_p, first, thin)) return;
+    const int n = ls.n, ntrans = T - 1, nq = (n + 3) >> 2;
+    const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (idx == 0) *b.nsamples += (unsigned long long)nchains;
+    if (idx >= (long long)T * nq) return;
+    const int t = (int)(idx / nq), k0 = 4 * (int)(idx - (long long)t * nq), m = min(4, n - k0);
+    const bool words = (n & 3) == 0;
+    const size_t row = (size_t)t * n + k0;
+    int o[4];
+    bool any = false;
+    double L[4] = { 0, 0, 0, 0 }, G[4] = { 0, 0, 0, 0 }, Q[4] = { 0, 0, 0, 0 };
+#pragma unroll
+    for (int j = 0; j < 4; j++) {
+        o[j] = j < m ? obs[row + j] : -1;
+        if (o[j] >= 0) { any = true; L[j] = b.lik[row + j]; G[j] = b.loglik[row + j]; Q[j] = b.loglik_sq[row + j]; }
+    }
+    if (!any) return;
+    for (int c = 0; c < nchains; c++) {
+        const uint32_t zprev = t > 0 ? load_cells4(z + (size_t)c * T * n + row - n, m, words) : 0u;
+        const double *Sc = S + (size_t)c * ntrans * n;
+        const mp_params p = par[c];
+        const Trans<R> tr0 = make_trans<R>(p, 0), tr1 = make_trans<R>(p, 1);
+#pragma unroll
+        for (int j = 0; j < 4; j++) {
+            if (o[j] < 0) continue;
+            double pd;
+            const double lp = obs_logpred<R>(sd, ls, p, tr0, tr1, era, Sc, o[j], ((zprev >> (8 * j)) & 0xffu) != 0u,
+                                             (long long)(row + j), t, k0 + j, pd);
+            L[j] += pd; G[j] += lp; Q[j] += lp * lp;
+        }
+    }
+#pragma unroll
+    for (int j = 0; j < 4; j++)
+        if (o[j] >= 0) { b.lik[row + j] = L[j]; b.loglik[row + j] = G[j]; b.loglik_sq[row + j] = Q[j]; }
 }
 
 // ------------------------------------------------------------------ rank-1 flip of the intermediate state

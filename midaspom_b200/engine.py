@@ -33,7 +33,7 @@ ABI_SYMBOLS = (
     "mp_get_scan_order", "mp_get_work_counters", "mp_get_scan_geometry", "mp_get_conn_path", "mp_set_scan_blocks",
     "mp_comm_unique_id", "mp_comm_init", "mp_comm_init_all", "mp_comm_destroy", "mp_comm_rank", "mp_comm_size", "mp_comm_last_error",
     "mp_gather_draws", "mp_gather_draws_all", "mp_sweep_sharded", "mp_sweep_sharded_all", "mp_forecast",
-    "mp_set_summaries", "mp_get_summaries",
+    "mp_set_summaries", "mp_get_summaries", "mp_set_waic", "mp_get_waic",
 )
 
 
@@ -132,6 +132,8 @@ def load_library(build_if_missing: bool = True) -> C.CDLL:
     L.mp_forecast.argtypes = [vp, C.c_int, C.c_int, C.c_uint64, dp, C.POINTER(C.c_int32), C.POINTER(C.c_uint32)]
     L.mp_set_summaries.argtypes = [vp, C.c_int, C.c_int]
     L.mp_get_summaries.argtypes = [vp, C.POINTER(C.c_int64), C.POINTER(C.c_uint32), dp, C.POINTER(C.c_uint32), dp, C.c_int]
+    L.mp_set_waic.argtypes = [vp, C.c_int, C.c_int]
+    L.mp_get_waic.argtypes = [vp, C.POINTER(C.c_int64), dp, dp, dp, C.c_int]
     L.mp_device_ptr.argtypes = [vp, C.c_int, C.POINTER(vp), C.POINTER(C.c_size_t)]
     L.mp_get_stream.argtypes = [vp, C.POINTER(vp)]
     L.mp_set_timing.argtypes = [vp, C.c_int]
@@ -492,6 +494,20 @@ class Engine:
         self._ck(self.lib.mp_get_summaries(self.h, C.byref(ns), _p(zc, u32p), _p(zp, _dp), _p(yc, u32p), _p(ss, _dp), int(reset)),
                  "mp_get_summaries")
         return dict(nsamples=ns.value, z_count=zc, z_prob=zp, y_count=yc, S_sum=ss)
+
+    # -- pointwise predictive densities for WAIC
+    def set_waic(self, first_sweep=0, thin=1):
+        """mp_set_waic: accumulate the predictive density of every observation at the end of sweeps first_sweep,
+        first_sweep + thin, ... (thin=0: off).  Zeroes the sums."""
+        self._ck(self.lib.mp_set_waic(self.h, int(first_sweep), int(thin)), "mp_set_waic")
+
+    def waic_sums(self, reset=False):
+        """mp_get_waic: dict(nsamples, lik_sum, loglik_sum, loglik_sq [T, N]), sums over the accumulated sweeps and this engine's
+        chains, 0 in cells that are not observations; reduce them with midaspom_b200.waic."""
+        ns = C.c_int64()
+        out = [np.zeros((self.T, self.N)) for _ in range(3)]
+        self._ck(self.lib.mp_get_waic(self.h, C.byref(ns), *[_p(a, _dp) for a in out], int(reset)), "mp_get_waic")
+        return dict(nsamples=ns.value, lik_sum=out[0], loglik_sum=out[1], loglik_sq=out[2])
 
     @staticmethod
     def _one_param(p):
