@@ -197,7 +197,18 @@ __global__ void __launch_bounds__(NTHR) k_conn(ConnArgs<R> a)
         const int g0 = slot0 / 32, ngroups = (n + 31) / 32;
         const float b = (float)parp[c].b;
         const float law_max = fmaxf(b * log2f(a.area_max), b * log2f(a.area_min)) + 1e-3f;     // log2 of max_l A_l^b, rounded up
-        auto thr_of = [&](int g) { return CONN_CULL_LOG2 + log2f(a.mlow[(size_t)c * ngroups + g]) - law_max; };   // log2f(0) = -inf
+        // mlow bounds the resident S, which belongs to the current parameters (set 0).  For the proposal (set 1) it becomes a
+        // bound of S' through w' = w^p A^(b' - p b) with p = alpha' / alpha: S' >= A^(b' - p b)_min S^p for p <= 1, since
+        // (sum w)^p <= sum w^p, and S' >= A^(b' - p b)_min n^(1 - p) S^p for p > 1 (power means over the n <= N sources).
+        // Without it a proposal with a larger alpha would be culled at 2^-30 of the current S rather than of its own.
+        float lscale = 1.f, loff = 0.f;
+        if (set == 1 && (parp[c].alpha != a.par[0][c].alpha || parp[c].b != a.par[0][c].b)) {
+            const double p = parp[c].alpha / a.par[0][c].alpha;
+            const float db = (float)(parp[c].b - p * a.par[0][c].b);
+            lscale = (float)p;
+            loff = fminf(db * log2f(a.area_max), db * log2f(a.area_min)) - (p > 1.0 ? (float)(p - 1.0) * log2f((float)n) : 0.f) - 1e-3f;
+        }
+        auto thr_of = [&](int g) { return CONN_CULL_LOG2 + lscale * log2f(a.mlow[(size_t)c * ngroups + g]) + loff - law_max; };   // log2f(0) = -inf
         tbox = a.box32[g0]; thr_cta = thr_of(g0);
         for (int i = 1; i < NTHR * TGT / 32; i++)
             if (g0 + i < gend) { tbox = box_union(tbox, a.box32[g0 + i]); thr_cta = fminf(thr_cta, thr_of(g0 + i)); }
