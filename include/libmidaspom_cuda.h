@@ -25,6 +25,7 @@
  *   mp_forecast               future.c:359-386 at large N: the simulation loop started from the sampler's own chains
  *   mp_set_summaries / mp_get_summaries   (no counterpart) posterior occupancy, survival and connectivity of every patch-year
  *   mp_set_waic / mp_get_waic  Rscript/hypothesis_test.R at large N: pointwise predictive densities for WAIC
+ *   mp_ppc                    (no counterpart) posterior-predictive replicates of the observation table from the chains
  *
  * All device memory is owned by the engine handle; host buffers are owned by the caller.  One
  * handle per GPU / host thread (thread-compatible, not thread-safe).  There is no CPU fallback:
@@ -262,6 +263,31 @@ int mp_simulate_ensemble(mp_engine *h, const mp_params *par_per_sim /* nsims */,
  * MP_ERR_STATE: no landscape, no chain state, a chain with alpha <= 0. */
 int mp_forecast(mp_engine *h, int nyears, int nrep, uint64_t seed, const double *scenario,
                 int32_t *occupied_out, uint32_t *incidence_out);
+/* Posterior-predictive check of the fit (no reference counterpart): nrep replicates per chain of the whole observation table,
+ * simulated from the chain's own imputed year 0 and resident parameters under the fit's own era flags, observed through the
+ * table's missing-cell mask and, with detection on, the chain's p (DESIGN.md §2 defines every step and statistic).
+ * Trajectory (c, r) is simulation number (chain_offset + c) * nrep + r under `seed`, the numbering of mp_forecast, so results do
+ * not depend on how chains are sharded.  Statistics, integers per (chain, replicate, year t):
+ *   0 detected   observed cells with rep_tk = 1
+ *   1 colonised  cells observed in t-1 and t with rep 0 -> 1 (0 in year 0)
+ *   2 extinct    cells observed in t-1 and t with rep 1 -> 0 (0 in year 0)
+ * stats_out      (nullable): n_chains * nrep * T * MP_NPPC int32, [chain][replicate][year][statistic]
+ * obs_stats_out  (nullable): T * MP_NPPC int32, the same statistics of the observation table itself
+ * patch_ge / patch_gt (nullable): N uint32 each, the number of this engine's replicates whose count of years observed occupied,
+ *   D_k = sum_t [rep_tk = 1], is >= / > that of the observations, sum_t [obs_tk = 1].  Chain-sharded engines add theirs.
+ * Replicates start from the chains' imputed year 0, so without detection their year 0 reproduces the observed cells exactly: the
+ * check concerns years 1 .. T-1.
+ * Leaves all sampler state as it was: chain state, S and its validity flags, draws, sweep counter, scales, captured graphs, the
+ * summaries and the WAIC sums.  Synchronous, on the engine stream after any queued sweeps.  Each transition runs mp_forecast's
+ * year (k_conn shared by a chain's replicates; FP32 engines on landscapes with positions cull it with the floor of DESIGN.md §5,
+ * MP_CONN_CULL=0 disables), then one observation kernel per year.  Counted under MP_K_SIM and in MP_CNT_CONN_*; mp_set_shard does
+ * not apply.  Device memory: one arena per call of mp_forecast's size plus C nrep N 4 bytes of per-replicate records and
+ * C nrep T MP_NPPC 4 bytes of statistics.
+ * MP_ERR_ARG: nrep < 1 or > 65535, (chain_offset + n_chains) * nrep >= 2^32.
+ * MP_ERR_STATE: no observations, no landscape, no chain state, a chain with alpha <= 0. */
+#define MP_NPPC 3   /* detected, colonised, extinct */
+int mp_ppc(mp_engine *h, int nrep, uint64_t seed, int32_t *stats_out, int32_t *obs_stats_out, uint32_t *patch_ge,
+           uint32_t *patch_gt);
 
 /* ---- exact small-n engine: the reference's own algorithm (state enumeration on an (e,c) grid) ----
  * Replaces the whole hot loop of MIDASPOM.out, main_MIDASPOM.c:198-290 (state tables) and :341-395

@@ -20,7 +20,8 @@ namespace mp {
 // Counter-based RNG (Salmon et al., SC'11): the stream of a chain depends only on
 // (seed, global chain id, sweep, kind, cell) -- never on grid/block geometry.
 enum : uint32_t { RK_INIT_PARAM = 1, RK_INIT_Z = 2, RK_SIM_EXT = 3, RK_SIM_COL = 4, RK_Z = 5, RK_Y = 6,
-                  RK_AB = 7, RK_C = 8, RK_E = 9, RK_P = 10, RK_K = 11, RK_KSRC = 12, RK_DSRC = 13 };
+                  RK_AB = 7, RK_C = 8, RK_E = 9, RK_P = 10, RK_K = 11, RK_KSRC = 12, RK_DSRC = 13,
+                  RK_PPC_DET = 14 };
 
 __host__ __device__ inline uint32_t mulhi32(uint32_t a, uint32_t b)
 {

@@ -1494,12 +1494,15 @@ int mp_simulate_ensemble(mp_engine *h, const mp_params *par_per_sim, const uint8
     return simulate_impl(h, par_per_sim, 1, z0_per_sim, nyears, nsims, seed, era_all, z_out, occupied_out);
 }
 
-// ---- posterior-predictive forecast from the chains' own state
+// ---- replicates of the chains' own state: the year loop of mp_forecast and mp_ppc
 // Buffers of one call (one arena); states and S are [chain][replicate][patch], records [chain][word][padded slot]
 struct FcBufs {
     const mp_params *par; void *aw; uint8_t *zc, *yc; double *S; void *rec; float *mlow; int32_t *occ; uint32_t *inc;
 };
-extern "C++" template <typename R> int forecast_t(mp_engine *h, const FcBufs &b, int nyears, int nrep, uint64_t seed, int era_all)
+// nyears transitions of nrep trajectories per chain from z[c][t0]; transition t applies K, Ksrc iff era[t].  after_year(t) runs
+// once the states of year t are in zc: t = 0 after the start states, t + 1 after the colonisation draws of transition t.
+extern "C++" template <typename R, typename F>
+int replicate_t(mp_engine *h, const FcBufs &b, int t0, int nyears, int nrep, uint64_t seed, const uint8_t *era, F after_year)
 {
     Timed tm(h, MP_K_SIM);
     const int n = h->cfg.n_patches, C = h->cfg.n_chains, T = h->cfg.n_years, npad = conn_npad(n), nwords = (nrep + 31) / 32;
@@ -1509,9 +1512,11 @@ extern "C++" template <typename R> int forecast_t(mp_engine *h, const FcBufs &b,
     if (h->geom != MP_GEOM_COORDS) { lsrc.px = nullptr; lsrc.py = nullptr; }
     k_area_weights<R><<<dim3(tiles, C), 256, 0, h->stream>>>(b.par, h->have_area ? h->d_area : nullptr, (R *)b.aw, n);
     CK(cudaGetLastError());
-    k_fc_init<<<dim3(tiles, C), 256, 0, h->stream>>>(h->d_z, T, n, nrep, nyears, b.zc, b.occ, b.inc);
+    k_fc_init<<<dim3(tiles, C), 256, 0, h->stream>>>(h->d_z, T, t0, n, nrep, nyears, b.zc, b.occ, b.inc);
     CK(cudaGetLastError());
-    // k_conn over the forecast's own buffers: every target, the replicates in place of the years, the forecast's culling floor
+    int rc;
+    if ((rc = after_year(0)) != MP_OK) return rc;
+    // k_conn over the call's own buffers: every target, the replicates in place of the years, the call's culling floor
     ConnArgs<R> a;
     a.ls = ls;
     a.par[0] = a.par[1] = b.par;
@@ -1522,9 +1527,8 @@ extern "C++" template <typename R> int forecast_t(mp_engine *h, const FcBufs &b,
     a.perm = h->d_perm; a.box32 = (const float4 *)h->d_tile_box;
     a.mlow = b.mlow; a.area_max = (float)h->area_max; a.area_min = (float)h->area_min;
     a.stats = h->d_work;
-    int rc;
     for (int t = 0; t < nyears; t++) {
-        k_fc_ext<R><<<dim3(tiles, nrep, C), 256, 0, h->stream>>>(b.par, n, nrep, seed, sim0, t, era_all, b.zc, b.yc);
+        k_fc_ext<R><<<dim3(tiles, nrep, C), 256, 0, h->stream>>>(b.par, n, nrep, seed, sim0, t, era[t], b.zc, b.yc);
         CK(cudaGetLastError());
         k_pack_sources<R><<<dim3((npad + 255) / 256, C, nwords), 256, 0, h->stream>>>(lsrc, h->d_perm, (const R *)b.aw, nullptr, b.yc, nrep,
                                                                                       nwords, 1, (SrcRec<R> *)b.rec);
@@ -1535,11 +1539,54 @@ extern "C++" template <typename R> int forecast_t(mp_engine *h, const FcBufs &b,
         default: rc = launch_conn_args<R, MP_GEOM_DENSE>(h, a, 1, false); break;
         }
         if (rc != MP_OK) return rc;
-        k_fc_col<R><<<dim3(tiles, C), 256, 0, h->stream>>>(ls, b.par, nrep, seed, sim0, t, nyears, era_all, b.S, b.yc, b.zc, b.occ, b.inc);
+        k_fc_col<R><<<dim3(tiles, C), 256, 0, h->stream>>>(ls, b.par, nrep, seed, sim0, t, nyears, era[t], b.S, b.yc, b.zc, b.occ, b.inc);
         CK(cudaGetLastError());
+        if ((rc = after_year(t + 1)) != MP_OK) return rc;
     }
     return MP_OK;
 }
+// The part of a call's arena that replicate_t needs: parameters, A^b, current / surviving states, S, source records, culling
+// floor.  rep_carve reserves it at the front of the arena, rep_upload points b at it and uploads the parameters and the floor.
+struct RepLayout { size_t par, aw, zc, yc, S, rec, mlow; };
+extern "C++" template <typename F> RepLayout rep_carve(const mp_engine *h, int nrep, F carve)
+{
+    const size_t N = nN(h), C = nC(h), cells = C * (size_t)nrep * N, ngroups = (N + 31) / 32;
+    const size_t nwords = ((size_t)nrep + 31) / 32, npad = (size_t)conn_npad((int)N);
+    const size_t rec_bytes = is64(h) ? sizeof(SrcRec<double>) : sizeof(SrcRec<float>);
+    RepLayout L;
+    L.par = carve(C * sizeof(mp_params)); L.aw = carve(C * N * rsz(h)); L.zc = carve(cells); L.yc = carve(cells);
+    L.S = carve(cells * 8); L.rec = carve(C * nwords * npad * rec_bytes); L.mlow = carve(C * ngroups * sizeof(float));
+    return L;
+}
+// Culling floor of k_conn (FP32 engines with positions): a source group is skipped for a target group when every weight
+// between them is below 2^-30 mlow_c, so the skipped weights change c K_t S of a target by less than N 2^-30 mlow_c c Keff_c =
+// 2^-32 (the resolution of the uniform that decides a colonisation) with mlow_c = 2^-2 / (c Keff_c N), Keff_c >= every K_t of
+// chain c that the call applies.
+static int rep_upload(mp_engine *h, unsigned char *arena, const RepLayout &L, const std::vector<mp_params> &par,
+                      const std::vector<double> &Keff, FcBufs &b)
+{
+    const size_t N = nN(h), C = nC(h), ngroups = (N + 31) / 32;
+    std::vector<float> mlow(C * ngroups);
+    for (size_t c = 0; c < C; c++)
+        std::fill(mlow.begin() + c * ngroups, mlow.begin() + (c + 1) * ngroups, (float)std::min(0.25 / (par[c].c * Keff[c] * (double)N), 3.0e38));
+    b.par = (const mp_params *)(arena + L.par); b.aw = arena + L.aw; b.zc = arena + L.zc; b.yc = arena + L.yc;
+    b.S = (double *)(arena + L.S); b.rec = arena + L.rec; b.mlow = (float *)(arena + L.mlow);
+    b.occ = nullptr; b.inc = nullptr;
+    CK(cudaMemcpyAsync(arena + L.par, par.data(), C * sizeof(mp_params), cudaMemcpyHostToDevice, h->stream));
+    CK(cudaMemcpyAsync(b.mlow, mlow.data(), mlow.size() * sizeof(float), cudaMemcpyHostToDevice, h->stream));
+    return MP_OK;
+}
+// the chains' parameters after any queued sweeps
+static int chain_params(mp_engine *h, std::vector<mp_params> &par, const char *who)
+{
+    par.resize(nC(h));
+    CK(cudaMemcpyAsync(par.data(), h->d_par, nC(h) * sizeof(mp_params), cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    for (const mp_params &p : par) REQUIRE(p.alpha > 0.0, MP_ERR_STATE, std::string(who) + ": every chain needs alpha > 0");
+    return MP_OK;
+}
+
+// ---- posterior-predictive forecast from the chains' own state
 int mp_forecast(mp_engine *h, int nyears, int nrep, uint64_t seed, const double *scenario, int32_t *occupied_out, uint32_t *incidence_out)
 {
     if (!h) return MP_ERR_ARG;
@@ -1551,51 +1598,115 @@ int mp_forecast(mp_engine *h, int nyears, int nrep, uint64_t seed, const double 
     REQUIRE(!scenario || scenario[0] > 0.0, MP_ERR_ARG, "mp_forecast: the scenario needs K > 0");
     int rc = check_ready(h);
     if (rc != MP_OK) return rc;
-    const size_t N = nN(h), C = nC(h), cells = C * (size_t)nrep * N, ngroups = (N + 31) / 32;
-    const size_t nwords = ((size_t)nrep + 31) / 32, npad = (size_t)conn_npad((int)N);
-    // the chains' parameters after any queued sweeps; a scenario replaces K, Ksrc, dsrc and applies them every year
-    std::vector<mp_params> par(C);
-    CK(cudaMemcpyAsync(par.data(), h->d_par, C * sizeof(mp_params), cudaMemcpyDeviceToHost, h->stream));
-    CK(cudaStreamSynchronize(h->stream));
-    for (size_t c = 0; c < C; c++) {
-        REQUIRE(par[c].alpha > 0.0, MP_ERR_STATE, "mp_forecast: every chain needs alpha > 0");
-        if (scenario) { par[c].K = scenario[0]; par[c].Ksrc = scenario[1]; par[c].dsrc = scenario[2]; }
-    }
-    // Culling floor of k_conn (FP32 engines with positions): a source group is skipped for a target group when every weight
-    // between them is below 2^-30 mlow_c, so the skipped weights change c K S of a target by less than N 2^-30 mlow_c c K = 2^-32
-    // (the resolution of the uniform that decides a colonisation) with mlow_c = 2^-2 / (c K N); K = 1 without a scenario.
-    const double Keff = scenario ? scenario[0] : 1.0;
-    std::vector<float> mlow(C * ngroups);
-    for (size_t c = 0; c < C; c++)
-        std::fill(mlow.begin() + c * ngroups, mlow.begin() + (c + 1) * ngroups, (float)std::min(0.25 / (par[c].c * Keff * (double)N), 3.0e38));
-    // one arena per call: parameters, A^b, current / surviving states, S, source records, culling floor, outputs
+    const size_t N = nN(h), C = nC(h);
+    // a scenario replaces K, Ksrc, dsrc and applies them every year
+    std::vector<mp_params> par;
+    if ((rc = chain_params(h, par, "mp_forecast")) != MP_OK) return rc;
+    if (scenario)
+        for (mp_params &p : par) { p.K = scenario[0]; p.Ksrc = scenario[1]; p.dsrc = scenario[2]; }
+    const std::vector<double> Keff(C, scenario ? scenario[0] : 1.0);
+    const std::vector<uint8_t> era((size_t)nyears, scenario ? 1 : 0);
+    // one arena per call: replicate_t's buffers, outputs
     size_t off = 0;
     auto carve = [&](size_t bytes) { const size_t o = off; off += (bytes + 255) / 256 * 256; return o; };
-    const size_t rec_bytes = is64(h) ? sizeof(SrcRec<double>) : sizeof(SrcRec<float>);
+    const RepLayout L = rep_carve(h, nrep, carve);
     const size_t occ_bytes = C * (size_t)nrep * (nyears + 1) * 4, inc_bytes = (size_t)(nyears + 1) * N * 4;
-    const size_t o_par = carve(C * sizeof(mp_params)), o_aw = carve(C * N * rsz(h)), o_zc = carve(cells), o_yc = carve(cells),
-                 o_S = carve(cells * 8), o_rec = carve(C * nwords * npad * rec_bytes), o_mlow = carve(C * ngroups * sizeof(float)),
-                 o_occ = carve(occupied_out ? occ_bytes : 0), o_inc = carve(incidence_out ? inc_bytes : 0);
+    const size_t o_occ = carve(occupied_out ? occ_bytes : 0), o_inc = carve(incidence_out ? inc_bytes : 0);
     unsigned char *arena = nullptr;
     cudaError_t e;
 #define FCCK(call) if ((e = (call)) != cudaSuccess) { h->err = std::string(#call) + ": " + cudaGetErrorString(e); rc = MP_ERR_CUDA; goto done; }
     FCCK(cudaMalloc(&arena, std::max<size_t>(off, 256)));
     {
         FcBufs b;
-        b.par = (const mp_params *)(arena + o_par); b.aw = arena + o_aw; b.zc = arena + o_zc; b.yc = arena + o_yc;
-        b.S = (double *)(arena + o_S); b.rec = arena + o_rec; b.mlow = (float *)(arena + o_mlow);
+        if ((rc = rep_upload(h, arena, L, par, Keff, b)) != MP_OK) goto done;
         b.occ = occupied_out ? (int32_t *)(arena + o_occ) : nullptr; b.inc = incidence_out ? (uint32_t *)(arena + o_inc) : nullptr;
-        FCCK(cudaMemcpyAsync(arena + o_par, par.data(), C * sizeof(mp_params), cudaMemcpyHostToDevice, h->stream));
-        FCCK(cudaMemcpyAsync(b.mlow, mlow.data(), mlow.size() * sizeof(float), cudaMemcpyHostToDevice, h->stream));
         if (b.occ) FCCK(cudaMemsetAsync(b.occ, 0, occ_bytes, h->stream));
         if (b.inc) FCCK(cudaMemsetAsync(b.inc, 0, inc_bytes, h->stream));
-        rc = is64(h) ? forecast_t<double>(h, b, nyears, nrep, seed, scenario ? 1 : 0) : forecast_t<float>(h, b, nyears, nrep, seed, scenario ? 1 : 0);
+        auto none = [](int) { return MP_OK; };
+        const int t0 = h->cfg.n_years - 1;
+        rc = is64(h) ? replicate_t<double>(h, b, t0, nyears, nrep, seed, era.data(), none)
+                     : replicate_t<float>(h, b, t0, nyears, nrep, seed, era.data(), none);
         if (rc != MP_OK) goto done;
         if (occupied_out) FCCK(cudaMemcpyAsync(occupied_out, b.occ, occ_bytes, cudaMemcpyDeviceToHost, h->stream));
         if (incidence_out) FCCK(cudaMemcpyAsync(incidence_out, b.inc, inc_bytes, cudaMemcpyDeviceToHost, h->stream));
         FCCK(cudaStreamSynchronize(h->stream));
     }
 #undef FCCK
+done:
+    cudaStreamSynchronize(h->stream);
+    cudaFree(arena);
+    return rc;
+}
+
+// ---- posterior-predictive replicates of the observation table (DESIGN.md §2)
+int mp_ppc(mp_engine *h, int nrep, uint64_t seed, int32_t *stats_out, int32_t *obs_stats_out, uint32_t *patch_ge, uint32_t *patch_gt)
+{
+    if (!h) return MP_ERR_ARG;
+    CK(cudaSetDevice(h->cfg.device));
+    REQUIRE(nrep >= 1 && nrep <= 65535, MP_ERR_ARG, "mp_ppc: need 1 <= nrep <= 65535");
+    REQUIRE((uint64_t)(h->cfg.chain_offset + h->cfg.n_chains) * (uint64_t)nrep <= 0xffffffffull, MP_ERR_ARG,
+            "mp_ppc: simulation numbers (chain_offset + n_chains) * nrep must fit in 32 bits");
+    int rc = check_ready(h);
+    if (rc != MP_OK) return rc;
+    REQUIRE(h->have_obs, MP_ERR_STATE, "mp_ppc: observations not set");
+    const int T = h->cfg.n_years;
+    const size_t N = nN(h), C = nC(h);
+    std::vector<mp_params> par;
+    if ((rc = chain_params(h, par, "mp_ppc")) != MP_OK) return rc;
+    // the fit's era flags, transition by transition (none set: none apply)
+    std::vector<uint8_t> era((size_t)T, 0);
+    std::vector<int8_t> obs(T * N);
+    if (h->have_era) CK(cudaMemcpyAsync(era.data(), h->d_era, T - 1, cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaMemcpyAsync(obs.data(), h->d_obs, obs.size(), cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    bool any_era = false;
+    for (int t = 0; t + 1 < T; t++) any_era = any_era || era[t] != 0;
+    std::vector<double> Keff(C, 1.0);
+    if (any_era)
+        for (size_t c = 0; c < C; c++) Keff[c] = std::max(1.0, par[c].K);
+    if (obs_stats_out) {
+        std::fill(obs_stats_out, obs_stats_out + (size_t)T * MP_NPPC, 0);
+        for (int t = 0; t < T; t++)
+            for (size_t k = 0; k < N; k++) {
+                const int o = obs[t * N + k], op = t > 0 ? obs[(t - 1) * N + k] : -1;
+                obs_stats_out[t * MP_NPPC + 0] += o == 1;
+                if (o >= 0 && op >= 0) { obs_stats_out[t * MP_NPPC + 1] += op == 0 && o == 1; obs_stats_out[t * MP_NPPC + 2] += op == 1 && o == 0; }
+            }
+    }
+    // one arena per call: replicate_t's buffers, per-replicate records, statistics, per-patch counts
+    size_t off = 0;
+    auto carve = [&](size_t bytes) { const size_t o = off; off += (bytes + 255) / 256 * 256; return o; };
+    const RepLayout L = rep_carve(h, nrep, carve);
+    const size_t stats_bytes = C * (size_t)nrep * T * MP_NPPC * 4;
+    const size_t o_rec = carve(C * (size_t)nrep * N * 4), o_stats = carve(stats_bytes), o_ge = carve(N * 4), o_gt = carve(N * 4);
+    unsigned char *arena = nullptr;
+    cudaError_t e;
+#define PPCK(call) if ((e = (call)) != cudaSuccess) { h->err = std::string(#call) + ": " + cudaGetErrorString(e); rc = MP_ERR_CUDA; goto done; }
+    PPCK(cudaMalloc(&arena, std::max<size_t>(off, 256)));
+    {
+        FcBufs b;
+        if ((rc = rep_upload(h, arena, L, par, Keff, b)) != MP_OK) goto done;
+        uint32_t *rec = (uint32_t *)(arena + o_rec), *ge = (uint32_t *)(arena + o_ge), *gt = (uint32_t *)(arena + o_gt);
+        int32_t *stats = (int32_t *)(arena + o_stats);
+        PPCK(cudaMemsetAsync(stats, 0, stats_bytes, h->stream));
+        PPCK(cudaMemsetAsync(ge, 0, N * 4, h->stream));
+        PPCK(cudaMemsetAsync(gt, 0, N * 4, h->stream));
+        const dim3 grid((unsigned)((N + 255) / 256), (unsigned)C);
+        const uint32_t sim0 = (uint32_t)h->cfg.chain_offset * (uint32_t)nrep;
+        auto observe = [&](int t) {
+            k_ppc_obs<<<grid, 256, 0, h->stream>>>(b.par, h->d_obs, T, (int)N, nrep, seed, sim0, t, h->cfg.detect, b.zc, rec, stats, ge, gt);
+            CK(cudaGetLastError());
+            return MP_OK;
+        };
+        rc = is64(h) ? replicate_t<double>(h, b, 0, T - 1, nrep, seed, era.data(), observe)
+                     : replicate_t<float>(h, b, 0, T - 1, nrep, seed, era.data(), observe);
+        if (rc != MP_OK) goto done;
+        if (stats_out) PPCK(cudaMemcpyAsync(stats_out, stats, stats_bytes, cudaMemcpyDeviceToHost, h->stream));
+        if (patch_ge) PPCK(cudaMemcpyAsync(patch_ge, ge, N * 4, cudaMemcpyDeviceToHost, h->stream));
+        if (patch_gt) PPCK(cudaMemcpyAsync(patch_gt, gt, N * 4, cudaMemcpyDeviceToHost, h->stream));
+        PPCK(cudaStreamSynchronize(h->stream));
+    }
+#undef PPCK
 done:
     cudaStreamSynchronize(h->stream);
     cudaFree(arena);

@@ -12,6 +12,7 @@
 //  k_propose_* / k_decide_* / k_update_ep / k_record   Metropolis bookkeeping, one warp per chain
 //  k_sim_init / k_sim_ext / k_sim_col   forward simulator (future.c:64-110)
 //  k_fc_init / k_fc_ext / k_fc_col      posterior-predictive forecast from the chains (with k_pack_sources + k_conn)
+//  k_ppc_obs       observations and statistics of posterior-predictive replicates of the data (mp_ppc, with the forecast's year)
 #pragma once
 #include "mp_device.cuh"
 #include "mp_conn.cuh"   // k_pack_sources, k_group_min_S, k_conn
@@ -828,14 +829,15 @@ k_sim_col(Landscape<R> ls, const mp_params *__restrict__ pars, int per_sim, cons
     if ((tid & 31) == 0 && occ_out && c2) atomicAdd(&occ_out[(size_t)si * (nyears + 1) + t + 1], c2);
 }
 
-// ------------------------------------------------------------------ posterior-predictive forecast (mp_forecast)
-// nrep trajectories per chain from the chain's own z[c][T-1] and parameters, states laid out [chain][replicate][patch].
+// ------------------------------------------------------------------ posterior-predictive forecast (mp_forecast) and replicates (mp_ppc)
+// nrep trajectories per chain from the chain's own z[c][t0] and parameters, states laid out [chain][replicate][patch]
+// (t0 = T-1 for the forecast, 0 for the replicates of the data).
 // Trajectory (c, r) is simulation number sim0 + c * nrep + r of mp_simulate_ensemble: the same Philox draws per patch number.
 // One year = k_fc_ext, then S of every (chain, replicate) from k_conn with the replicates in place of the years (k_pack_sources
 // packs 32 replicates per record word), then k_fc_col.
 //   k_fc_init  grid (patch tiles, chains): start states, year-0 counts and incidence
 static __global__ void __launch_bounds__(256)
-k_fc_init(const uint8_t *__restrict__ z, int T, int n, int nrep, int nyears, uint8_t *__restrict__ zc, int32_t *__restrict__ occ,
+k_fc_init(const uint8_t *__restrict__ z, int T, int t0, int n, int nrep, int nyears, uint8_t *__restrict__ zc, int32_t *__restrict__ occ,
           uint32_t *__restrict__ inc)
 {
     __shared__ int s_cnt;
@@ -844,7 +846,7 @@ k_fc_init(const uint8_t *__restrict__ z, int T, int n, int nrep, int nyears, uin
     __syncthreads();
     int v = 0;
     if (k < n) {
-        v = z[((size_t)c * T + T - 1) * n + k] != 0;
+        v = z[((size_t)c * T + t0) * n + k] != 0;
         for (int r = 0; r < nrep; r++) zc[((size_t)c * nrep + r) * n + k] = (uint8_t)v;
         if (inc && v) atomicAdd(&inc[k], (uint32_t)nrep);
     }
@@ -911,6 +913,71 @@ k_fc_col(Landscape<R> ls, const mp_params *__restrict__ pars, int nrep, uint64_t
         __syncthreads();
     }
     if (inc && mine) atomicAdd(&inc[(size_t)(t + 1) * n + k], mine);
+}
+
+//   k_ppc_obs  grid (patch tiles, chains): the observation of year t of every replicate, after k_fc_init (t = 0) and after
+//              each k_fc_col (t + 1).  One thread per (chain, patch) runs all replicates of the patch.  A cell missing in obs
+//              stays missing; otherwise rep = z, with detection z && u < p, u keyed by (sim, year, RK_PPC_DET, patch number).
+//              The record word of a (chain, replicate, patch) holds the replicate's previous observation (bit 0) and its
+//              number of years observed occupied D (bits 1-31).  detected / colonised / extinct of every (trajectory, year):
+//              one shared-memory atomic per warp, one global atomic per CTA, replicate and statistic.  In the last year each
+//              thread adds to patch_ge / patch_gt its replicates with D >= / > the observed D of the patch.
+static __global__ void __launch_bounds__(256)
+k_ppc_obs(const mp_params *__restrict__ pars, const int8_t *__restrict__ obs, int T, int n, int nrep, uint64_t seed, uint32_t sim0,
+          int t, int detect, const uint8_t *__restrict__ zc, uint32_t *__restrict__ rec, int32_t *__restrict__ stats,
+          uint32_t *__restrict__ patch_ge, uint32_t *__restrict__ patch_gt)
+{
+    __shared__ int s_cnt[32 * MP_NPPC];
+    const int c = blockIdx.y, tid = threadIdx.x, k = blockIdx.x * 256 + tid;
+    const bool live = k < n, last = t == T - 1;
+    const int o = live ? obs[(size_t)t * n + k] : -1;
+    const bool both = o >= 0 && t > 0 && obs[(size_t)(t - 1) * n + k] >= 0;   // observed in t-1 and t: a transition to count
+    const double p = pars[c].p;
+    uint32_t dobs = 0, ge = 0, gt = 0;
+    if (last && live)
+        for (int s = 0; s < T; s++) dobs += obs[(size_t)s * n + k] == 1;
+    for (int r0 = 0; r0 < nrep; r0 += 32) {
+        const int nr = min(32, nrep - r0);
+        if (tid < 32 * MP_NPPC) s_cnt[tid] = 0;
+        __syncthreads();
+        for (int j = 0; j < nr; j++) {
+            const int r = r0 + j;
+            int det = 0, col = 0, ext = 0;
+            if (live) {
+                const size_t i = ((size_t)c * nrep + r) * n + k;
+                uint32_t w = t > 0 ? rec[i] : 0u;
+                if (o >= 0) {
+                    int v = zc[i];
+                    if (v && detect) {
+                        const uint4 u = rng(seed, sim0 + (uint32_t)c * (uint32_t)nrep + (uint32_t)r, (uint32_t)t, RK_PPC_DET, (uint32_t)k, 0);
+                        v = u01(u.x) < p;
+                    }
+                    const int prev = (int)(w & 1u);
+                    det = v; col = both && !prev && v; ext = both && prev && !v;
+                    w = (((w >> 1) + (uint32_t)v) << 1) | (uint32_t)v;
+                }
+                if (last) { ge += (w >> 1) >= dobs; gt += (w >> 1) > dobs; }
+                else rec[i] = w;
+            }
+            const int a = __reduce_add_sync(0xffffffffu, det), b = __reduce_add_sync(0xffffffffu, col),
+                      e = __reduce_add_sync(0xffffffffu, ext);
+            if ((tid & 31) == 0) {
+                if (a) atomicAdd(&s_cnt[j * MP_NPPC + 0], a);
+                if (b) atomicAdd(&s_cnt[j * MP_NPPC + 1], b);
+                if (e) atomicAdd(&s_cnt[j * MP_NPPC + 2], e);
+            }
+        }
+        __syncthreads();
+        if (tid < nr * MP_NPPC && s_cnt[tid]) {
+            const int j = tid / MP_NPPC, s = tid - j * MP_NPPC;
+            atomicAdd(&stats[(((size_t)c * nrep + r0 + j) * T + t) * MP_NPPC + s], s_cnt[tid]);
+        }
+        __syncthreads();
+    }
+    if (last && live) {
+        if (ge) atomicAdd(&patch_ge[k], ge);
+        if (gt) atomicAdd(&patch_gt[k], gt);
+    }
 }
 
 // ------------------------------------------------------------------ peak probes (roofline denominators)

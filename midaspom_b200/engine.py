@@ -17,6 +17,7 @@ from . import build as _build
 FP32, FP64 = 0, 1
 GEOM_LINEAR, GEOM_COORDS, GEOM_DENSE = 0, 1, 2
 NDRAW, NLSIG, NPART = 11, 8, 4
+PPC_STATS = ("detected", "colonised", "extinct")   # the MP_NPPC statistics of mp_ppc, in order
 KERNEL_CATEGORIES = ("conn", "col", "sweep_y", "sweep_z", "small", "sim")
 WORK_COUNTERS = ("scan_trips", "scan_exec", "scan_retired", "scan_commit", "scan_dense", "conn_exec", "conn_total", "gemm_tiles", "scan_blocks")
 DRAW_FIELDS = ("e", "c", "alpha", "b", "p", "loglik", "n_y1", "n_z1", "K", "Ksrc", "dsrc")
@@ -33,7 +34,7 @@ ABI_SYMBOLS = (
     "mp_get_scan_order", "mp_get_work_counters", "mp_get_scan_geometry", "mp_get_conn_path", "mp_set_scan_blocks",
     "mp_comm_unique_id", "mp_comm_init", "mp_comm_init_all", "mp_comm_destroy", "mp_comm_rank", "mp_comm_size", "mp_comm_last_error",
     "mp_gather_draws", "mp_gather_draws_all", "mp_sweep_sharded", "mp_sweep_sharded_all", "mp_forecast",
-    "mp_set_summaries", "mp_get_summaries", "mp_set_waic", "mp_get_waic",
+    "mp_set_summaries", "mp_get_summaries", "mp_set_waic", "mp_get_waic", "mp_ppc",
 )
 
 
@@ -130,6 +131,8 @@ def load_library(build_if_missing: bool = True) -> C.CDLL:
     L.mp_simulate.argtypes = [vp, pp, u8p, C.c_int, C.c_int, C.c_uint64, C.c_int, u8p, C.POINTER(C.c_int32)]
     L.mp_simulate_ensemble.argtypes = [vp, pp, u8p, C.c_int, C.c_int, C.c_uint64, C.c_int, u8p, C.POINTER(C.c_int32)]
     L.mp_forecast.argtypes = [vp, C.c_int, C.c_int, C.c_uint64, dp, C.POINTER(C.c_int32), C.POINTER(C.c_uint32)]
+    L.mp_ppc.argtypes = [vp, C.c_int, C.c_uint64, C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.POINTER(C.c_uint32),
+                         C.POINTER(C.c_uint32)]
     L.mp_set_summaries.argtypes = [vp, C.c_int, C.c_int]
     L.mp_get_summaries.argtypes = [vp, C.POINTER(C.c_int64), C.POINTER(C.c_uint32), dp, C.POINTER(C.c_uint32), dp, C.c_int]
     L.mp_set_waic.argtypes = [vp, C.c_int, C.c_int]
@@ -475,6 +478,19 @@ class Engine:
         self._ck(self.lib.mp_forecast(self.h, int(nyears), int(nrep), int(seed), _p(scen, _dp), _p(occ, C.POINTER(C.c_int32)),
                                       _p(inc, C.POINTER(C.c_uint32))), "mp_forecast")
         return occ, inc
+
+    def ppc(self, nrep, seed=1):
+        """Posterior-predictive replicates of the observation table (mp_ppc): nrep per chain from the chain's imputed year 0,
+        parameters and era flags, observed through the table's mask (and detection).  Returns dict(stats [C, nrep, T, 3] int32,
+        obs_stats [T, 3] int32, patch_ge, patch_gt [N] uint32, nrep_total = C * nrep); statistics in PPC_STATS order.  Pool
+        calls and chain shards with midaspom_b200.ppc_check."""
+        stats = np.zeros((self.C, nrep, self.T, len(PPC_STATS)), dtype=np.int32)
+        obs_stats = np.zeros((self.T, len(PPC_STATS)), dtype=np.int32)
+        ge, gt = np.zeros(self.N, dtype=np.uint32), np.zeros(self.N, dtype=np.uint32)
+        i32p, u32p = C.POINTER(C.c_int32), C.POINTER(C.c_uint32)
+        self._ck(self.lib.mp_ppc(self.h, int(nrep), int(seed), _p(stats, i32p), _p(obs_stats, i32p), _p(ge, u32p), _p(gt, u32p)),
+                 "mp_ppc")
+        return dict(stats=stats, obs_stats=obs_stats, patch_ge=ge, patch_gt=gt, nrep_total=self.C * int(nrep))
 
     # -- posterior summaries of the latent state
     def set_summaries(self, first_sweep=0, thin=1):
