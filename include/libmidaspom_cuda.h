@@ -26,6 +26,7 @@
  *   mp_set_summaries / mp_get_summaries   (no counterpart) posterior occupancy, survival and connectivity of every patch-year
  *   mp_set_waic / mp_get_waic  Rscript/hypothesis_test.R at large N: pointwise predictive densities for WAIC
  *   mp_ppc                    (no counterpart) posterior-predictive replicates of the observation table from the chains
+ *   mp_capacity               (no counterpart) metapopulation capacity and patch values of the landscape per parameter set
  *
  * All device memory is owned by the engine handle; host buffers are owned by the caller.  One
  * handle per GPU / host thread (thread-compatible, not thread-safe).  There is no CPU fallback:
@@ -288,6 +289,31 @@ int mp_forecast(mp_engine *h, int nyears, int nrep, uint64_t seed, const double 
 #define MP_NPPC 3   /* detected, colonised, extinct */
 int mp_ppc(mp_engine *h, int nrep, uint64_t seed, int32_t *stats_out, int32_t *obs_stats_out, uint32_t *patch_ge,
            uint32_t *patch_gt);
+/* Metapopulation capacity of the landscape (Hanski & Ovaskainen 2000) and patch values (Ovaskainen & Hanski 2001), one eigenproblem
+ * per parameter set (no reference counterpart; DESIGN.md §2 defines the quantities).  lambda_M is the largest eigenvalue of the
+ * symmetric M~_kl = sqrt(a_k a_l) exp(-alpha d_kl) (k != l), M~_kk = 0, a = A^b; only alpha and b of a set are read.  LOBPCG with
+ * block size 1 from the all-ones vector over the kept patches, stopped when ||M~x - theta x|| / theta <= rtol.
+ *   par        nsets parameter sets; NULL: the chains' resident parameters (nsets = n_chains), after any queued sweeps
+ *   keep       (nullable) N flags in patch order: 0 removes the patch as source and target (the principal submatrix)
+ *   out3       nsets*3: lambda (Rayleigh quotient of the returned vector: a lower bound of lambda_M), relative residual
+ *              ||M~x - lambda x|| / lambda, relative bound of the culled weights (||E||_2 / lambda; 0 when nothing is culled)
+ *   iters_out  (nullable) nsets iterations; a set that has not converged after max_iter reports max_iter and a residual above rtol
+ *              (not an error)
+ *   value_out  (nullable) nsets*N patch values V_k = x_k^2 / ||x||^2 in patch order (sum 1; 0 on removed patches); removing patch k
+ *              changes lambda_M by about -2 lambda V_k
+ *   value_sum  (nullable) N: the values summed over the sets
+ * Synchronous, on the engine stream after any queued sweeps.  Leaves everything as it was: chain state, S and its validity flags,
+ * draws, sweep counter, scales, captured graphs, summaries and WAIC sums.  Kernels are counted under MP_K_SIM, the (32 target x 32
+ * source) tiles of the products in MP_CNT_CONN_EXEC / MP_CNT_CONN_TOTAL; mp_set_shard does not apply.  FP32 engines on landscapes
+ * with positions skip tiles whose largest weight is below 2^-30 theta0 / N (theta0: the Rayleigh quotient of the start vector under
+ * an unculled product), MP_CONN_CULL=0 disables; the FP64 engine never culls.  A set's results depend only on its (alpha, b), the
+ * landscape, keep, rtol and max_iter, bit for bit: not on nsets, the other sets, the batching or chain_offset.
+ * Device memory: one arena per call of about min(nsets, ~1 GB worth) x N x (48 + 4 | 8) bytes; more sets run in batches.
+ * MP_ERR_ARG: nsets < 1, rtol <= 0, max_iter < 1, alpha <= 0, fewer than 2 kept patches, par = NULL with nsets != n_chains.
+ * MP_ERR_STATE: no landscape, par = NULL before any chain parameters are set.
+ * MP_ERR_UNSUPPORTED: a dense landscape whose distance matrix is not symmetric. */
+int mp_capacity(mp_engine *h, int nsets, const mp_params *par, const uint8_t *keep, double rtol, int max_iter, double *out3,
+                int32_t *iters_out, double *value_out, double *value_sum);
 
 /* ---- exact small-n engine: the reference's own algorithm (state enumeration on an (e,c) grid) ----
  * Replaces the whole hot loop of MIDASPOM.out, main_MIDASPOM.c:198-290 (state tables) and :341-395

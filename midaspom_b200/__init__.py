@@ -8,7 +8,8 @@ from .engine import (Engine, MpConfig, MpParams, MpSamplerConfig, MpError, load_
                      GEOM_DENSE, FP32, FP64, NDRAW, NLSIG, NPART, KERNEL_CATEGORIES, ABI_SYMBOLS, PPC_STATS, exact_posterior, exact_variant)
 from .waic import waic, compare_waic
 from .ppc import ppc_check
+from .capacity import persistence
 
 __all__ = ["Engine", "MpConfig", "MpParams", "MpSamplerConfig", "MpError", "load_library", "GEOM_LINEAR",
            "GEOM_COORDS", "GEOM_DENSE", "FP32", "FP64", "NDRAW", "NLSIG", "NPART", "KERNEL_CATEGORIES", "ABI_SYMBOLS", "exact_posterior", "exact_variant",
-           "waic", "compare_waic", "PPC_STATS", "ppc_check"]
+           "waic", "compare_waic", "PPC_STATS", "ppc_check", "persistence"]

@@ -5,6 +5,7 @@
 #include "mp_kernels.cuh"
 #include "mp_sweep_cull.cuh"   // k_build_candidates, CandRec, BlockTask, k_block_valid
 #include "mp_comm.h"
+#include "mp_capacity.cuh"
 
 using namespace mp;
 
@@ -925,7 +926,7 @@ int mp_set_params(mp_engine *h, const mp_params *par)
     for (size_t c = 0; c < nC(h); c++) REQUIRE(par[c].K > 0.0 && par[c].alpha > 0.0, MP_ERR_ARG, "need K > 0 and alpha > 0");
     h->any_src = false; h->S_valid = false;
     for (size_t c = 0; c < nC(h); c++) if (par[c].Ksrc != 0.0) h->any_src = true;
-    h->par_host.assign(par, par + nC(h)); h->par_host_valid = true;
+    h->par_host.assign(par, par + nC(h)); h->par_host_valid = true; h->have_params = true;
     CK(cudaMemcpyAsync(h->d_par, par, nC(h) * sizeof(mp_params), cudaMemcpyHostToDevice, h->stream));
     CK(cudaStreamSynchronize(h->stream));
     return MP_OK;
@@ -1707,6 +1708,308 @@ int mp_ppc(mp_engine *h, int nrep, uint64_t seed, int32_t *stats_out, int32_t *o
         PPCK(cudaStreamSynchronize(h->stream));
     }
 #undef PPCK
+done:
+    cudaStreamSynchronize(h->stream);
+    cudaFree(arena);
+    return rc;
+}
+
+}  // extern "C"
+
+// ---- metapopulation capacity (DESIGN.md §2): LOBPCG with block size 1 (Knyazev 2001) on M~ = D^1/2 K D^1/2, per parameter set
+
+// Rayleigh-Ritz step of one set on the basis (x, r, p), p only when has_p.  g: the CAP_NGRAM inner products of k_cap_gram.  The
+// basis is scaled to unit norms; while the Cholesky factor of its Gram matrix has a squared pivot below CAP_GRAM_TOL, p and then r
+// leave the basis (Hetmaniuk & Lehoucq 2006: restart without the search direction).  Returns the coefficients of the Ritz vector of
+// the largest Ritz value mu (unit norm, x coefficient >= 0) and the size of the basis that was used.
+constexpr double CAP_GRAM_TOL = 1e-10;
+static int cap_ritz(const double *g, bool has_p, double c[3], double &mu)
+{
+    const double A[3][3] = { { g[0], g[1], g[2] }, { g[1], g[3], g[4] }, { g[2], g[4], g[5] } };
+    const double B[3][3] = { { g[6], g[7], g[8] }, { g[7], g[9], g[10] }, { g[8], g[10], g[11] } };
+    int m = has_p ? 3 : 2;
+    double d[3] = { 0, 0, 0 }, L[3][3];
+    for (int i = 0; i < m; i++) {
+        if (!(B[i][i] > 0.0) || !std::isfinite(B[i][i])) { m = i; break; }
+        d[i] = 1.0 / std::sqrt(B[i][i]);
+    }
+    for (;; m--) {                                        // m >= 1: x itself always has a positive norm
+        bool ok = true;
+        for (int i = 0; i < m && ok; i++)
+            for (int j = 0; j <= i; j++) {
+                double s = B[i][j] * d[i] * d[j];
+                for (int q = 0; q < j; q++) s -= L[i][q] * L[j][q];
+                if (i == j) { if (!(s > CAP_GRAM_TOL)) { ok = false; break; } L[i][i] = std::sqrt(s); }
+                else L[i][j] = s / L[j][j];
+            }
+        if (ok || m == 1) break;
+    }
+    if (m == 1) { c[0] = d[0]; c[1] = c[2] = 0.0; mu = A[0][0] * d[0] * d[0]; return 1; }
+    // C = L^-1 An L^-T (An: A scaled like B), then its eigenpairs by cyclic Jacobi rotations
+    double Y[3][3], Cm[3][3], V[3][3];
+    for (int col = 0; col < m; col++)
+        for (int i = 0; i < m; i++) {
+            double s = A[i][col] * d[i] * d[col];
+            for (int q = 0; q < i; q++) s -= L[i][q] * Y[q][col];
+            Y[i][col] = s / L[i][i];
+        }
+    for (int col = 0; col < m; col++)
+        for (int i = 0; i < m; i++) {
+            double s = Y[col][i];
+            for (int q = 0; q < i; q++) s -= L[i][q] * Cm[q][col];
+            Cm[i][col] = s / L[i][i];
+        }
+    for (int i = 0; i < m; i++)
+        for (int j = 0; j < m; j++) { V[i][j] = i == j; if (j > i) Cm[i][j] = Cm[j][i] = 0.5 * (Cm[i][j] + Cm[j][i]); }
+    for (int sweep = 0; sweep < 64; sweep++) {
+        double off = 0.0, diag = 0.0;
+        for (int i = 0; i < m; i++) { diag += Cm[i][i] * Cm[i][i]; for (int j = i + 1; j < m; j++) off += Cm[i][j] * Cm[i][j]; }
+        if (off <= 1e-36 * diag) break;
+        for (int p = 0; p < m; p++)
+            for (int q = p + 1; q < m; q++) {
+                if (Cm[p][q] == 0.0) continue;
+                const double th = (Cm[q][q] - Cm[p][p]) / (2.0 * Cm[p][q]);
+                const double t = (th >= 0 ? 1.0 : -1.0) / (std::fabs(th) + std::sqrt(th * th + 1.0));
+                const double cs = 1.0 / std::sqrt(t * t + 1.0), sn = t * cs;
+                for (int k = 0; k < m; k++) {                 // Cm <- J^T Cm J, V <- V J
+                    const double a = Cm[k][p], b = Cm[k][q];
+                    Cm[k][p] = cs * a - sn * b; Cm[k][q] = sn * a + cs * b;
+                }
+                for (int k = 0; k < m; k++) {
+                    const double a = Cm[p][k], b = Cm[q][k];
+                    Cm[p][k] = cs * a - sn * b; Cm[q][k] = sn * a + cs * b;
+                }
+                for (int k = 0; k < m; k++) {
+                    const double a = V[k][p], b = V[k][q];
+                    V[k][p] = cs * a - sn * b; V[k][q] = sn * a + cs * b;
+                }
+            }
+    }
+    int top = 0;
+    for (int i = 1; i < m; i++) if (Cm[i][i] > Cm[top][top]) top = i;
+    mu = Cm[top][top];
+    double y[3] = { 0, 0, 0 };
+    for (int i = m - 1; i >= 0; i--) {                    // L^T y = V[:, top]
+        double s = V[i][top];
+        for (int q = i + 1; q < m; q++) s -= L[q][i] * y[q];
+        y[i] = s / L[i][i];
+    }
+    const double sg = y[0] < 0.0 ? -1.0 : 1.0;
+    for (int i = 0; i < 3; i++) c[i] = i < m ? sg * y[i] * d[i] : 0.0;
+    return m;
+}
+
+struct CapOut { double *out3; int32_t *iters; double *value, *value_sum; };
+// sets [s0, s0 + nb) of one batch in the call's arena; every output row of the batch is written
+template <typename R>
+static int capacity_batch(mp_engine *h, unsigned char *arena, const size_t *o, int nbmax, const mp_params *par, int s0, int nb,
+                          double rtol, int max_iter, bool cull, const std::vector<int> &perm, const CapOut &out)
+{
+    const int n = h->cfg.n_patches, npad = cap_npad(n), nchunk = (n + CAP_CHUNK - 1) / CAP_CHUNK;
+    CapSet *d_cs = (CapSet *)(arena + o[4]);
+    double *vec = (double *)(arena + o[3]), *part = (double *)(arena + o[7]);
+    unsigned *bound = (unsigned *)(arena + o[6]);
+    CapArgs<R> a;
+    a.ls = view<R>(h); a.cs = d_cs; a.lx = (const R *)(arena + o[0]); a.ly = (const R *)(arena + o[1]); a.hs = (const R *)(arena + o[2]);
+    a.vec = vec; a.box32 = (const float4 *)h->d_tile_box; a.bound = bound; a.stats = h->d_work; a.npad = npad;
+    // the arena of the previous batch: vectors and bounds start from zero (p, Ap, padding), then the batch's constants
+    CK(cudaMemsetAsync(vec, 0, (size_t)nbmax * CAP_NVEC * npad * 8, h->stream));
+    CK(cudaMemsetAsync(bound, 0, (size_t)nbmax * 4, h->stream));
+    std::vector<double> b(nb);
+    std::vector<CapSet> cs(nb);
+    for (int i = 0; i < nb; i++) {
+        const mp_params &p = par[s0 + i];
+        b[i] = p.b;
+        cs[i] = CapSet{ p.alpha, 1.0, 0.0, 0.0, 0.0, -INFINITY, (float)(std::max(p.b * std::log2(h->area_max), p.b * std::log2(h->area_min)) + 1e-3), i, 0 };
+    }
+    CK(cudaMemcpyAsync(arena + o[5], b.data(), nb * 8, cudaMemcpyHostToDevice, h->stream));
+    k_cap_prep<R><<<dim3((npad + 255) / 256, nb), 256, 0, h->stream>>>(a.ls, h->d_perm, h->have_area ? h->d_area : nullptr,
+                                                                        (const uint8_t *)(arena + o[8]), (const double *)(arena + o[5]),
+                                                                        npad, (R *)(arena + o[0]), (R *)(arena + o[1]), (R *)(arena + o[2]), vec);
+    CK(cudaGetLastError());
+    std::vector<CapSet> up;                               // the active sets of a launch, in batch order
+    std::vector<double> hp;
+    auto launch_mv = [&](bool culled, int vin, int vout) -> int {
+        const dim3 grid(npad / CAP_NT, (unsigned)up.size());
+        constexpr bool CAN = sizeof(R) == 4;              // the FP64 engine never culls
+        const bool cl = CAN && culled;
+#define MV(G) do { if (cl) k_cap_mv<R, G, CAN><<<grid, CAP_NT, 0, h->stream>>>(a, vin, vout); \
+                    else k_cap_mv<R, G, false><<<grid, CAP_NT, 0, h->stream>>>(a, vin, vout); } while (0)
+        switch (h->geom) {
+        case MP_GEOM_LINEAR: MV(MP_GEOM_LINEAR); break;
+        case MP_GEOM_COORDS: MV(MP_GEOM_COORDS); break;
+        default: k_cap_mv<R, MP_GEOM_DENSE, false><<<grid, CAP_NT, 0, h->stream>>>(a, vin, vout); break;
+        }
+#undef MV
+        CK(cudaGetLastError());
+        return MP_OK;
+    };
+    auto upload = [&]() -> int {
+        CK(cudaMemcpyAsync(d_cs, up.data(), up.size() * sizeof(CapSet), cudaMemcpyHostToDevice, h->stream));
+        return MP_OK;
+    };
+    // k_cap_update (gram = false) or k_cap_gram over the sets in `up`; hp[i * K + j]: sum j of up[i], chunks added in order
+    auto reduce = [&](bool gram) -> int {
+        const int K = gram ? CAP_NGRAM : 3;
+        const dim3 grid(nchunk, (unsigned)up.size());
+        if (gram) k_cap_gram<<<grid, CAP_RT, 0, h->stream>>>(d_cs, vec, n, npad, part);
+        else k_cap_update<<<grid, CAP_RT, 0, h->stream>>>(d_cs, vec, n, npad, part);
+        CK(cudaGetLastError());
+        std::vector<double> raw(up.size() * nchunk * K);
+        CK(cudaMemcpyAsync(raw.data(), part, raw.size() * 8, cudaMemcpyDeviceToHost, h->stream));
+        CK(cudaStreamSynchronize(h->stream));
+        hp.assign(up.size() * K, 0.0);
+        for (size_t i = 0; i < up.size(); i++)
+            for (int ch = 0; ch < nchunk; ch++)
+                for (int j = 0; j < K; j++) hp[i * K + j] += raw[(i * nchunk + ch) * K + j];
+        return MP_OK;
+    };
+    int rc;
+    // start: x = 1 on the kept patches, Ax by an unculled product; theta0 = its Rayleigh quotient sets the culling floor
+    // tau = 2^-30 theta0 / N (DESIGN.md §5), then Ax again under the floor and r = Ax - theta0 x
+    std::vector<double> theta(nb), res(nb);
+    std::vector<int> iters(nb, 0);
+    std::vector<char> has_p(nb, 0);
+    up = cs;
+    if ((rc = upload()) != MP_OK || (rc = launch_mv(false, CAP_X, CAP_AX)) != MP_OK || (rc = reduce(false)) != MP_OK) return rc;
+    for (int i = 0; i < nb; i++) {
+        theta[i] = hp[i * 3 + 1] / hp[i * 3];
+        cs[i].mu = theta[i];
+        if (cull && theta[i] > 0.0) cs[i].thr = (float)(CONN_CULL_LOG2 + std::log2(theta[i] / n)) - cs[i].lamax;
+    }
+    up = cs;
+    if ((rc = upload()) != MP_OK) return rc;
+    if (cull && (rc = launch_mv(true, CAP_X, CAP_AX)) != MP_OK) return rc;
+    if ((rc = reduce(false)) != MP_OK) return rc;
+    std::vector<int> act;
+    for (int i = 0; i < nb; i++) {
+        res[i] = std::sqrt(hp[i * 3 + 2] / hp[i * 3]) / theta[i];
+        if (!(res[i] <= rtol)) act.push_back(i);
+    }
+    for (int it = 1; it <= max_iter && !act.empty(); it++) {
+        up.clear();
+        for (int i : act) up.push_back(cs[i]);
+        if ((rc = upload()) != MP_OK || (rc = launch_mv(cull, CAP_R, CAP_AR)) != MP_OK || (rc = reduce(true)) != MP_OK) return rc;
+        for (size_t j = 0; j < act.size(); j++) {
+            CapSet &c = cs[act[j]];
+            double co[3], mu;
+            const int m = cap_ritz(&hp[j * CAP_NGRAM], has_p[act[j]] != 0, co, mu);
+            c.cx = co[0]; c.cr = co[1]; c.cp = co[2]; c.mu = mu;
+            has_p[act[j]] = m >= 2;
+            up[j] = c;
+        }
+        if ((rc = upload()) != MP_OK || (rc = reduce(false)) != MP_OK) return rc;
+        std::vector<int> next;
+        for (size_t j = 0; j < act.size(); j++) {
+            const int i = act[j];
+            const double xx = hp[j * 3], th = hp[j * 3 + 1] / xx;
+            iters[i] = it;
+            res[i] = std::sqrt(hp[j * 3 + 2] / xx) / th;
+            if (!(res[i] <= rtol)) next.push_back(i);
+        }
+        act.swap(next);
+    }
+    // report: a fresh product of every returned x, its Rayleigh quotient and residual
+    for (int i = 0; i < nb; i++) { cs[i].cx = 1.0; cs[i].cr = cs[i].cp = 0.0; cs[i].mu = 0.0; }
+    up = cs;
+    if ((rc = upload()) != MP_OK || (rc = launch_mv(cull, CAP_X, CAP_AX)) != MP_OK || (rc = reduce(false)) != MP_OK) return rc;
+    std::vector<double> xx(nb);
+    for (int i = 0; i < nb; i++) { xx[i] = hp[i * 3]; theta[i] = hp[i * 3 + 1] / xx[i]; cs[i].mu = theta[i]; }
+    up = cs;
+    if ((rc = upload()) != MP_OK || (rc = reduce(false)) != MP_OK) return rc;
+    std::vector<unsigned> bits(nb);
+    CK(cudaMemcpyAsync(bits.data(), bound, nb * 4, cudaMemcpyDeviceToHost, h->stream));
+    std::vector<double> x;
+    if (out.value || out.value_sum) {
+        x.resize((size_t)nb * npad);
+        for (int i = 0; i < nb; i++)
+            CK(cudaMemcpyAsync(&x[(size_t)i * npad], vec + ((size_t)i * CAP_NVEC + CAP_X) * npad, (size_t)npad * 8, cudaMemcpyDeviceToHost, h->stream));
+    }
+    CK(cudaStreamSynchronize(h->stream));
+    for (int i = 0; i < nb; i++) {
+        float bf;
+        std::memcpy(&bf, &bits[i], 4);
+        double *o3 = out.out3 + (size_t)(s0 + i) * 3;
+        o3[0] = theta[i];
+        o3[1] = std::sqrt(hp[i * 3 + 2] / xx[i]) / theta[i];
+        o3[2] = (double)bf / theta[i];
+        if (out.iters) out.iters[s0 + i] = iters[i];
+        for (int s = 0; s < n && !x.empty(); s++) {
+            const double v = x[(size_t)i * npad + s] * x[(size_t)i * npad + s] / xx[i];
+            if (out.value) out.value[(size_t)(s0 + i) * n + perm[s]] = v;
+            if (out.value_sum) out.value_sum[perm[s]] += v;
+        }
+    }
+    return MP_OK;
+}
+
+extern "C" {
+int mp_capacity(mp_engine *h, int nsets, const mp_params *par, const uint8_t *keep, double rtol, int max_iter, double *out3,
+                int32_t *iters_out, double *value_out, double *value_sum)
+{
+    if (!h) return MP_ERR_ARG;
+    CK(cudaSetDevice(h->cfg.device));
+    REQUIRE(out3, MP_ERR_ARG, "mp_capacity: out3 is required");
+    REQUIRE(nsets >= 1 && rtol > 0.0 && max_iter >= 1, MP_ERR_ARG, "mp_capacity: need nsets >= 1, rtol > 0 and max_iter >= 1");
+    REQUIRE(h->have_landscape, MP_ERR_STATE, "mp_capacity: landscape not set");
+    REQUIRE(par || h->have_params, MP_ERR_STATE, "mp_capacity: par = NULL reads the chains' parameters, and none are set");
+    REQUIRE(par || nsets == h->cfg.n_chains, MP_ERR_ARG, "mp_capacity: par = NULL needs nsets = n_chains");
+    const int n = h->cfg.n_patches;
+    std::vector<mp_params> pv;
+    if (!par) {
+        pv.resize(nC(h));
+        CK(cudaMemcpyAsync(pv.data(), h->d_par, nC(h) * sizeof(mp_params), cudaMemcpyDeviceToHost, h->stream));
+        CK(cudaStreamSynchronize(h->stream));
+        par = pv.data();
+    }
+    for (int s = 0; s < nsets; s++) REQUIRE(par[s].alpha > 0.0, MP_ERR_ARG, "mp_capacity: every set needs alpha > 0");
+    int nkeep = n;
+    if (keep) { nkeep = 0; for (int k = 0; k < n; k++) nkeep += keep[k] != 0; }
+    REQUIRE(nkeep >= 2, MP_ERR_ARG, "mp_capacity: need at least 2 kept patches");
+    Timed tm(h, MP_K_SIM);
+    const size_t npad = (size_t)cap_npad(n), R = rsz(h), nchunk = (n + CAP_CHUNK - 1) / CAP_CHUNK;
+    // one arena per call, reused by the batches of at most ~1 GB: positions, area constants, vectors, b, launch records, bounds,
+    // reduction partials, keep, symmetry flag
+    const size_t per_set = npad * (R + CAP_NVEC * 8) + 8 + sizeof(CapSet) + 4 + nchunk * CAP_NGRAM * 8 + 4 * 256;
+    const int nbmax = (int)std::max<size_t>(1, std::min<size_t>({ (size_t)nsets, ((size_t)1 << 30) / per_set, 65535 }));
+    size_t off = 0, o[10];
+    auto carve = [&](size_t bytes) { const size_t r = off; off += (bytes + 255) / 256 * 256; return r; };
+    o[0] = carve(npad * R); o[1] = carve(npad * R); o[2] = carve(nbmax * npad * R); o[3] = carve(nbmax * CAP_NVEC * npad * 8);
+    o[4] = carve(nbmax * sizeof(CapSet)); o[5] = carve(nbmax * 8); o[6] = carve(nbmax * 4); o[7] = carve(nbmax * nchunk * CAP_NGRAM * 8);
+    o[8] = carve(n); o[9] = carve(4);
+    unsigned char *arena = nullptr;
+    int rc = MP_OK;
+    cudaError_t e;
+#define CAPCK(call) if ((e = (call)) != cudaSuccess) { h->err = std::string(#call) + ": " + cudaGetErrorString(e); rc = MP_ERR_CUDA; goto done; }
+    CAPCK(cudaMalloc(&arena, off));
+    {
+        std::vector<uint8_t> kp(n, 1);
+        if (keep) for (int k = 0; k < n; k++) kp[k] = keep[k] != 0;
+        CAPCK(cudaMemcpyAsync(arena + o[8], kp.data(), n, cudaMemcpyHostToDevice, h->stream));
+        if (h->geom == MP_GEOM_DENSE) {                   // M~ is symmetric only for a symmetric distance matrix
+            int *flag = (int *)(arena + o[9]), hf = 0;
+            CAPCK(cudaMemsetAsync(flag, 0, 4, h->stream));
+            const dim3 grid((n + 255) / 256, std::min(n, 65535));
+            if (is64(h)) k_cap_symcheck<double><<<grid, 256, 0, h->stream>>>((const double *)h->d_dist, n, flag);
+            else k_cap_symcheck<float><<<grid, 256, 0, h->stream>>>((const float *)h->d_dist, n, flag);
+            CAPCK(cudaGetLastError());
+            CAPCK(cudaMemcpyAsync(&hf, flag, 4, cudaMemcpyDeviceToHost, h->stream));
+            CAPCK(cudaStreamSynchronize(h->stream));
+            if (hf) { h->err = "mp_capacity: the distance matrix is not symmetric"; rc = MP_ERR_UNSUPPORTED; goto done; }
+        }
+        std::vector<int> perm(n);
+        CAPCK(cudaMemcpyAsync(perm.data(), h->d_perm, n * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
+        CAPCK(cudaStreamSynchronize(h->stream));
+        if (value_sum) std::fill(value_sum, value_sum + n, 0.0);
+        const bool cull = !is64(h) && h->geom != MP_GEOM_DENSE && h->conn_cull && h->have_boxes;
+        const CapOut out{ out3, iters_out, value_out, value_sum };
+        for (int s0 = 0; s0 < nsets && rc == MP_OK; s0 += nbmax) {
+            const int nb = std::min(nbmax, nsets - s0);
+            rc = is64(h) ? capacity_batch<double>(h, arena, o, nbmax, par, s0, nb, rtol, max_iter, cull, perm, out)
+                         : capacity_batch<float>(h, arena, o, nbmax, par, s0, nb, rtol, max_iter, cull, perm, out);
+        }
+    }
+#undef CAPCK
 done:
     cudaStreamSynchronize(h->stream);
     cudaFree(arena);

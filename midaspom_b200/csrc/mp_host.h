@@ -66,6 +66,7 @@ struct mp_engine {
     double area_max = 1.0, area_min = 1.0;
     bool have_boxes = false; int conn_cull = 1;   // MP_CONN_CULL=0 disables the culling of k_conn
     void *d_gemm = nullptr; size_t gemm_bytes = 0;   // BF16 occupancy columns + source records of the tensor-core path (mp_conn_gemm.cu)
+    bool have_params = false;                  // mp_set_params (or mp_init_chains) has run
     std::vector<mp_params> par_host;           // parameters as last uploaded by mp_set_params ...
     bool par_host_valid = false;               // ... still what the device holds (the sampler changes them on the device)
     int use_gemm = 1, gemm_min_n = 1024;       // tensor-core connectivity for chains sharing (alpha, b): MP_CONN_GEMM=0 disables, MP_CONN_GEMM_MIN_N

@@ -8,6 +8,7 @@ computes on the CPU.
 from __future__ import annotations
 
 import ctypes as C
+import hashlib
 from pathlib import Path
 
 import numpy as np
@@ -34,7 +35,7 @@ ABI_SYMBOLS = (
     "mp_get_scan_order", "mp_get_work_counters", "mp_get_scan_geometry", "mp_get_conn_path", "mp_set_scan_blocks",
     "mp_comm_unique_id", "mp_comm_init", "mp_comm_init_all", "mp_comm_destroy", "mp_comm_rank", "mp_comm_size", "mp_comm_last_error",
     "mp_gather_draws", "mp_gather_draws_all", "mp_sweep_sharded", "mp_sweep_sharded_all", "mp_forecast",
-    "mp_set_summaries", "mp_get_summaries", "mp_set_waic", "mp_get_waic", "mp_ppc",
+    "mp_set_summaries", "mp_get_summaries", "mp_set_waic", "mp_get_waic", "mp_ppc", "mp_capacity",
 )
 
 
@@ -133,6 +134,7 @@ def load_library(build_if_missing: bool = True) -> C.CDLL:
     L.mp_forecast.argtypes = [vp, C.c_int, C.c_int, C.c_uint64, dp, C.POINTER(C.c_int32), C.POINTER(C.c_uint32)]
     L.mp_ppc.argtypes = [vp, C.c_int, C.c_uint64, C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.POINTER(C.c_uint32),
                          C.POINTER(C.c_uint32)]
+    L.mp_capacity.argtypes = [vp, C.c_int, pp, u8p, C.c_double, C.c_int, dp, C.POINTER(C.c_int32), dp, dp]
     L.mp_set_summaries.argtypes = [vp, C.c_int, C.c_int]
     L.mp_get_summaries.argtypes = [vp, C.POINTER(C.c_int64), C.POINTER(C.c_uint32), dp, C.POINTER(C.c_uint32), dp, C.c_int]
     L.mp_set_waic.argtypes = [vp, C.c_int, C.c_int]
@@ -175,6 +177,7 @@ class Engine:
             self.h = None
             raise MpError(f"mp_create failed ({rc}): {msg}")
         self.N, self.T, self.C = n_patches, n_years, n_chains
+        self._landscape_key = b""
 
     # -- lifetime
     def close(self):
@@ -208,16 +211,27 @@ class Engine:
             raise ValueError(f"expected shape {shape}, got {a.shape}")
         return a
 
+    def _remember_landscape(self, *parts):
+        """Fingerprint of the landscape as uploaded (capacity results carry it so that results of different landscapes are not
+        pooled)."""
+        h = hashlib.sha256()
+        for a in parts:
+            h.update(b"-" if a is None else np.ascontiguousarray(a, dtype=np.float64).tobytes())
+        self._landscape_key = h.digest()
+
     def set_landscape_linear(self, spacing, area=None):
         area = self._f64(area, (self.N,))
+        self._remember_landscape(np.array([0.0, float(spacing)]), area)
         self._ck(self.lib.mp_set_landscape_linear(self.h, float(spacing), _p(area, _dp)), "mp_set_landscape_linear")
 
     def set_landscape_coords(self, x, y, area=None):
         x, y, area = self._f64(x, (self.N,)), self._f64(y, (self.N,)), self._f64(area, (self.N,))
+        self._remember_landscape(np.array([1.0]), x, y, area)
         self._ck(self.lib.mp_set_landscape_coords(self.h, _p(x, _dp), _p(y, _dp), _p(area, _dp)), "mp_set_landscape_coords")
 
     def set_landscape_dense(self, dist, area=None):
         dist, area = self._f64(dist, (self.N, self.N)), self._f64(area, (self.N,))
+        self._remember_landscape(np.array([2.0]), dist, area)
         self._ck(self.lib.mp_set_landscape_dense(self.h, _p(dist, _dp), _p(area, _dp)), "mp_set_landscape_dense")
 
     def set_source_units(self, src_unit=None):
@@ -491,6 +505,38 @@ class Engine:
         self._ck(self.lib.mp_ppc(self.h, int(nrep), int(seed), _p(stats, i32p), _p(obs_stats, i32p), _p(ge, u32p), _p(gt, u32p)),
                  "mp_ppc")
         return dict(stats=stats, obs_stats=obs_stats, patch_ge=ge, patch_gt=gt, nrep_total=self.C * int(nrep))
+
+    def capacity(self, params=None, keep=None, rtol=1e-6, max_iter=1000, values=False):
+        """Metapopulation capacity lambda_M and patch values of the landscape (mp_capacity), one eigenproblem per parameter set.
+        params: None (the chains' resident parameters), a list of parameter dicts, or rows of ``get_draws`` (any array whose last
+        axis holds the NDRAW fields; the alpha and b columns are read).  keep: N flags, 0 removes a patch.  Returns dict(lam,
+        residual, cull_bound, iters [nsets], values [nsets, N] or None, value_sum [N] or None, fingerprint); pool the results of
+        several calls with the matching draws through midaspom_b200.persistence."""
+        if params is None:
+            arr, nsets = None, self.C
+        else:
+            if isinstance(params, np.ndarray):
+                rows = np.asarray(params, dtype=np.float64).reshape(-1, NDRAW)
+                params = [dict(alpha=r[DRAW_FIELDS.index("alpha")], b=r[DRAW_FIELDS.index("b")]) for r in rows]
+            elif isinstance(params, dict):
+                params = [params]
+            nsets = len(params)
+            arr = (MpParams * nsets)()
+            for i, p in enumerate(params):
+                arr[i] = self._one_param(p)
+        keep_a = None if keep is None else np.ascontiguousarray(np.asarray(keep) != 0, dtype=np.uint8)
+        if keep_a is not None and keep_a.shape != (self.N,):
+            raise ValueError(f"keep must have shape {(self.N,)}")
+        out3 = np.zeros((nsets, 3))
+        iters = np.zeros(nsets, dtype=np.int32)
+        vals = np.zeros((nsets, self.N)) if values else None
+        vsum = np.zeros(self.N) if values else None
+        self._ck(self.lib.mp_capacity(self.h, int(nsets), arr, _p(keep_a, _u8p), float(rtol), int(max_iter), _p(out3, _dp),
+                                      _p(iters, C.POINTER(C.c_int32)), _p(vals, _dp), _p(vsum, _dp)), "mp_capacity")
+        kept = np.ones(self.N, dtype=np.uint8) if keep_a is None else keep_a
+        fp = hashlib.sha256(self._landscape_key + kept.tobytes()).hexdigest()
+        return dict(lam=out3[:, 0].copy(), residual=out3[:, 1].copy(), cull_bound=out3[:, 2].copy(), iters=iters, values=vals,
+                    value_sum=vsum, fingerprint=fp)
 
     # -- posterior summaries of the latent state
     def set_summaries(self, first_sweep=0, thin=1):
