@@ -27,6 +27,7 @@
  *   mp_set_waic / mp_get_waic  Rscript/hypothesis_test.R at large N: pointwise predictive densities for WAIC
  *   mp_ppc                    (no counterpart) posterior-predictive replicates of the observation table from the chains
  *   mp_capacity               (no counterpart) metapopulation capacity and patch values of the landscape per parameter set
+ *   mp_set_sources / mp_get_sources   (no counterpart) colonisations attributed to their source patches and distances
  *
  * All device memory is owned by the engine handle; host buffers are owned by the caller.  One
  * handle per GPU / host thread (thread-compatible, not thread-safe).  There is no CPU fallback:
@@ -233,6 +234,35 @@ int mp_set_waic(mp_engine *h, int first_sweep, int thin);
  * delta = sum_i (elpd_i^A - elpd_i^B), se = sqrt(n_obs var_i(elpd_i^A - elpd_i^B)).
  * MP_ERR_STATE: WAIC sums not set. */
 int mp_get_waic(mp_engine *h, int64_t *nsamples, double *lik_sum, double *loglik_sum, double *loglik_sq, int reset);
+/* Attribution of every colonisation to its source patches (no reference counterpart), accumulated on the device at the end
+ * of every qualifying sweep, summed over this engine's chains.  first_sweep / thin as for mp_set_summaries; thin = 0 switches
+ * them off and frees them; setting them zeroes every array.  For a sample (chain after a qualifying sweep, its final z, y,
+ * resident S and parameters) and transition t = 0 .. T-2:
+ *   event        target k with y_tk = 0 and z_{t+1,k} = 1 (the cells whose likelihood term is log C_tk)
+ *   pressure     P_tk = K_t S_tk + Ksrc_t g_k (K_t, Ksrc_t, g_k as in C_tk; P = S without era flags)
+ *   shares       source l (y_tl = 1): rho_tkl = K_t w(k<-l) / P_tk;  external: rho_tk,ext = Ksrc_t g_k / P_tk; they sum to 1
+ *   unattributed an event with P_tk = 0 (an initial or impossible state): counted, not attributed
+ * rho is the share of the colonisation pressure, not an observed causal link: read it as "which source colonised k" only under
+ * independent propagule contributions.  nbins > 0 adds a histogram of rho over the source-target distance d (pair_distance's
+ * value in the landscape's unit): bins [b w, (b + 1) w), the last bin open (d >= (nbins - 1) w); nbins = 0: no histogram,
+ * bin_width ignored.  Per transition, sum_l src_sum + ext_sum = events - unattributed up to the difference between the
+ * resident S and a fresh sum of the same weights; sum_b dist_hist = sum_l src_sum up to the histogram's fixed point (each pair
+ * is rounded to 2^-40).  Three kernels per qualifying sweep (no floating-point atomics: bit-identical sums), counted under
+ * MP_K_SMALL; without sources a sweep launches exactly what it launched before.  The work is events x sources per (chain,
+ * transition), without culling.  Device memory: C (T-1) N (2 r + 8) + (T-1) N 8 + C (T-1) 24 + (T-1)(16 nbins + 24) + 8 bytes
+ * (each part rounded up to 256), r = 16 (FP32) or 32 (FP64) the record size.  mp_forecast, mp_ppc, mp_capacity, mp_connectivity,
+ * mp_loglik[_host], mp_simulate* and mp_flip_delta leave the sums unchanged.  mp_sweep_sharded[_all] ranks hold identical sums
+ * (phase 3 runs replicated there); chain-sharded engines add theirs.
+ * MP_ERR_ARG: first_sweep < 0, thin < 0, nbins < 0 or > 4096, or nbins > 0 with bin_width not finite and > 0. */
+int mp_set_sources(mp_engine *h, int first_sweep, int thin, int nbins, double bin_width);
+/* Copy (and with reset != 0 zero) the sums.  Every output is nullable.  Synchronous, after any queued sweeps.
+ *   nsamples   accumulated sweeps x n_chains
+ *   events     (T-1)*2: events[t] at t, unattributed[t] at (T-1) + t
+ *   src_sum    (T-1)*N, patch order: sum over samples and events of rho_tkl (expected colonisations patch l seeded in t -> t+1)
+ *   ext_sum    T-1: sum of rho_tk,ext
+ *   dist_hist  (T-1)*nbins: sum of rho_tkl over the pairs in each distance bin (untouched without a histogram)
+ * MP_ERR_STATE: source sums not set. */
+int mp_get_sources(mp_engine *h, int64_t *nsamples, uint64_t *events, double *src_sum, double *ext_sum, double *dist_hist, int reset);
 
 /* ---- forward simulator ---- */
 /* nsims independent trajectories of nyears from z0 (N bytes); era_all != 0 applies K/Ksrc every

@@ -9,7 +9,8 @@ from .engine import (Engine, MpConfig, MpParams, MpSamplerConfig, MpError, load_
 from .waic import waic, compare_waic
 from .ppc import ppc_check
 from .capacity import persistence
+from .sources import colonisation_sources
 
 __all__ = ["Engine", "MpConfig", "MpParams", "MpSamplerConfig", "MpError", "load_library", "GEOM_LINEAR",
            "GEOM_COORDS", "GEOM_DENSE", "FP32", "FP64", "NDRAW", "NLSIG", "NPART", "KERNEL_CATEGORIES", "ABI_SYMBOLS", "exact_posterior", "exact_variant",
-           "waic", "compare_waic", "PPC_STATS", "ppc_check", "persistence"]
+           "waic", "compare_waic", "PPC_STATS", "ppc_check", "persistence", "colonisation_sources"]

@@ -14,7 +14,7 @@ OBJ_DIR = LIB_DIR / "obj"
 LIB = LIB_DIR / "libmidaspom_cuda.so"
 SOURCES = [CSRC / "mp_engine.cu", CSRC / "mp_sweep_fast_linear.cu", CSRC / "mp_sweep_fast_coords.cu",
            CSRC / "mp_sweep_fast_dense.cu", CSRC / "mp_exact.cu", CSRC / "mp_conn_gemm.cu", CSRC / "mp_comm.cu", CSRC / "mp_conn32.cu"]
-HEADERS = [CSRC / "mp_device.cuh", CSRC / "mp_kernels.cuh", CSRC / "mp_conn.cuh", CSRC / "mp_sweep_fast.cuh", CSRC / "mp_sweep_cull.cuh", CSRC / "mp_capacity.cuh", CSRC / "mp_host.h", CSRC / "mp_comm.h",
+HEADERS = [CSRC / "mp_device.cuh", CSRC / "mp_kernels.cuh", CSRC / "mp_conn.cuh", CSRC / "mp_sweep_fast.cuh", CSRC / "mp_sweep_cull.cuh", CSRC / "mp_capacity.cuh", CSRC / "mp_sources.cuh", CSRC / "mp_host.h", CSRC / "mp_comm.h",
            PKG.parent / "include" / "libmidaspom_cuda.h"]
 
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "-Xcompiler", "-fPIC"] + os.environ.get("MP_NVCC_EXTRA", "").split()

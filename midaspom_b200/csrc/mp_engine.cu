@@ -6,6 +6,7 @@
 #include "mp_sweep_cull.cuh"   // k_build_candidates, CandRec, BlockTask, k_block_valid
 #include "mp_comm.h"
 #include "mp_capacity.cuh"
+#include "mp_sources.cuh"
 
 using namespace mp;
 
@@ -486,6 +487,58 @@ template <typename R> static int launch_waic(mp_engine *h)
     CK(cudaGetLastError());
     return MP_OK;
 }
+// ---- colonisation sources (mp_set_sources): the per-sample lists, staging array, per-(chain, transition) externals and counts
+// and integer histogram, then the sums (src_sum, ext_sum, events, dist_hist, sample counter)
+struct SrcLayout { size_t evt, src, stage, ct_ext, ct_cnt, hist_i, sums, src_sum, ext_sum, events, dist_hist, nsamples, bytes; };
+static SrcLayout src_layout(const mp_engine *h, int nbins)
+{
+    SrcLayout L;
+    size_t off = 0;
+    auto carve = [&](size_t bytes) { const size_t o = off; off += (bytes + 255) / 256 * 256; return o; };
+    const size_t rows = nC(h) * (nT(h) - 1), cells = rows * nN(h), nb = (size_t)nbins;
+    L.evt = carve(cells * (is64(h) ? sizeof(EvtRec<double>) : sizeof(EvtRec<float>)));
+    L.src = carve(cells * (is64(h) ? sizeof(SrcRec<double>) : sizeof(SrcRec<float>)));
+    L.stage = carve(cells * 8); L.ct_ext = carve(rows * 8); L.ct_cnt = carve(rows * 16); L.hist_i = carve((nT(h) - 1) * nb * 8);
+    L.sums = off;
+    L.src_sum = carve(ycells(h) * 8); L.ext_sum = carve((nT(h) - 1) * 8); L.events = carve(2 * (nT(h) - 1) * 8);
+    L.dist_hist = carve((nT(h) - 1) * nb * 8); L.nsamples = carve(8); L.bytes = off;
+    return L;
+}
+template <typename R, int GEOM> static void launch_src_contract(mp_engine *h, const SrcBufs &b)
+{
+    const int T = h->cfg.n_years;
+    const dim3 grid((h->cfg.n_patches + SRC_TILE - 1) / SRC_TILE, T - 1, h->cfg.n_chains);
+    if (b.nbins > 0)
+        k_src_contract<R, GEOM, true><<<grid, SRC_TILE, (size_t)b.nbins * 8, h->stream>>>(h->d_ctr, h->src_first, h->src_thin, view<R>(h),
+                                                                                          h->d_par, T, b);
+    else
+        k_src_contract<R, GEOM, false><<<grid, SRC_TILE, 0, h->stream>>>(h->d_ctr, h->src_first, h->src_thin, view<R>(h), h->d_par, T, b);
+}
+// three launches, each gated on the device by the sweep counter
+template <typename R> static int launch_sources(mp_engine *h)
+{
+    const SrcLayout L = src_layout(h, h->src_nbins);
+    unsigned char *base = h->d_src;
+    SrcBufs b;
+    b.evt = base + L.evt; b.src = base + L.src; b.stage = (double *)(base + L.stage); b.ct_ext = (double *)(base + L.ct_ext);
+    b.ct_cnt = (uint32_t *)(base + L.ct_cnt); b.hist_i = (unsigned long long *)(base + L.hist_i);
+    b.src_sum = (double *)(base + L.src_sum); b.ext_sum = (double *)(base + L.ext_sum); b.events = (unsigned long long *)(base + L.events);
+    b.dist_hist = (double *)(base + L.dist_hist); b.nsamples = (unsigned long long *)(base + L.nsamples);
+    b.nbins = h->src_nbins; b.bin_width = h->src_bin_width;
+    const int T = h->cfg.n_years, n = h->cfg.n_patches;
+    k_src_lists<R><<<dim3(T - 1, h->cfg.n_chains), SRC_LIST_THREADS, 0, h->stream>>>(h->d_ctr, h->src_first, h->src_thin, view<R>(h),
+        h->geom == MP_GEOM_COORDS ? 1 : 0, h->d_perm, h->d_par, h->have_era ? h->d_era : nullptr, (const R *)h->d_aw[0], h->d_z, h->d_y,
+        h->d_S[0], T, b);
+    CK(cudaGetLastError());
+    if (h->geom == MP_GEOM_COORDS) launch_src_contract<R, MP_GEOM_COORDS>(h, b);
+    else if (h->geom == MP_GEOM_DENSE) launch_src_contract<R, MP_GEOM_DENSE>(h, b);
+    else launch_src_contract<R, MP_GEOM_LINEAR>(h, b);
+    CK(cudaGetLastError());
+    const long long threads = (long long)(T - 1) * std::max(n, h->src_nbins);
+    k_src_finish<<<(unsigned)((threads + 255) / 256), 256, 0, h->stream>>>(h->d_ctr, h->src_first, h->src_thin, n, T, h->cfg.n_chains, b);
+    CK(cudaGetLastError());
+    return MP_OK;
+}
 
 // phase 3: e and p from the sufficient counts, record the draw
 template <typename R> static int phase_finish(mp_engine *h)
@@ -513,6 +566,10 @@ template <typename R> static int phase_finish(mp_engine *h)
         if (h->waic_thin > 0) {                              // the same for the WAIC sums
             h->t_launch[MP_K_SMALL]++;
             if ((rc = launch_waic<R>(h)) != MP_OK) return rc;
+        }
+        if (h->src_thin > 0) {                               // and for the colonisation sources (three launches)
+            h->t_launch[MP_K_SMALL] += 3;
+            if ((rc = launch_sources<R>(h)) != MP_OK) return rc;
         }
         k_advance<<<1, 1, 0, h->stream>>>(h->d_ctr, h->cfg.max_draws);
         CK(cudaGetLastError());
@@ -555,7 +612,7 @@ int mp_destroy(mp_engine *h)
     for (auto e : h->pool) cudaEventDestroy(e);
     void *ptrs[] = { h->d_area, h->d_src_unit, h->d_px, h->d_py, h->d_dist, h->d_obs, h->d_era, h->d_par, h->d_prop,
                      h->d_lsig, h->d_z, h->d_y, h->d_srec, h->d_S[0], h->d_S[1], h->d_aw[0], h->d_aw[1], h->d_partial[0],
-                     h->d_partial[1], h->d_llc, h->d_logu, h->d_parts, h->d_scalar, h->d_flags, h->d_counts, h->d_draws, h->d_cand, h->d_cand_count, h->d_task_order, h->d_ljac, h->d_perm, h->d_scan, h->d_minv, h->d_tile_box, h->d_mlow, h->d_work, h->d_gemm, h->d_tlist, h->d_btasks, h->d_blockmode, h->d_scan_work, h->d_comm_send, h->d_comm_recv, h->d_ctr, h->d_sum, h->d_waic };
+                     h->d_partial[1], h->d_llc, h->d_logu, h->d_parts, h->d_scalar, h->d_flags, h->d_counts, h->d_draws, h->d_cand, h->d_cand_count, h->d_task_order, h->d_ljac, h->d_perm, h->d_scan, h->d_minv, h->d_tile_box, h->d_mlow, h->d_work, h->d_gemm, h->d_tlist, h->d_btasks, h->d_blockmode, h->d_scan_work, h->d_comm_send, h->d_comm_recv, h->d_ctr, h->d_sum, h->d_waic, h->d_src };
     for (void *p : ptrs) if (p) cudaFree(p);
     if (h->stream) cudaStreamDestroy(h->stream);
     delete h;
@@ -1399,6 +1456,47 @@ int mp_get_waic(mp_engine *h, int64_t *nsamples, double *lik_sum, double *loglik
     if (loglik_sum) CK(cudaMemcpyAsync(loglik_sum, h->d_waic + plane, plane, cudaMemcpyDeviceToHost, h->stream));
     if (loglik_sq) CK(cudaMemcpyAsync(loglik_sq, h->d_waic + 2 * plane, plane, cudaMemcpyDeviceToHost, h->stream));
     if (reset) CK(cudaMemsetAsync(h->d_waic, 0, waic_bytes(h), h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    if (nsamples) *nsamples = (int64_t)ns;
+    return MP_OK;
+}
+int mp_set_sources(mp_engine *h, int first_sweep, int thin, int nbins, double bin_width)
+{
+    if (!h) return MP_ERR_ARG;
+    REQUIRE(first_sweep >= 0 && thin >= 0, MP_ERR_ARG, "mp_set_sources: first_sweep and thin must be >= 0");
+    REQUIRE(nbins >= 0 && nbins <= SRC_MAX_BINS, MP_ERR_ARG, "mp_set_sources: nbins must be in [0, 4096]");
+    REQUIRE(nbins == 0 || (std::isfinite(bin_width) && bin_width > 0.0), MP_ERR_ARG, "mp_set_sources: bin_width must be finite and > 0");
+    CK(cudaSetDevice(h->cfg.device));
+    int rc = quiesce(h);                                 // the captured sweeps launch the source kernels or not: capture again
+    if (rc != MP_OK) return rc;
+    const size_t old = h->d_src ? src_layout(h, h->src_nbins).bytes : 0;
+    h->src_first = first_sweep; h->src_thin = thin; h->src_nbins = nbins; h->src_bin_width = nbins > 0 ? bin_width : 0.0;
+    const size_t bytes = src_layout(h, nbins).bytes;
+    if (h->d_src && (thin == 0 || bytes != old)) { CK(cudaFree(h->d_src)); h->d_src = nullptr; }
+    if (thin == 0) return MP_OK;
+    if (!h->d_src) {
+        cudaError_t e = cudaMalloc(&h->d_src, bytes);
+        if (e != cudaSuccess) { h->d_src = nullptr; h->src_thin = 0; h->err = std::string("mp_set_sources: ") + cudaGetErrorString(e); return MP_ERR_CUDA; }
+    }
+    CK(cudaMemsetAsync(h->d_src, 0, bytes, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    return MP_OK;
+}
+int mp_get_sources(mp_engine *h, int64_t *nsamples, uint64_t *events, double *src_sum, double *ext_sum, double *dist_hist, int reset)
+{
+    if (!h) return MP_ERR_ARG;
+    REQUIRE(h->d_src, MP_ERR_STATE, "mp_get_sources: source sums not set (mp_set_sources)");
+    CK(cudaSetDevice(h->cfg.device));
+    const SrcLayout L = src_layout(h, h->src_nbins);
+    const size_t ntrans = nT(h) - 1;
+    unsigned long long ns = 0;
+    CK(cudaMemcpyAsync(&ns, h->d_src + L.nsamples, 8, cudaMemcpyDeviceToHost, h->stream));
+    if (events) CK(cudaMemcpyAsync(events, h->d_src + L.events, 2 * ntrans * 8, cudaMemcpyDeviceToHost, h->stream));
+    if (src_sum) CK(cudaMemcpyAsync(src_sum, h->d_src + L.src_sum, ycells(h) * 8, cudaMemcpyDeviceToHost, h->stream));
+    if (ext_sum) CK(cudaMemcpyAsync(ext_sum, h->d_src + L.ext_sum, ntrans * 8, cudaMemcpyDeviceToHost, h->stream));
+    if (dist_hist && h->src_nbins > 0)
+        CK(cudaMemcpyAsync(dist_hist, h->d_src + L.dist_hist, ntrans * h->src_nbins * 8, cudaMemcpyDeviceToHost, h->stream));
+    if (reset) CK(cudaMemsetAsync(h->d_src + L.sums, 0, L.bytes - L.sums, h->stream));
     CK(cudaStreamSynchronize(h->stream));
     if (nsamples) *nsamples = (int64_t)ns;
     return MP_OK;

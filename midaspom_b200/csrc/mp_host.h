@@ -109,6 +109,10 @@ struct mp_engine {
     // pointwise predictive densities for WAIC (mp_set_waic): lik, loglik, loglik_sq [T][N] and the uint64 sample counter
     unsigned char *d_waic = nullptr;
     int waic_first = 0, waic_thin = 0;    // waic_thin == 0: off
+    // colonisation sources (mp_set_sources): per-sample lists and staging arrays, then the sums (mp_sources.cuh, src_layout)
+    unsigned char *d_src = nullptr;
+    int src_first = 0, src_thin = 0, src_nbins = 0;   // src_thin == 0: off
+    double src_bin_width = 0.0;
     // timing
     bool timing = false;
     struct Span { cudaEvent_t a, b; int cat; };

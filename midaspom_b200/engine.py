@@ -36,6 +36,7 @@ ABI_SYMBOLS = (
     "mp_comm_unique_id", "mp_comm_init", "mp_comm_init_all", "mp_comm_destroy", "mp_comm_rank", "mp_comm_size", "mp_comm_last_error",
     "mp_gather_draws", "mp_gather_draws_all", "mp_sweep_sharded", "mp_sweep_sharded_all", "mp_forecast",
     "mp_set_summaries", "mp_get_summaries", "mp_set_waic", "mp_get_waic", "mp_ppc", "mp_capacity",
+    "mp_set_sources", "mp_get_sources",
 )
 
 
@@ -139,6 +140,8 @@ def load_library(build_if_missing: bool = True) -> C.CDLL:
     L.mp_get_summaries.argtypes = [vp, C.POINTER(C.c_int64), C.POINTER(C.c_uint32), dp, C.POINTER(C.c_uint32), dp, C.c_int]
     L.mp_set_waic.argtypes = [vp, C.c_int, C.c_int]
     L.mp_get_waic.argtypes = [vp, C.POINTER(C.c_int64), dp, dp, dp, C.c_int]
+    L.mp_set_sources.argtypes = [vp, C.c_int, C.c_int, C.c_int, C.c_double]
+    L.mp_get_sources.argtypes = [vp, C.POINTER(C.c_int64), C.POINTER(C.c_uint64), dp, dp, dp, C.c_int]
     L.mp_device_ptr.argtypes = [vp, C.c_int, C.POINTER(vp), C.POINTER(C.c_size_t)]
     L.mp_get_stream.argtypes = [vp, C.POINTER(vp)]
     L.mp_set_timing.argtypes = [vp, C.c_int]
@@ -570,6 +573,29 @@ class Engine:
         out = [np.zeros((self.T, self.N)) for _ in range(3)]
         self._ck(self.lib.mp_get_waic(self.h, C.byref(ns), *[_p(a, _dp) for a in out], int(reset)), "mp_get_waic")
         return dict(nsamples=ns.value, lik_sum=out[0], loglik_sum=out[1], loglik_sq=out[2])
+
+    # -- colonisations attributed to their sources
+    def set_sources(self, first_sweep=0, thin=1, nbins=0, bin_width=0.0):
+        """mp_set_sources: attribute the colonisations of every transition to their source patches at the end of sweeps
+        first_sweep, first_sweep + thin, ... (thin=0: off); nbins > 0 adds a histogram of the shares over source-target
+        distance bins of width bin_width (the last bin open).  Zeroes the sums."""
+        self._ck(self.lib.mp_set_sources(self.h, int(first_sweep), int(thin), int(nbins), float(bin_width)), "mp_set_sources")
+        self._src_bins = (int(nbins), float(bin_width) if int(nbins) > 0 else 0.0)
+
+    def sources(self, reset=False):
+        """mp_get_sources: dict(nsamples, events, unattributed [T-1] uint64, src_sum [T-1, N], ext_sum [T-1], dist_hist
+        [T-1, nbins] or None, bin_width, fingerprint), sums over the accumulated sweeps and this engine's chains; reduce them
+        with midaspom_b200.colonisation_sources."""
+        nbins, width = getattr(self, "_src_bins", (0, 0.0))
+        ns = C.c_int64()
+        ev = np.zeros((2, self.T - 1), dtype=np.uint64)
+        src = np.zeros((self.T - 1, self.N))
+        ext = np.zeros(self.T - 1)
+        hist = np.zeros((self.T - 1, nbins)) if nbins > 0 else None
+        self._ck(self.lib.mp_get_sources(self.h, C.byref(ns), _p(ev, C.POINTER(C.c_uint64)), _p(src, _dp), _p(ext, _dp),
+                                         _p(hist, _dp), int(reset)), "mp_get_sources")
+        return dict(nsamples=ns.value, events=ev[0].copy(), unattributed=ev[1].copy(), src_sum=src, ext_sum=ext, dist_hist=hist,
+                    bin_width=width, fingerprint=hashlib.sha256(self._landscape_key).hexdigest())
 
     @staticmethod
     def _one_param(p):
